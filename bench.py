@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: Gato training step (GatoPolicy.forward + backward + masked loss) in tokens/s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference] [--only]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference] [--only] [--dump-outputs DIR]
 
 One "step" = one fwd+bwd pass of the hot path over one synthetic batch of the named BASELINE.json config
 (default cfg2 = configs[1]: MuJoCo 3-task control, d768 L6 H24, batch 32, k=240).  N>1: launched by torchrun,
@@ -19,6 +19,9 @@ it) with the per-shape table in `roofline.shapes`; `front_end` = tokeniser / ima
 bandwidth; `configs` = the same measurements for cfg3 / cfg4 / cfg5 (the configurations BASELINE.json names for the
 scaling claim), at every N; `cpu_baseline` / `--impl reference` = the UNMODIFIED reference (oracle/_ref, placed there by
 oracle/build_ref.py) on this host's cores (the oracle port only when no reference tree is present).
+
+`--dump-outputs DIR` (rank 0): what the last timed step of --config returned to its caller, as DIR/<name>.npy (see
+sample_outputs).  Inputs and weights are seeded, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -358,6 +361,43 @@ def dp_grad_check(model, sync, batch, world):
             "what": "arena after the production all-reduce vs the fp64 mean of the all-gathered local gradient arenas, max over ranks"}
 
 
+DUMP_LOGITS = 1 << 20          # sampled logits
+DUMP_GRAD = 1 << 18            # elements kept of a larger gradient
+DUMP_LIMIT = 64 << 20          # bytes written in all
+
+
+def sample_outputs(model, logits, loss, plan):
+    """Host copies of what one fwd+bwd step hands its caller: `loss`; `logits`, a sample of DUMP_LOGITS entries of the valid
+    (non-padding) rows -- padding rows carry no defined values; `grad.<parameter name>` for every parameter that received a
+    gradient, whole, or a sample of DUMP_GRAD entries when larger.  The sample indices come from a fixed seed and the shapes
+    alone, so two builds given the same arguments sample the same entries.  Loss and logits repeat bit for bit from run to
+    run; gradients summed with fp32 atomics differ in their rounding."""
+    rs = np.random.RandomState(0)
+    out = {"loss": loss.detach().float().cpu().numpy()}
+    if logits is not None and logits.numel():
+        rows = np.concatenate([b * plan.width + np.arange(plan.first_valid[b], plan.seq_len) for b in range(plan.B)])
+        r = rows[rs.randint(0, rows.shape[0], DUMP_LOGITS)]
+        c = rs.randint(0, logits.shape[-1], DUMP_LOGITS)
+        bi, si, ci = (torch.from_numpy(a).to(logits.device) for a in (r // plan.width, r % plan.width, c))
+        out["logits"] = logits[bi, si, ci].float().cpu().numpy()
+    for name, p in model.named_parameters():
+        if p.grad is None:
+            continue
+        g = p.grad.detach().reshape(-1)
+        if g.numel() > DUMP_GRAD:
+            g = g[torch.from_numpy(np.sort(rs.randint(0, g.numel(), DUMP_GRAD))).to(g.device)]
+        out["grad." + name] = g.float().cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_LIMIT, f"output dump of {total} bytes exceeds {DUMP_LIMIT}"
+    return out
+
+
+def write_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def measure_config(cfg_name, args, dev, rank, world, local, headline):
     """One BASELINE.json configuration: W warm-up + K timed fwd+bwd steps (HBM-resident batch), the GEMM roofline pass, and the
     end-to-end loop from pinned host memory.  Returns the fields of the JSON line for this configuration."""
@@ -383,9 +423,9 @@ def measure_config(cfg_name, args, dev, rank, world, local, headline):
 
     def step(batch):
         model.zero_grad()          # what optimizer.zero_grad() does every step in trainer.py:186
-        _, loss = model(batch, compute_loss=True)
+        logits, loss = model(batch, compute_loss=True)
         loss.backward()
-        return loss
+        return logits, loss
 
     plan = build_plan(host_batch, patch_size=16, context_len=cfgd["context_len"], pad_seq=False)
     tokens_per_step = plan.n_valid_tokens
@@ -412,14 +452,19 @@ def measure_config(cfg_name, args, dev, rank, world, local, headline):
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step(dev_batch)
+    last = step(dev_batch)         # held past the loop only: an earlier step's outputs never outlive it
     e1.record()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     ms = e0.elapsed_time(e1)
     launches = model.launches - l0
+    if headline and args.dump_outputs and rank == 0:
+        # copied now: the passes below run the step again into the same (graph-owned) buffers
+        write_outputs(args.dump_outputs, sample_outputs(model, *last, plan))
+    del last
 
     # ---- roofline of the dominant kernel: CUDA events around every tensor-core GEMM launch.  The timed region above
     # replays the step from CUDA graphs (no room for per-launch events), so the same step is run eagerly right after it
@@ -484,10 +529,10 @@ def measure_config(cfg_name, args, dev, rank, world, local, headline):
     # then drain it so that every copy of the timed steps is issued inside the timed region
     nxt = model.stage(pin_batch, compute_loss=True)
     for _ in range(3):
-        loss = step(nxt)
+        _, loss = step(nxt)
         nxt = model.stage(pin_batch, compute_loss=True)
         loss.item()
-    step(nxt).item()
+    step(nxt)[1].item()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
@@ -498,7 +543,7 @@ def measure_config(cfg_name, args, dev, rank, world, local, headline):
     f0.record()
     nxt = model.stage(pin_batch, compute_loss=True)
     for k in range(args.steps):
-        loss = step(nxt)
+        _, loss = step(nxt)
         if k + 1 < args.steps:
             nxt = model.stage(pin_batch, compute_loss=True)
         loss.item()              # the D2H read of the loss closes every step
@@ -586,7 +631,7 @@ def run_ours(args):
         for name in ("cfg3", "cfg4", "cfg5"):
             if name != args.config:
                 sub = argparse.Namespace(**vars(args))
-                sub.steps, sub.warmup = max(5, min(args.steps, 10)), 3
+                sub.warmup = 3
                 r = measure_config(name, sub, dev, rank, world, local, headline=False)
                 r["steps"], r["warmup"] = sub.steps, sub.warmup
                 others[name] = r
@@ -631,7 +676,13 @@ def main():
     ap.add_argument("--no-graphs", action="store_true", help="launch every kernel eagerly instead of replaying the step from CUDA graphs")
     ap.add_argument("--gemm-report", action="store_true", help="per-shape GEMM timings (CUDA events) on stderr")
     ap.add_argument("--only", action="store_true", help="measure --config only (skip the cfg3 / cfg4 / cfg5 entries of \"configs\")")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of --config returned (loss, sampled logits, "
+                                                          "gradients) to DIR/<name>.npy; --impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours only")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -25,16 +25,18 @@ FILES = ["gato/__init__.py", "gato/policy/__init__.py", "gato/policy/gato_policy
          "gato/policy/input_tokenizers.py", "gato/transformers/__init__.py", "gato/transformers/trajectory_gpt2.py"]
 
 
-def build(src: str = "/root/reference") -> bool:
-    """Returns True when oracle/_ref/gato_ref.zip holds the reference's path files (packed now or already there)."""
+def build(src: str = "/root/reference", dst: str = DST) -> bool:
+    """Returns True when <dst>/gato_ref.zip (by default oracle/_ref/gato_ref.zip) holds the reference's path files (packed now
+    or already there)."""
+    archive = os.path.join(dst, "gato_ref.zip")
     if not os.path.isfile(os.path.join(src, "gato", "policy", "gato_policy.py")):
-        return os.path.isfile(ARCHIVE)
-    os.makedirs(DST, exist_ok=True)
-    loose = os.path.join(DST, "gato")          # an earlier version of this recipe left loose files: remove them
+        return os.path.isfile(archive)
+    os.makedirs(dst, exist_ok=True)
+    loose = os.path.join(dst, "gato")          # an earlier version of this recipe left loose files: remove them
     if os.path.isdir(loose):
         shutil.rmtree(loose)
     manifest = []
-    tmp = ARCHIVE + ".tmp"
+    tmp = archive + ".tmp"
     with zipfile.ZipFile(tmp, "w", compression=zipfile.ZIP_DEFLATED) as z:
         for rel in FILES:
             s = os.path.join(src, rel)
@@ -43,8 +45,8 @@ def build(src: str = "/root/reference") -> bool:
             info.compress_type = zipfile.ZIP_DEFLATED
             z.writestr(info, data)
             manifest.append(f"{hashlib.sha256(data).hexdigest()}  {rel}")
-    os.replace(tmp, ARCHIVE)
-    with open(os.path.join(DST, "MANIFEST.sha256"), "w") as f:
+    os.replace(tmp, archive)
+    with open(os.path.join(dst, "MANIFEST.sha256"), "w") as f:
         f.write("\n".join(manifest) + "\n")
     return True
 

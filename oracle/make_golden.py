@@ -6,7 +6,8 @@ committed, the reference is not.  Inputs and weights are derived from numpy MT19
 OUTPUTS.  What is recorded:
 
   tokenizer_kat.npz   ContinuousTokenizer.encode (input_tokenizers.py:17-30) on hand-picked edge
-                      values and 400k values (random + clustered on bin edges), both tokenizers;
+                      values and a fixed seeded subset of 550k values (random + clustered on bin
+                      edges; ``kat_subset``, which keeps the file small), both tokenizers;
                       PatchPosEncoding eval bins for n=1..40 (embeddings.py:80-100).
   tok_<cfg>.npz       tokenize_input_dicts ids / target masks / token masks (gato_policy.py:195-432)
                       for the five BASELINE.json configs at the real vocabulary (50257+1024+1024).
@@ -14,6 +15,9 @@ OUTPUTS.  What is recorded:
                       and token-embedding samples, per-parameter gradient norms and samples.
   scale_<cfg>.npz     the same record for the five BASELINE.json configs AT MODEL SCALE (d=768 / L=6 / H=24 and the
                       real 52 305-row vocabulary; cfg1 d=128 / L=3 / H=1) on a reduced batch (``SCALE_BATCH``).
+  oracle_vs_reference.npz   the ORACLE's outputs on the inputs of tests/test_oracle_vs_reference.py, which those tests
+                      compare with when no reference checkout is present (``python -m oracle.make_golden vsref``;
+                      see gen_vs_reference).
 """
 from __future__ import annotations
 
@@ -71,12 +75,22 @@ def kat_values() -> np.ndarray:
     return np.concatenate([edge, wide, unit, near, pre]).astype(np.float32)
 
 
+KAT_KEEP = 40_000
+
+
+def kat_subset(x: np.ndarray) -> np.ndarray:
+    """Every hand-picked edge value (the first 21) and a fixed seeded sample of the rest, in their original order."""
+    rs = np.random.RandomState(12)
+    rest = np.sort(rs.choice(np.arange(21, x.shape[0]), KAT_KEEP - 21, replace=False))
+    return x[np.concatenate([np.arange(21), rest])]
+
+
 def gen_tokenizer_kat():
     ref_shim.install_shims()
     from gato.policy.input_tokenizers import ContinuousTokenizer
     from gato.policy.embeddings import PatchPosEncoding
 
-    x = kat_values()
+    x = kat_subset(kat_values())
     obs_tok = ContinuousTokenizer(use_mu_law=True, mu=100, M=256, n_bins=1024, offset=50257)
     act_tok = ContinuousTokenizer(use_mu_law=False, mu=100, M=256, n_bins=1024, offset=50257)
     obs = obs_tok.encode(torch.from_numpy(x.copy())).numpy()
@@ -235,11 +249,174 @@ def gen_fwd_small():
             print("fwd", case, mode, tuple(logits.shape), float(loss))
 
 
+# --------------------------------------------------------------------------------------
+# tests/test_oracle_vs_reference.py: inputs, and the record its tests compare the oracle with when no reference checkout is
+# present.  The record holds the ORACLE's outputs on these inputs, taken at a revision where every one of those tests passed
+# against the live reference; it pins the oracle to what the reference was shown to produce.  With a reference checkout the
+# tests compare with the reference itself, as before.
+# --------------------------------------------------------------------------------------
+VSREF = os.path.join(GOLD, "oracle_vs_reference.npz")
+
+
+def _f32(a):
+    return torch.from_numpy(np.asarray(a, dtype=np.float32))
+
+
+def vsref_forward_inputs(seed: int):
+    cfg = O.GatoConfig(embed_dim=64, layers=2, heads=2, context_len=128, text_tokens=200)
+    rs = np.random.RandomState(seed)
+    batch = [
+        dict(continuous_obs=_f32(rs.standard_normal((5, 4)) * 4), continuous_actions=_f32(np.clip(rs.standard_normal((5, 2)), -1, 1))),
+        dict(images=_f32(rs.randint(0, 256, (2, 3, 32, 32))), discrete_actions=torch.from_numpy(rs.randint(0, 6, (2, 1)).astype(np.int32))),
+        dict(text=rs.randint(0, 200, (23,)).tolist()),
+        dict(images=torch.from_numpy(rs.randint(0, 256, (1, 3, 48, 32)).astype(np.uint8)), text=torch.from_numpy(rs.randint(0, 200, (7,)))),
+    ]
+    return cfg, O.make_weights(cfg, seed=seed), batch
+
+
+def vsref_sweep_values() -> np.ndarray:
+    rs = np.random.RandomState(99)
+    return np.concatenate([rs.standard_normal(300_000) * 10, rs.uniform(-1.5, 1.5, 300_000),
+                           np.exp(rs.uniform(-30, 10, 200_000))]).astype(np.float32)
+
+
+VSREF_SWEEP_KEEP = 40_000
+
+
+def vsref_sweep_index(n: int) -> np.ndarray:
+    """The recorded entries of the sweep: a fixed seeded sample (the whole sweep's ids would not fit a small file)."""
+    return np.sort(np.random.RandomState(13).choice(n, VSREF_SWEEP_KEEP, replace=False))
+
+
+def vsref_dropout_inputs():
+    cfg = O.GatoConfig(embed_dim=64, layers=2, heads=2, context_len=64, text_tokens=200)
+    rs = np.random.RandomState(5)
+    batch = [
+        dict(continuous_obs=_f32(rs.standard_normal((4, 3)) * 4), continuous_actions=_f32(np.clip(rs.standard_normal((4, 2)), -1, 1))),
+        dict(text=rs.randint(0, 200, (17,)).tolist()),
+    ]
+    return cfg, O.make_weights(cfg, seed=5), batch
+
+
+def vsref_dropout_masks(cfg, batch, p_embd=0.1, p=0.25):
+    """The Bernoulli multipliers the test draws for the reference's dropout calls, in their call order (embeddings, then per
+    layer attention weights / attention residual / MLP residual), from one generator seeded with 77."""
+    B, S = O.tokenize(batch, cfg).tokens.shape
+    gen = torch.Generator().manual_seed(77)
+    draw = lambda shape, q: (torch.rand(shape, generator=gen) >= q).to(torch.float32) / (1.0 - q)  # noqa: E731
+    drop = {"embd": draw((B, S, cfg.embed_dim), p_embd)}
+    for i in range(cfg.layers):
+        drop[("attn", i)] = draw((B, cfg.heads, S, S), p)
+        drop[("resid_attn", i)] = draw((B, S, cfg.embed_dim), p)
+        drop[("resid_mlp", i)] = draw((B, S, cfg.embed_dim), p)
+    return drop
+
+
+def vsref_inference_inputs():
+    cfg = O.GatoConfig(embed_dim=64, layers=2, heads=2, context_len=48, text_tokens=200)
+    rs = np.random.RandomState(3)
+    text = dict(text=rs.randint(0, 200, (9,)).tolist())
+    rs = np.random.RandomState(3)
+    rs.randint(0, 200, (9,))                   # the same draws the test makes before the control inputs
+    obs, act = _f32(rs.standard_normal((3, 5)) * 2), _f32(np.clip(rs.standard_normal((3, 2)), -1, 1))
+    img = _f32(rs.randint(0, 256, (2, 3, 32, 32)))
+    dact = torch.from_numpy(rs.randint(0, 4, (2, 1)).astype(np.int32))
+    return cfg, O.make_weights(cfg, seed=9), text, (obs, act), (img, dact)
+
+
+def vsref_pretrained_checkpoint(path: str) -> None:
+    """A local GPT-2 checkpoint (transformers' own init, seed 5, weights x4 so that the erf and tanh GELU forms differ)."""
+    import transformers
+    cfg = transformers.GPT2Config(vocab_size=300, n_embd=64, n_layer=2, n_head=4, n_positions=128, n_ctx=128)
+    torch.manual_seed(5)
+    hf = transformers.GPT2Model(cfg)
+    with torch.no_grad():
+        for p in hf.parameters():
+            p.mul_(4.0)
+    hf.save_pretrained(path)
+
+
+def vsref_pretrained_weights(path: str, act: str):
+    """Oracle weights of --pretrained_lm: the decoder and wte from the checkpoint, wte in the text rows of embed_token, the
+    rest seeded."""
+    oc = O.GatoConfig(embed_dim=64, layers=2, heads=4, context_len=128, text_tokens=300, activation_fn=act, wte_rows=300)
+    w = O.make_weights(oc, seed=5)
+    raw = ref_shim.load_gpt2_checkpoint(path)
+    for k, t in raw.items():
+        if "transformer." + k in w:
+            w["transformer." + k] = t.detach().clone().to(torch.float32)
+    w["embed_token.weight"][:300] = raw["wte.weight"]
+    return oc, w
+
+
+def vsref_pretrained_batch():
+    rs = np.random.RandomState(6)
+    return [{"text": list(range(1, 40))}, {"continuous_obs": _f32(rs.standard_normal((5, 3))), "continuous_actions": _f32(rs.uniform(0, 1, (5, 2)))}]
+
+
+def _forward_record(out, w, prefix, rs, n_logits=4000):
+    lg = out.logits.detach().numpy()
+    B, S, V = lg.shape
+    li = np.stack([rs.randint(0, B, n_logits), rs.randint(0, S, n_logits), rs.randint(0, V, n_logits)], 1)
+    rec = {prefix + "tokens": out.tokens.numpy(), prefix + "target_masks": out.target_masks.numpy(), prefix + "token_masks": out.token_masks.numpy(),
+           prefix + "emb": out.token_embeddings.detach().numpy()[:, ::4], prefix + "logit_idx": li, prefix + "logit_val": lg[li[:, 0], li[:, 1], li[:, 2]],
+           prefix + "logits_rowsum": lg.sum(-1), prefix + "loss": np.float64(out.loss.item())}
+    for n, t in w.items():
+        if t.grad is not None:
+            g = t.grad.numpy().reshape(-1)
+            idx = rs.randint(0, g.shape[0], min(64, g.shape[0]))
+            rec[prefix + "gmax." + n], rec[prefix + "gidx." + n], rec[prefix + "gval." + n] = np.float64(np.abs(g).max()), idx, g[idx]
+    return rec
+
+
+def gen_vs_reference(tmp_dir: str):
+    """Writes VSREF from the oracle (see the comment above)."""
+    rs = np.random.RandomState(21)
+    rec = {}
+    for seed in (11, 12):
+        cfg, w, batch = vsref_forward_inputs(seed)
+        for t in w.values():
+            t.requires_grad_(True)
+        out = O.forward(w, batch, cfg, compute_loss=True)
+        out.loss.backward()
+        rec.update(_forward_record(out, w, f"fb{seed}.", rs))
+    x = vsref_sweep_values()
+    idx = vsref_sweep_index(x.shape[0])
+    for mu_law in (True, False):
+        rec[f"sweep.{int(mu_law)}"] = (O.discretize(x, mu_law, O.GatoConfig())[idx] - 50257).astype(np.uint16)
+    cfg, w, batch = vsref_dropout_inputs()
+    for t in w.values():
+        t.requires_grad_(True)
+    out = O.forward(w, batch, cfg, compute_loss=True, training=True, drop=vsref_dropout_masks(cfg, batch))
+    out.loss.backward()
+    rec.update(_forward_record(out, w, "drop.", rs))
+    cfg, w, text, (obs, act), (img, dact) = vsref_inference_inputs()
+    ologits, otoks = O.predict_text(w, text, cfg, max_length=6)
+    rec["inf.text_logits"], rec["inf.text_tokens"] = ologits.numpy(), np.asarray(otoks)
+    rec["inf.cont_action"] = O.predict_control(w, dict(continuous_obs=obs, continuous_actions=act), cfg, action_tokens=2).numpy()
+    rec["inf.disc_action"] = np.asarray(int(O.predict_control(w, dict(images=img, discrete_actions=dact), cfg, action_tokens=1, discrete_n=4)))
+    vsref_pretrained_checkpoint(tmp_dir)
+    for act_fn in ("gelu_new", "gelu"):
+        oc, w = vsref_pretrained_weights(tmp_dir, act_fn)
+        out = O.forward(w, vsref_pretrained_batch(), oc, compute_loss=True)
+        valid = out.logits.detach().numpy()[out.token_masks.bool().numpy()]
+        pick = np.random.RandomState(22).randint(0, valid.size, 4000)
+        rec["pre.idx"], rec[f"pre.{act_fn}.logits"] = pick, valid.reshape(-1)[pick]
+    rec["source"] = np.array("oracle")
+    np.savez_compressed(VSREF, **rec)
+    print("oracle_vs_reference", os.path.getsize(VSREF), "bytes")
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(os.cpu_count() or 1)
     if len(sys.argv) > 1 and sys.argv[1] == "scale":
         gen_fwd_scale(sys.argv[2:] or None)
+        return
+    if len(sys.argv) > 1 and sys.argv[1] == "vsref":      # needs no reference checkout
+        import tempfile
+        with tempfile.TemporaryDirectory() as d:
+            gen_vs_reference(d)
         return
     gen_tokenizer_kat()
     gen_tok_configs()

@@ -241,6 +241,13 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert out2.returncode == 0 and "{" not in out2.stdout
 
 
+def test_bench_rejects_arguments_it_cannot_honour():
+    """--steps below 1 would time nothing; --dump-outputs writes what the GPU arm's step returned, so the CPU arm refuses it."""
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and extra[-2] in out.stderr, (extra, out.stderr[-500:])
+
+
 @pytest.mark.parametrize("seed", range(12))
 def test_plan_matches_oracle_on_random_mixed_batches(seed):
     """Random mixtures of every modality (text lists / tensors, uint8 / float frames of several sizes, precomputed image
@@ -266,29 +273,44 @@ def test_plan_matches_oracle_on_random_mixed_batches(seed):
 
 
 def test_vendored_reference_recipe(tmp_path):
-    """oracle/build_ref.py: the archive under oracle/_ref/ holds the mounted reference's path files byte for byte (no loose reference
-    source in the tree) and imports through the shims (what bench.py --impl reference uses on the GPU box)."""
+    """oracle/build_ref.py: the archive holds the reference's path files byte for byte (an empty entry for a package without an
+    __init__.py), leaves no loose reference source beside it and lists every file in its manifest.  Packed from a reference
+    checkout when one is present -- and then imported through the shims (what bench.py --impl reference uses) -- else from a
+    stand-in tree of the same layout."""
+    import hashlib
     import zipfile
-    from oracle import build_ref
-    if not os.path.isdir("/root/reference/gato"):
-        pytest.skip("no /root/reference in this container")
-    assert build_ref.build()
-    with zipfile.ZipFile(build_ref.ARCHIVE) as z:
+    from oracle import build_ref, ref_shim
+    if ref_shim.reference_kind() == "mounted":
+        src = ref_shim.REFERENCE_ROOT
+    else:
+        src = str(tmp_path / "src")
+        for k, rel in enumerate(build_ref.FILES):
+            if rel != "gato/transformers/__init__.py":
+                os.makedirs(os.path.dirname(os.path.join(src, rel)), exist_ok=True)
+                open(os.path.join(src, rel), "wb").write(f"# {rel}\n".encode() * (k + 1))
+    dst = str(tmp_path / "_ref")
+    assert build_ref.build(src, dst)
+    archive = os.path.join(dst, "gato_ref.zip")
+    manifest = open(os.path.join(dst, "MANIFEST.sha256")).read().split("\n")
+    with zipfile.ZipFile(archive) as z:
         assert sorted(z.namelist()) == sorted(build_ref.FILES)
         for rel in build_ref.FILES:
-            src = os.path.join("/root/reference", rel)
-            if os.path.exists(src):
-                assert z.read(rel) == open(src, "rb").read(), rel
-    assert not os.path.isdir(os.path.join(build_ref.DST, "gato")), "loose reference sources under oracle/_ref"
-    code = ("from oracle import ref_shim; assert ref_shim.reference_kind() == 'vendored', ref_shim.REFERENCE_ROOT; "
+            p = os.path.join(src, rel)
+            data = open(p, "rb").read() if os.path.exists(p) else b""
+            assert z.read(rel) == data, rel
+            assert f"{hashlib.sha256(data).hexdigest()}  {rel}" in manifest, rel
+    assert not os.path.isdir(os.path.join(dst, "gato")), "loose reference sources beside the archive"
+    # oracle/_ref must stay out of the history
+    assert "oracle/_ref/" in open(os.path.join(ROOT, ".gitignore")).read()
+    if ref_shim.reference_kind() != "mounted":
+        return
+    code = ("from oracle import ref_shim; import os; assert ref_shim.REFERENCE_ROOT == os.environ['NEKO_REFERENCE_ROOT'], ref_shim.REFERENCE_ROOT; "
             "G = ref_shim.load_reference_policy_class(); "
             "m = G(device='cpu', embed_dim=32, layers=1, heads=1, dropout=0.0, resid_mid_channels=128, context_len=32); "
             "l, loss = m([{'text': [1, 2, 3]}], compute_loss=True); loss.backward(); print('ok')")
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=ROOT,
-                         env=dict(os.environ, NEKO_REFERENCE_ROOT=build_ref.ARCHIVE))
+                         env=dict(os.environ, NEKO_REFERENCE_ROOT=archive))
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-1500:]
-    # oracle/_ref must stay out of the history
-    assert "oracle/_ref/" in open(os.path.join(ROOT, ".gitignore")).read()
 
 
 def test_copy_engine_bucket_schedule_covers_the_arena_once():

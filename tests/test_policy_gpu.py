@@ -780,3 +780,30 @@ def test_kv_cached_image_response_matches_full_recompute():
             if float(top[0] - top[1]) <= 4 * LOGIT_TOL:
                 break
             assert t_kv[i] == t_full[i], (question, i)
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs, run twice with the same arguments: float arrays only, 64 MB at most, loss and logits bit for bit
+    the same (gradients summed with fp32 atomics may round differently), and the line reports the --steps it was given."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    runs = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--only", "--steps", "2", "--no-cpu-baseline", "--no-front-end",
+                              "--dump-outputs", str(d)], capture_output=True, text=True, timeout=900, cwd=root)
+        assert out.returncode == 0, out.stderr[-3000:]
+        line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 2 and line["value"] > 0
+        runs.append({f[:-4]: np.load(d / f) for f in os.listdir(d) if f.endswith(".npy")})
+    a, b = runs
+    assert len(os.listdir(tmp_path / "0")) == len(a) and set(a) == set(b)
+    assert {"loss", "logits"} < set(a) and any(k.startswith("grad.") for k in a)
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert np.array_equal(a["loss"], b["loss"]) and np.array_equal(a["logits"], b["logits"])
+    assert np.isfinite(a["logits"]).all()
+    for k in a:
+        assert a[k].shape == b[k].shape, k
