@@ -76,7 +76,7 @@ typedef struct neko_sample_desc {
   int32_t cact_off;
   int32_t dact_off;
   int32_t patch_off;     /* first row of this sample in patch_emb [P_total, d]           */
-  int32_t reserved0;
+  int32_t row_base;      /* packed layout: first row of this sample (prefix sum of lengths) */
   int32_t reserved1;
 } neko_sample_desc;
 
@@ -102,6 +102,15 @@ int neko_tokenize_embed_fwd(const neko_sample_desc* descs, int B, int d, const n
                             int64_t* tokens, float* target_masks, float* token_masks,
                             float* token_embeddings, int32_t* err_flag, void* stream);
 
+/* Packed (padding-free) layout: the same ids / masks / embeddings, but sample b's valid position s is written to row
+ * descs[b].row_base + (s - seq_off) of tokens [T], target/token masks [T] and token_embeddings [T,d] (T = sum of the
+ * sample lengths); padding positions write nothing.  seq_len / width of host_params as in the padded call. */
+int neko_tokenize_embed_packed_fwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* host_params,
+                                   const float* fvals, const int32_t* ivals, const float* patch_emb,
+                                   const float* embed_table, const float* pos_table, const float* sep_vec,
+                                   int64_t* tokens, float* target_masks, float* token_masks,
+                                   float* token_embeddings, int32_t* err_flag, void* stream);
+
 /* Backward of the embedding half (autograd of gato_policy.py:275-393): scatter-adds into
  * d_embed_table [vocab,d], d_pos_table [ctx_rows,d], d_sep [d] (all fp32, accumulated) and writes
  * d_patch_emb [P_total,d] (nullable). */
@@ -109,6 +118,11 @@ int neko_embed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok_p
                    const int64_t* tokens, const float* d_token_embeddings,
                    float* d_embed_table, float* d_pos_table, float* d_sep, float* d_patch_emb,
                    void* stream);
+/* neko_embed_bwd on the packed layout: tokens [T], d_token_embeddings [T,d] (rows as in the packed forward). */
+int neko_embed_packed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* host_params,
+                          const int64_t* tokens, const float* d_token_embeddings,
+                          float* d_embed_table, float* d_pos_table, float* d_sep, float* d_patch_emb,
+                          void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * LayerNorm (ln_1 / ln_2 / ln_f, trajectory_gpt2.py:323,353,779). x fp32 [N,d] -> y bf16 (fp16 if out_f16).
@@ -196,6 +210,18 @@ int neko_attention_decode(const uint16_t* q, const uint16_t* k_cache, const uint
 int neko_attention_bwd(const uint16_t* qkv, const uint16_t* out, const uint16_t* dout, const float* lse,
                        const int32_t* first_valid, uint16_t* dqkv, float* delta, int B, int S, int S_valid,
                        int H, int dh, int out_f16, const neko_dropout* drop, void* stream);
+/* Variable-length (packed) causal attention: sample b owns rows [cu_seqlens[b], cu_seqlens[b+1]) of qkv bf16 [T,3*H*dh],
+ * out bf16 [T,H*dh] and lse fp32 [H,T]; query q of a sample attends its own keys [0, q].  S_max = longest sample (grid
+ * extent).  Attention dropout keeps the padded layout's coordinates so the masks equal neko_attention_fwd's bit for bit:
+ * row (b*H + h)*S_width + first_valid[b] + q, column first_valid[b] + k, where S_width is the padded row length (S, or
+ * context_len with --pad_seq) and first_valid[b] = S - length of b.  Head dims 16, 32, 64, 128 (mma.sync kernels). */
+int neko_attention_varlen_fwd(const uint16_t* qkv, const int32_t* cu_seqlens, const int32_t* first_valid, uint16_t* out,
+                              uint16_t* out2_bf16 /* nullable second copy */, float* lse, int B, int T, int S_max, int S_width,
+                              int H, int dh, int out_f16, const neko_dropout* drop, void* stream);
+/* dqkv bf16 [T,3*H*dh]; delta fp32 [H,T] is caller-provided scratch. */
+int neko_attention_varlen_bwd(const uint16_t* qkv, const uint16_t* out, const uint16_t* dout, const float* lse,
+                              const int32_t* cu_seqlens, const int32_t* first_valid, uint16_t* dqkv, float* delta, int B, int T,
+                              int S_max, int S_width, int H, int dh, int out_f16, const neko_dropout* drop, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Masked cross entropy (gato_policy.py:174-186).  rows int32 [n_rows]: flat source positions

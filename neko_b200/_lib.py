@@ -22,7 +22,7 @@ class SampleDesc(C.Structure):
     """neko_sample_desc (include/neko_b200.h)."""
     _fields_ = [(n, C.c_int32) for n in (
         "n_timesteps", "n_patches", "n_text", "n_cobs", "n_dobs", "n_cact", "n_dact", "seq_off",
-        "text_off", "cobs_off", "dobs_off", "cact_off", "dact_off", "patch_off", "reserved0", "reserved1")]
+        "text_off", "cobs_off", "dobs_off", "cact_off", "dact_off", "patch_off", "row_base", "reserved1")]
 
 
 class TokParams(C.Structure):

@@ -77,15 +77,53 @@ __device__ __forceinline__ void frag_b_kn(const Tile<DH>& t, int k0, int n0, int
   ldsm_x4_t(t.addr(k0 + (lane & 7) + (((lane >> 3) & 1) << 3), n0 + ((lane >> 4) << 3)), b[0], b[1], b[2], b[3]);
 }
 
+// Where one (sample, head) lives.  Padded layout: sample b is rows [b*S, (b+1)*S) of qkv / out / dout, keys and queries
+// from first_valid[b] up to S_valid, statistics (lse, delta) at [b, h, :] of [B, H, S].  VARLEN (packed layout, no
+// padding rows): sample b is rows [cu[b], cu[b+1]) with keys and queries from 0, statistics at [h, cu[b]:] of [H, T].
+// The dropout coordinates stay those of the padded layout: row (b*H + h)*S + first_valid[b] + query, column
+// first_valid[b] + key, with S the padded width -- the masks are the padded kernels' bit for bit.
+struct AttnSeq {
+  long long row0;   // first row of the sample
+  long long stat0;  // first lse / delta element of this (sample, head)
+  int lo;           // first valid key / query
+  int valid;        // queries and keys in [lo, valid) are live
+  int end;          // rows [0, end) exist: tile loads zero-fill past it, write-out stops there
+  int doff;         // dropout row / column offset
+};
+template <bool VARLEN>
+__device__ __forceinline__ AttnSeq attn_seq(int b, int h, int H, int S, int S_valid, int T, const int32_t* __restrict__ first_valid,
+                                            const int32_t* __restrict__ cu_seqlens) {
+  AttnSeq r;
+  if (VARLEN) {
+    const int c0 = cu_seqlens[b];
+    r.row0 = c0; r.stat0 = (long long)h * T + c0; r.lo = 0; r.valid = r.end = cu_seqlens[b + 1] - c0; r.doff = first_valid[b];
+  } else {
+    r.row0 = (long long)b * S; r.stat0 = ((long long)b * H + h) * S; r.lo = first_valid[b]; r.valid = S_valid; r.end = S; r.doff = 0;
+  }
+  return r;
+}
+// multipliers of keys (col, col + 1) for any column parity (VARLEN: the column offset first_valid[b] may be odd)
+__device__ __forceinline__ void drop_cols(uint32_t rowkey, int col, uint32_t thr16, float scale, float& m0, float& m1) {
+  const uint32_t b0 = drop_bits(rowkey, (uint32_t)col >> 1);
+  if ((col & 1) == 0) {
+    m0 = (b0 & 0xffffu) >= thr16 ? scale : 0.f;
+    m1 = (b0 >> 16) >= thr16 ? scale : 0.f;
+  } else {
+    m0 = (b0 >> 16) >= thr16 ? scale : 0.f;
+    m1 = (drop_bits(rowkey, ((uint32_t)col >> 1) + 1u) & 0xffffu) >= thr16 ? scale : 0.f;
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // forward
 // ---------------------------------------------------------------------------------------------
 // DROP: attn_dropout (trajectory_gpt2.py:179) on the softmax weights: the row sum (normaliser) uses the undropped
 // probabilities, the P V product the masked and rescaled ones; mask element = (row (b*H + h)*S + query, column key).
-template <int DH, bool DROP>
+template <int DH, bool DROP, bool VARLEN>
 __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __restrict__ qkv, const int32_t* __restrict__ first_valid,
                                                                bf16* __restrict__ out, bf16* __restrict__ out2, float* __restrict__ lse, int S,
-                                                               int S_valid, int H, float scale_log2, int out_f16, DropCfg drop) {
+                                                               int S_valid, int H, float scale_log2, int out_f16, DropCfg drop,
+                                                               const int32_t* __restrict__ cu_seqlens, int T) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   pdl_launch_dependents();
   pdl_wait();
@@ -95,13 +133,20 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __res
   auto sV = [&](int bi) { return Tile<DH>{s0 + (3 + bi) * Tile<DH>::BYTES}; };
 
   const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * ATT_BLK;
+  AttnSeq sq{};
+  if (VARLEN) {
+    sq = attn_seq<VARLEN>(b, h, H, S, S_valid, T, first_valid, cu_seqlens);
+    if (q0 >= sq.end) return;
+  }
+  // the padded instantiations take every bound from the kernel arguments, as they always have (same code, same registers)
+  const int r_end = VARLEN ? sq.end : S, s_valid = VARLEN ? sq.valid : S_valid, doff = VARLEN ? sq.doff : 0;
   const int d = H * DH;
   const long long pitch = 3LL * d;
-  const bf16* base = qkv + (long long)b * S * pitch;
-  const int lo = first_valid[b];
+  const bf16* base = qkv + (VARLEN ? sq.row0 : (long long)b * S) * pitch;
+  const int lo = VARLEN ? sq.lo : first_valid[b];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, q = lane & 3;
   const int row_a = q0 + warp * 16 + g, row_b = row_a + 8;
-  const int q_hi = min(q0 + ATT_BLK, S_valid);  // queries in [max(q0,lo), q_hi) are live
+  const int q_hi = min(q0 + ATT_BLK, s_valid);  // queries in [max(q0,lo), q_hi) are live
 
   float o[DH / 8][4];
 #pragma unroll
@@ -110,23 +155,23 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __res
   uint32_t rk_a = 0u, rk_b = 0u;
   if (DROP) {
     const uint32_t dkey = drop_key(drop);
-    rk_a = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + row_a));
-    rk_b = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + row_b));
+    rk_a = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + doff + row_a));
+    rk_b = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + doff + row_b));
   }
 
   if (q_hi > lo && q_hi > q0) {
     const int j_begin = (lo / ATT_BLK) * ATT_BLK;
-    load_tile_async<DH>(sQ, base + h * DH, pitch, q0, S);
-    load_tile_async<DH>(sK(0), base + d + h * DH, pitch, j_begin, S);
-    load_tile_async<DH>(sV(0), base + 2 * d + h * DH, pitch, j_begin, S);
+    load_tile_async<DH>(sQ, base + h * DH, pitch, q0, r_end);
+    load_tile_async<DH>(sK(0), base + d + h * DH, pitch, j_begin, r_end);
+    load_tile_async<DH>(sV(0), base + 2 * d + h * DH, pitch, j_begin, r_end);
     cp_async_commit();
     uint32_t qa[DH / 16][4];
     int buf = 0;
     for (int j0 = j_begin; j0 < q_hi; j0 += ATT_BLK, buf ^= 1) {
       const bool more = (j0 + ATT_BLK) < q_hi;
       if (more) {  // prefetch the next K/V tile into the other buffer
-        load_tile_async<DH>(sK(buf ^ 1), base + d + h * DH, pitch, j0 + ATT_BLK, S);
-        load_tile_async<DH>(sV(buf ^ 1), base + 2 * d + h * DH, pitch, j0 + ATT_BLK, S);
+        load_tile_async<DH>(sK(buf ^ 1), base + d + h * DH, pitch, j0 + ATT_BLK, r_end);
+        load_tile_async<DH>(sV(buf ^ 1), base + 2 * d + h * DH, pitch, j0 + ATT_BLK, r_end);
         cp_async_commit();
         cp_async_wait<1>();
       } else {
@@ -158,10 +203,10 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __res
 #pragma unroll
         for (int n = 0; n < ATT_BLK / 8; ++n) {
           const int key = j0 + n * 8 + 2 * q;
-          if (key < lo || key > row_a || row_a >= S_valid) s[n][0] = -INFINITY;
-          if (key + 1 < lo || key + 1 > row_a || row_a >= S_valid) s[n][1] = -INFINITY;
-          if (key < lo || key > row_b || row_b >= S_valid) s[n][2] = -INFINITY;
-          if (key + 1 < lo || key + 1 > row_b || row_b >= S_valid) s[n][3] = -INFINITY;
+          if (key < lo || key > row_a || row_a >= s_valid) s[n][0] = -INFINITY;
+          if (key + 1 < lo || key + 1 > row_a || row_a >= s_valid) s[n][1] = -INFINITY;
+          if (key < lo || key > row_b || row_b >= s_valid) s[n][2] = -INFINITY;
+          if (key + 1 < lo || key + 1 > row_b || row_b >= s_valid) s[n][3] = -INFINITY;
         }
       }
 #pragma unroll
@@ -193,12 +238,20 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __res
       if (DROP) {
 #pragma unroll
         for (int n = 0; n < ATT_BLK / 8; ++n) {
-          const uint32_t pr = (uint32_t)((j0 + n * 8) >> 1) + q;
           float m0, m1;
-          drop_pair(rk_a, pr, drop.thr16, drop.scale, m0, m1);
-          s[n][0] *= m0; s[n][1] *= m1;
-          drop_pair(rk_b, pr, drop.thr16, drop.scale, m0, m1);
-          s[n][2] *= m0; s[n][3] *= m1;
+          if (VARLEN) {
+            const int col = doff + j0 + n * 8 + 2 * q;
+            drop_cols(rk_a, col, drop.thr16, drop.scale, m0, m1);
+            s[n][0] *= m0; s[n][1] *= m1;
+            drop_cols(rk_b, col, drop.thr16, drop.scale, m0, m1);
+            s[n][2] *= m0; s[n][3] *= m1;
+          } else {
+            const uint32_t pr = (uint32_t)((j0 + n * 8) >> 1) + q;
+            drop_pair(rk_a, pr, drop.thr16, drop.scale, m0, m1);
+            s[n][0] *= m0; s[n][1] *= m1;
+            drop_pair(rk_b, pr, drop.thr16, drop.scale, m0, m1);
+            s[n][2] *= m0; s[n][3] *= m1;
+          }
         }
       }
 #pragma unroll
@@ -229,27 +282,27 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __res
     l_b += __shfl_xor_sync(0xffffffffu, l_b, 2);
   }
   // write-out: dead rows (padding) -> zeros, lse = +inf so that backward sees p = 0
-  if (row_a < lo || row_a >= S_valid) l_a = 0.f;   // padding rows
-  if (row_b < lo || row_b >= S_valid) l_b = 0.f;
+  if (row_a < lo || row_a >= s_valid) l_a = 0.f;   // padding rows
+  if (row_b < lo || row_b >= s_valid) l_b = 0.f;
   const float inv_a = (l_a > 0.f) ? 1.f / l_a : 0.f, inv_b = (l_b > 0.f) ? 1.f / l_b : 0.f;
   const float kLn2 = 0.6931471805599453f;
-  bf16* ob = out + (long long)b * S * d + h * DH;
-  bf16* ob2 = out2 ? out2 + (long long)b * S * d + h * DH : nullptr;
-  if (row_a < S) {
+  bf16* ob = out + (VARLEN ? sq.row0 : (long long)b * S) * d + h * DH;
+  bf16* ob2 = out2 ? out2 + (VARLEN ? sq.row0 : (long long)b * S) * d + h * DH : nullptr;
+  if (row_a < r_end) {
 #pragma unroll
     for (int n = 0; n < DH / 8; ++n) {
       *reinterpret_cast<uint32_t*>(ob + (long long)row_a * d + n * 8 + 2 * q) = pack_16x2(o[n][0] * inv_a, o[n][1] * inv_a, out_f16 != 0);
       if (ob2) *reinterpret_cast<uint32_t*>(ob2 + (long long)row_a * d + n * 8 + 2 * q) = pack_bf16x2(o[n][0] * inv_a, o[n][1] * inv_a);
     }
-    if (q == 0) lse[((long long)b * H + h) * S + row_a] = (l_a > 0.f) ? (m_a * scale_log2 + log2f(l_a)) * kLn2 : INFINITY;
+    if (q == 0) lse[(VARLEN ? sq.stat0 : ((long long)b * H + h) * S) + row_a] = (l_a > 0.f) ? (m_a * scale_log2 + log2f(l_a)) * kLn2 : INFINITY;
   }
-  if (row_b < S) {
+  if (row_b < r_end) {
 #pragma unroll
     for (int n = 0; n < DH / 8; ++n) {
       *reinterpret_cast<uint32_t*>(ob + (long long)row_b * d + n * 8 + 2 * q) = pack_16x2(o[n][2] * inv_b, o[n][3] * inv_b, out_f16 != 0);
       if (ob2) *reinterpret_cast<uint32_t*>(ob2 + (long long)row_b * d + n * 8 + 2 * q) = pack_bf16x2(o[n][2] * inv_b, o[n][3] * inv_b);
     }
-    if (q == 0) lse[((long long)b * H + h) * S + row_b] = (l_b > 0.f) ? (m_b * scale_log2 + log2f(l_b)) * kLn2 : INFINITY;
+    if (q == 0) lse[(VARLEN ? sq.stat0 : ((long long)b * H + h) * S) + row_b] = (l_b > 0.f) ? (m_b * scale_log2 + log2f(l_b)) * kLn2 : INFINITY;
   }
 }
 
@@ -258,12 +311,13 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_fwd_kernel(const bf16* __res
 // then the dK/dV kernel.  No atomics: each kernel owns its output rows and recomputes P.
 // ---------------------------------------------------------------------------------------------
 // With dropout:  O = (P o M) V  (M = mask * 1/(1-p)),  dP = (dO V^T) o M,  dS = P o (dP - delta),  delta = rowsum(dO o O).
-template <int DH, bool DROP>
+template <int DH, bool DROP, bool VARLEN>
 __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ out,
                                                                   const bf16* __restrict__ dout, const float* __restrict__ lse,
                                                                   float* __restrict__ delta, const int32_t* __restrict__ first_valid,
-                                                                  bf16* __restrict__ dqkv, int S, int S_valid, int H, float scale,
-                                                                  float scale_log2, int out_f16, DropCfg drop) {
+                                                                  const int32_t* __restrict__ cu_seqlens, bf16* __restrict__ dqkv, int S,
+                                                                  int S_valid, int T, int H, float scale, float scale_log2, int out_f16,
+                                                                  DropCfg drop) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   pdl_launch_dependents();
   pdl_wait();
@@ -276,17 +330,19 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __
   float* s_delta = reinterpret_cast<float*>(smem_raw + 7 * Tile<DH>::BYTES);
 
   const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * ATT_BLK;
+  const AttnSeq sq = attn_seq<VARLEN>(b, h, H, S, S_valid, T, first_valid, cu_seqlens);
+  if (VARLEN && q0 >= sq.end) return;
   const int d = H * DH;
   const long long pitch = 3LL * d;
-  const bf16* base = qkv + (long long)b * S * pitch;
-  const bf16* dob = dout + (long long)b * S * d + h * DH;
-  const bf16* ob = out + (long long)b * S * d + h * DH;
-  const int lo = first_valid[b];
+  const bf16* base = qkv + sq.row0 * pitch;
+  const bf16* dob = dout + sq.row0 * d + h * DH;
+  const bf16* ob = out + sq.row0 * d + h * DH;
+  const int lo = sq.lo;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, q = lane & 3;
   const int row_a = q0 + warp * 16 + g, row_b = row_a + 8;
-  const int q_hi = min(q0 + ATT_BLK, S_valid);
+  const int q_hi = min(q0 + ATT_BLK, sq.valid);
   const float kLog2e = 1.4426950408889634f;
-  float* delta_b = delta + ((long long)b * H + h) * S;
+  float* delta_b = delta + sq.stat0;
 
   float dq[DH / 8][4];
 #pragma unroll
@@ -295,31 +351,31 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __
   uint32_t rk_a = 0u, rk_b = 0u;
   if (DROP) {
     const uint32_t dkey = drop_key(drop);
-    rk_a = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + row_a));
-    rk_b = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + row_b));
+    rk_a = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + sq.doff + row_a));
+    rk_b = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + sq.doff + row_b));
   }
   const bool live = (q_hi > lo) && (q_hi > q0);
   if (!live) {
     // delta of dead rows is never read with a non-zero P, but keep the buffer defined
-    if (threadIdx.x < ATT_BLK && q0 + threadIdx.x < S) delta_b[q0 + threadIdx.x] = 0.f;
+    if (threadIdx.x < ATT_BLK && q0 + threadIdx.x < sq.end) delta_b[q0 + threadIdx.x] = 0.f;
   } else {
-    const float* lse_b = lse + ((long long)b * H + h) * S;
+    const float* lse_b = lse + sq.stat0;
     const int j_begin = (lo / ATT_BLK) * ATT_BLK;
-    load_tile_async<DH>(sQ, base + h * DH, pitch, q0, S);
-    load_tile_async<DH>(sdO, dob, d, q0, S);
-    load_tile_async<DH>(sO, ob, d, q0, S);
-    load_tile_async<DH>(sK(0), base + d + h * DH, pitch, j_begin, S);
-    load_tile_async<DH>(sV(0), base + 2 * d + h * DH, pitch, j_begin, S);
+    load_tile_async<DH>(sQ, base + h * DH, pitch, q0, sq.end);
+    load_tile_async<DH>(sdO, dob, d, q0, sq.end);
+    load_tile_async<DH>(sO, ob, d, q0, sq.end);
+    load_tile_async<DH>(sK(0), base + d + h * DH, pitch, j_begin, sq.end);
+    load_tile_async<DH>(sV(0), base + 2 * d + h * DH, pitch, j_begin, sq.end);
     cp_async_commit();
-    const float lse_a = (row_a < S) ? lse_b[row_a] * kLog2e : INFINITY, lse_bb = (row_b < S) ? lse_b[row_b] * kLog2e : INFINITY;
+    const float lse_a = (row_a < sq.end) ? lse_b[row_a] * kLog2e : INFINITY, lse_bb = (row_b < sq.end) ? lse_b[row_b] * kLog2e : INFINITY;
     uint32_t qa[DH / 16][4], doa[DH / 16][4];
     float del_a = 0.f, del_b = 0.f;
     int buf = 0;
     for (int j0 = j_begin; j0 < q_hi; j0 += ATT_BLK, buf ^= 1) {
       const bool more = (j0 + ATT_BLK) < q_hi;
       if (more) {
-        load_tile_async<DH>(sK(buf ^ 1), base + d + h * DH, pitch, j0 + ATT_BLK, S);
-        load_tile_async<DH>(sV(buf ^ 1), base + 2 * d + h * DH, pitch, j0 + ATT_BLK, S);
+        load_tile_async<DH>(sK(buf ^ 1), base + d + h * DH, pitch, j0 + ATT_BLK, sq.end);
+        load_tile_async<DH>(sV(buf ^ 1), base + 2 * d + h * DH, pitch, j0 + ATT_BLK, sq.end);
         cp_async_commit();
         cp_async_wait<1>();
       } else {
@@ -343,7 +399,7 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __
           acc += __shfl_xor_sync(0xffffffffu, acc, 1);
           if (half == 0) {
             s_delta[r] = acc;
-            if (q0 + r < S) delta_b[q0 + r] = acc;
+            if (q0 + r < sq.end) delta_b[q0 + r] = acc;
           }
         }
 #pragma unroll
@@ -380,19 +436,27 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __
         float p2 = ex2_ftz(fmaf(s[n][2], scale_log2, -lse_bb)), p3 = ex2_ftz(fmaf(s[n][3], scale_log2, -lse_bb));
         if (need_mask) {
           const int key = j0 + n * 8 + 2 * q;
-          const bool va = row_a < S_valid, vb = row_b < S_valid;
+          const bool va = row_a < sq.valid, vb = row_b < sq.valid;
           if (!(va && key >= lo && key <= row_a)) p0 = 0.f;
           if (!(va && key + 1 >= lo && key + 1 <= row_a)) p1 = 0.f;
           if (!(vb && key >= lo && key <= row_b)) p2 = 0.f;
           if (!(vb && key + 1 >= lo && key + 1 <= row_b)) p3 = 0.f;
         }
         if (DROP) {
-          const uint32_t pr = (uint32_t)((j0 + n * 8) >> 1) + q;
           float m0, m1;
-          drop_pair(rk_a, pr, drop.thr16, drop.scale, m0, m1);
-          dp[n][0] *= m0; dp[n][1] *= m1;
-          drop_pair(rk_b, pr, drop.thr16, drop.scale, m0, m1);
-          dp[n][2] *= m0; dp[n][3] *= m1;
+          if (VARLEN) {
+            const int col = sq.doff + j0 + n * 8 + 2 * q;
+            drop_cols(rk_a, col, drop.thr16, drop.scale, m0, m1);
+            dp[n][0] *= m0; dp[n][1] *= m1;
+            drop_cols(rk_b, col, drop.thr16, drop.scale, m0, m1);
+            dp[n][2] *= m0; dp[n][3] *= m1;
+          } else {
+            const uint32_t pr = (uint32_t)((j0 + n * 8) >> 1) + q;
+            drop_pair(rk_a, pr, drop.thr16, drop.scale, m0, m1);
+            dp[n][0] *= m0; dp[n][1] *= m1;
+            drop_pair(rk_b, pr, drop.thr16, drop.scale, m0, m1);
+            dp[n][2] *= m0; dp[n][3] *= m1;
+          }
         }
         s[n][0] = p0 * (dp[n][0] - del_a) * scale;
         s[n][1] = p1 * (dp[n][1] - del_a) * scale;
@@ -418,13 +482,13 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __
       __syncthreads();
     }
   }
-  bf16* dqb = dqkv + (long long)b * S * pitch + h * DH;
-  if (row_a < S) {
+  bf16* dqb = dqkv + sq.row0 * pitch + h * DH;
+  if (row_a < sq.end) {
 #pragma unroll
     for (int n = 0; n < DH / 8; ++n)
       *reinterpret_cast<uint32_t*>(dqb + (long long)row_a * pitch + n * 8 + 2 * q) = pack_bf16x2(dq[n][0], dq[n][1]);
   }
-  if (row_b < S) {
+  if (row_b < sq.end) {
 #pragma unroll
     for (int n = 0; n < DH / 8; ++n)
       *reinterpret_cast<uint32_t*>(dqb + (long long)row_b * pitch + n * 8 + 2 * q) = pack_bf16x2(dq[n][2], dq[n][3]);
@@ -432,11 +496,12 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dq_kernel(const bf16* __
 }
 
 // dK, dV: one CTA owns 64 keys (4 warps x 16) of one head and sweeps the query tiles at or below it.
-template <int DH, bool DROP>
+template <int DH, bool DROP, bool VARLEN>
 __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dkv_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ dout,
                                                                    const float* __restrict__ lse, const float* __restrict__ delta,
-                                                                   const int32_t* __restrict__ first_valid, bf16* __restrict__ dqkv,
-                                                                   int S, int S_valid, int H, float scale, float scale_log2, DropCfg drop) {
+                                                                   const int32_t* __restrict__ first_valid,
+                                                                   const int32_t* __restrict__ cu_seqlens, bf16* __restrict__ dqkv, int S,
+                                                                   int S_valid, int T, int H, float scale, float scale_log2, DropCfg drop) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   pdl_launch_dependents();
   pdl_wait();
@@ -450,13 +515,15 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dkv_kernel(const bf16* _
   uint32_t* s_rk = reinterpret_cast<uint32_t*>(s_delta + 2 * ATT_BLK);       // [2][64] dropout row keys of the query tile
 
   const int b = blockIdx.z, h = blockIdx.y, j0 = blockIdx.x * ATT_BLK;
+  const AttnSeq sq = attn_seq<VARLEN>(b, h, H, S, S_valid, T, first_valid, cu_seqlens);
+  if (VARLEN && j0 >= sq.end) return;
   const int d = H * DH;
   const long long pitch = 3LL * d;
-  const bf16* base = qkv + (long long)b * S * pitch;
-  const bf16* dob = dout + (long long)b * S * d + h * DH;
-  const float* lse_b = lse + ((long long)b * H + h) * S;
-  const float* delta_b = delta + ((long long)b * H + h) * S;
-  const int lo = first_valid[b];
+  const bf16* base = qkv + sq.row0 * pitch;
+  const bf16* dob = dout + sq.row0 * d + h * DH;
+  const float* lse_b = lse + sq.stat0;
+  const float* delta_b = delta + sq.stat0;
+  const int lo = sq.lo;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, q = lane & 3;
   const int key_a = j0 + warp * 16 + g, key_b = key_a + 8;
   const float kLog2e = 1.4426950408889634f;
@@ -467,27 +534,27 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dkv_kernel(const bf16* _
     dk[n][0] = dk[n][1] = dk[n][2] = dk[n][3] = 0.f;
     dv[n][0] = dv[n][1] = dv[n][2] = dv[n][3] = 0.f;
   }
-  const bool live = (j0 + ATT_BLK > lo) && (j0 < S_valid);
+  const bool live = (j0 + ATT_BLK > lo) && (j0 < sq.valid);
   const uint32_t dkey = DROP ? drop_key(drop) : 0u;
   if (live) {
     auto load_q_tile = [&](int bufi, int i0) {
-      load_tile_async<DH>(sQ(bufi), base + h * DH, pitch, i0, S);
-      load_tile_async<DH>(sdO(bufi), dob, d, i0, S);
+      load_tile_async<DH>(sQ(bufi), base + h * DH, pitch, i0, sq.end);
+      load_tile_async<DH>(sdO(bufi), dob, d, i0, sq.end);
       if (threadIdx.x < ATT_BLK) {
         const int i = i0 + threadIdx.x;
-        s_lse[bufi * ATT_BLK + threadIdx.x] = (i < S) ? lse_b[i] * kLog2e : INFINITY;
-        s_delta[bufi * ATT_BLK + threadIdx.x] = (i < S) ? delta_b[i] : 0.f;
-        if (DROP) s_rk[bufi * ATT_BLK + threadIdx.x] = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + i));
+        s_lse[bufi * ATT_BLK + threadIdx.x] = (i < sq.end) ? lse_b[i] * kLog2e : INFINITY;
+        s_delta[bufi * ATT_BLK + threadIdx.x] = (i < sq.end) ? delta_b[i] : 0.f;
+        if (DROP) s_rk[bufi * ATT_BLK + threadIdx.x] = drop_rowkey(dkey, (uint32_t)((b * H + h) * S + sq.doff + i));
       }
     };
-    load_tile_async<DH>(sK, base + d + h * DH, pitch, j0, S);
-    load_tile_async<DH>(sV, base + 2 * d + h * DH, pitch, j0, S);
+    load_tile_async<DH>(sK, base + d + h * DH, pitch, j0, sq.end);
+    load_tile_async<DH>(sV, base + 2 * d + h * DH, pitch, j0, sq.end);
     load_q_tile(0, j0);
     cp_async_commit();
     uint32_t ka[DH / 16][4], va[DH / 16][4];
     int buf = 0;
-    for (int i0 = j0; i0 < S_valid; i0 += ATT_BLK, buf ^= 1) {
-      const bool more = (i0 + ATT_BLK) < S_valid;
+    for (int i0 = j0; i0 < sq.valid; i0 += ATT_BLK, buf ^= 1) {
+      const bool more = (i0 + ATT_BLK) < sq.valid;
       if (more) {
         load_q_tile(buf ^ 1, i0 + ATT_BLK);
         cp_async_commit();
@@ -532,17 +599,18 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dkv_kernel(const bf16* _
         float p00 = ex2_ftz(fmaf(st[n][0], scale_log2, -l0)), p01 = ex2_ftz(fmaf(st[n][1], scale_log2, -l1));
         float p10 = ex2_ftz(fmaf(st[n][2], scale_log2, -l0)), p11 = ex2_ftz(fmaf(st[n][3], scale_log2, -l1));
         if (need_mask) {   // diagonal tile, left padding inside the key tile, or right padding inside the query tile
-          if (!((key_a >= lo) && (key_a <= qi0) && (qi0 < S_valid))) p00 = 0.f;
-          if (!((key_a >= lo) && (key_a <= qi1) && (qi1 < S_valid))) p01 = 0.f;
-          if (!((key_b >= lo) && (key_b <= qi0) && (qi0 < S_valid))) p10 = 0.f;
-          if (!((key_b >= lo) && (key_b <= qi1) && (qi1 < S_valid))) p11 = 0.f;
+          if (!((key_a >= lo) && (key_a <= qi0) && (qi0 < sq.valid))) p00 = 0.f;
+          if (!((key_a >= lo) && (key_a <= qi1) && (qi1 < sq.valid))) p01 = 0.f;
+          if (!((key_b >= lo) && (key_b <= qi0) && (qi0 < sq.valid))) p10 = 0.f;
+          if (!((key_b >= lo) && (key_b <= qi1) && (qi1 < sq.valid))) p11 = 0.f;
         }
         const float d0 = dlp[c0], d1 = dlp[c0 + 1];
         float m00 = 1.f, m01 = 1.f, m10 = 1.f, m11 = 1.f;
-        if (DROP) {  // element (query, key): bits of key pair (key >> 1), half-word key & 1
+        if (DROP) {  // element (query, key): bits of column pair (col >> 1), half-word col & 1
           const uint32_t r0 = s_rk[buf * ATT_BLK + c0], r1 = s_rk[buf * ATT_BLK + c0 + 1];
-          const uint32_t sh = (uint32_t)(key_a & 1) << 4;   // key_b = key_a + 8 has the same parity
-          const uint32_t pa_ = (uint32_t)key_a >> 1, pb_ = (uint32_t)key_b >> 1;
+          const int col_a = sq.doff + key_a, col_b = col_a + 8;
+          const uint32_t sh = (uint32_t)(col_a & 1) << 4;   // col_b = col_a + 8 has the same parity
+          const uint32_t pa_ = (uint32_t)col_a >> 1, pb_ = (uint32_t)col_b >> 1;
           m00 = ((drop_bits(r0, pa_) >> sh) & 0xffffu) >= drop.thr16 ? drop.scale : 0.f;
           m01 = ((drop_bits(r1, pa_) >> sh) & 0xffffu) >= drop.thr16 ? drop.scale : 0.f;
           m10 = ((drop_bits(r0, pb_) >> sh) & 0xffffu) >= drop.thr16 ? drop.scale : 0.f;
@@ -580,16 +648,16 @@ __global__ void __launch_bounds__(ATT_THREADS) attn_bwd_dkv_kernel(const bf16* _
       __syncthreads();
     }
   }
-  bf16* dkb = dqkv + (long long)b * S * pitch + d + h * DH;
-  bf16* dvb = dqkv + (long long)b * S * pitch + 2 * d + h * DH;
-  if (key_a < S) {
+  bf16* dkb = dqkv + sq.row0 * pitch + d + h * DH;
+  bf16* dvb = dqkv + sq.row0 * pitch + 2 * d + h * DH;
+  if (key_a < sq.end) {
 #pragma unroll
     for (int n = 0; n < DH / 8; ++n) {
       *reinterpret_cast<uint32_t*>(dkb + (long long)key_a * pitch + n * 8 + 2 * q) = pack_bf16x2(dk[n][0], dk[n][1]);
       *reinterpret_cast<uint32_t*>(dvb + (long long)key_a * pitch + n * 8 + 2 * q) = pack_bf16x2(dv[n][0], dv[n][1]);
     }
   }
-  if (key_b < S) {
+  if (key_b < sq.end) {
 #pragma unroll
     for (int n = 0; n < DH / 8; ++n) {
       *reinterpret_cast<uint32_t*>(dkb + (long long)key_b * pitch + n * 8 + 2 * q) = pack_bf16x2(dk[n][2], dk[n][3]);
@@ -605,33 +673,37 @@ static size_t dq_smem() { return 7 * (size_t)Tile<DH>::BYTES + ATT_BLK * sizeof(
 template <int DH>
 static size_t dkv_smem() { return 6 * (size_t)Tile<DH>::BYTES + 6 * ATT_BLK * sizeof(float); }
 
-template <int DH, bool DROP>
-static int launch_fwd(const bf16* qkv, const int32_t* fv, bf16* out, bf16* out2, float* lse, int B, int S, int S_valid, int H, int out_f16,
-                      DropCfg drop, cudaStream_t st) {
+// VARLEN: S = the padded width (dropout coordinates), S_grid = the longest sample, T = packed rows; padded: S_grid = S, T unused
+template <int DH, bool DROP, bool VARLEN>
+static int launch_fwd(const bf16* qkv, const int32_t* fv, const int32_t* cu, bf16* out, bf16* out2, float* lse, int B, int S, int S_valid,
+                      int S_grid, int T, int H, int out_f16, DropCfg drop, cudaStream_t st) {
   const size_t smem = fwd_smem<DH>();
-  cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<DH, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<DH, DROP, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(attn_fwd)");
   const float scale_log2 = 1.4426950408889634f / sqrtf((float)DH);
-  dim3 grid((S + ATT_BLK - 1) / ATT_BLK, H, B);
-  launch_pdl(attn_fwd_kernel<DH, DROP>, grid, dim3(ATT_THREADS), smem, st, qkv, fv, out, out2, lse, S, S_valid, H, scale_log2, out_f16, drop);
+  dim3 grid((S_grid + ATT_BLK - 1) / ATT_BLK, H, B);
+  launch_pdl(attn_fwd_kernel<DH, DROP, VARLEN>, grid, dim3(ATT_THREADS), smem, st, qkv, fv, out, out2, lse, S, S_valid, H, scale_log2, out_f16,
+             drop, cu, T);
   NEKO_LAUNCH_CHECK("attn_fwd_kernel");
   return NEKO_OK;
 }
 
-template <int DH, bool DROP>
-static int launch_bwd(const bf16* qkv, const bf16* out, const bf16* dout, const float* lse, float* delta, const int32_t* fv, bf16* dqkv,
-                      int B, int S, int S_valid, int H, int out_f16, DropCfg drop, cudaStream_t st) {
+template <int DH, bool DROP, bool VARLEN>
+static int launch_bwd(const bf16* qkv, const bf16* out, const bf16* dout, const float* lse, float* delta, const int32_t* fv, const int32_t* cu,
+                      bf16* dqkv, int B, int S, int S_valid, int S_grid, int T, int H, int out_f16, DropCfg drop, cudaStream_t st) {
   const size_t s1 = dq_smem<DH>(), s2 = dkv_smem<DH>();
-  cudaError_t e = cudaFuncSetAttribute(attn_bwd_dq_kernel<DH, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s1);
+  cudaError_t e = cudaFuncSetAttribute(attn_bwd_dq_kernel<DH, DROP, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s1);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(attn_bwd_dq)");
-  e = cudaFuncSetAttribute(attn_bwd_dkv_kernel<DH, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s2);
+  e = cudaFuncSetAttribute(attn_bwd_dkv_kernel<DH, DROP, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s2);
   if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(attn_bwd_dkv)");
   const float scale = 1.0f / sqrtf((float)DH);
   const float scale_log2 = 1.4426950408889634f * scale;
-  dim3 grid((S + ATT_BLK - 1) / ATT_BLK, H, B);
-  launch_pdl(attn_bwd_dq_kernel<DH, DROP>, grid, dim3(ATT_THREADS), s1, st, qkv, out, dout, lse, delta, fv, dqkv, S, S_valid, H, scale, scale_log2, out_f16, drop);
+  dim3 grid((S_grid + ATT_BLK - 1) / ATT_BLK, H, B);
+  launch_pdl(attn_bwd_dq_kernel<DH, DROP, VARLEN>, grid, dim3(ATT_THREADS), s1, st, qkv, out, dout, lse, delta, fv, cu, dqkv, S, S_valid, T, H,
+             scale, scale_log2, out_f16, drop);
   NEKO_LAUNCH_CHECK("attn_bwd_dq_kernel");
-  launch_pdl(attn_bwd_dkv_kernel<DH, DROP>, grid, dim3(ATT_THREADS), s2, st, qkv, dout, lse, delta, fv, dqkv, S, S_valid, H, scale, scale_log2, drop);
+  launch_pdl(attn_bwd_dkv_kernel<DH, DROP, VARLEN>, grid, dim3(ATT_THREADS), s2, st, qkv, dout, lse, delta, fv, cu, dqkv, S, S_valid, T, H,
+             scale, scale_log2, drop);
   NEKO_LAUNCH_CHECK("attn_bwd_dkv_kernel");
   return NEKO_OK;
 }
@@ -715,8 +787,8 @@ int neko_attention_fwd(const uint16_t* qkv, const int32_t* first_valid, uint16_t
     const int rc_tc = attention_fwd_tc(x, first_valid, o, o2, lse, B, S, S_valid, H, dh, out_f16, dc, st);
     if (rc_tc <= 0) return rc_tc;
   }
-#define NEKO_ATT_FWD(DH_) (dc.seed ? launch_fwd<DH_, true>(x, first_valid, o, o2, lse, B, S, S_valid, H, out_f16, dc, st) \
-                                   : launch_fwd<DH_, false>(x, first_valid, o, o2, lse, B, S, S_valid, H, out_f16, dc, st))
+#define NEKO_ATT_FWD(DH_) (dc.seed ? launch_fwd<DH_, true, false>(x, first_valid, nullptr, o, o2, lse, B, S, S_valid, S, 0, H, out_f16, dc, st) \
+                                   : launch_fwd<DH_, false, false>(x, first_valid, nullptr, o, o2, lse, B, S, S_valid, S, 0, H, out_f16, dc, st))
   switch (dh) {
     case 16: return NEKO_ATT_FWD(16);
     case 32: return NEKO_ATT_FWD(32);
@@ -754,8 +826,60 @@ int neko_attention_bwd(const uint16_t* qkv, const uint16_t* out, const uint16_t*
   const bf16* g = reinterpret_cast<const bf16*>(dout);
   bf16* dx = reinterpret_cast<bf16*>(dqkv);
   const DropCfg dc = drop_cfg(drop);
-#define NEKO_ATT_BWD(DH_) (dc.seed ? launch_bwd<DH_, true>(x, o, g, lse, delta, first_valid, dx, B, S, S_valid, H, out_f16, dc, st) \
-                                   : launch_bwd<DH_, false>(x, o, g, lse, delta, first_valid, dx, B, S, S_valid, H, out_f16, dc, st))
+#define NEKO_ATT_BWD(DH_) (dc.seed ? launch_bwd<DH_, true, false>(x, o, g, lse, delta, first_valid, nullptr, dx, B, S, S_valid, S, 0, H, out_f16, dc, st) \
+                                   : launch_bwd<DH_, false, false>(x, o, g, lse, delta, first_valid, nullptr, dx, B, S, S_valid, S, 0, H, out_f16, dc, st))
+  switch (dh) {
+    case 16: return NEKO_ATT_BWD(16);
+    case 32: return NEKO_ATT_BWD(32);
+    case 64: return NEKO_ATT_BWD(64);
+    case 128: return NEKO_ATT_BWD(128);
+    default: set_error("attention: head dim %d not supported (16, 32, 64, 128)", dh); return NEKO_EINVAL;
+  }
+#undef NEKO_ATT_BWD
+}
+
+int neko_attention_varlen_fwd(const uint16_t* qkv, const int32_t* cu_seqlens, const int32_t* first_valid, uint16_t* out, uint16_t* out2_bf16,
+                              float* lse, int B, int T, int S_max, int S_width, int H, int dh, int out_f16, const neko_dropout* drop,
+                              void* stream) {
+  using namespace neko;
+  NEKO_REQUIRE(qkv && cu_seqlens && first_valid && out && lse, "attention_varlen_fwd: null pointer");
+  NEKO_REQUIRE(B > 0 && T > 0 && H > 0 && S_max > 0 && S_max <= S_width, "attention_varlen_fwd: bad sizes");
+  NEKO_REQUIRE((reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, "attention_varlen_fwd: misaligned");
+  NEKO_REQUIRE((long long)B * H * S_width < (1LL << 32), "attention_varlen_fwd: B*H*S_width exceeds the dropout row-id range");
+  const bf16* x = reinterpret_cast<const bf16*>(qkv);
+  bf16* o = reinterpret_cast<bf16*>(out);
+  bf16* o2 = reinterpret_cast<bf16*>(out2_bf16);
+  cudaStream_t st = as_stream(stream);
+  const DropCfg dc = drop_cfg(drop);
+#define NEKO_ATT_FWD(DH_) (dc.seed ? launch_fwd<DH_, true, true>(x, first_valid, cu_seqlens, o, o2, lse, B, S_width, S_max, S_max, T, H, out_f16, dc, st) \
+                                   : launch_fwd<DH_, false, true>(x, first_valid, cu_seqlens, o, o2, lse, B, S_width, S_max, S_max, T, H, out_f16, dc, st))
+  switch (dh) {
+    case 16: return NEKO_ATT_FWD(16);
+    case 32: return NEKO_ATT_FWD(32);
+    case 64: return NEKO_ATT_FWD(64);
+    case 128: return NEKO_ATT_FWD(128);
+    default: set_error("attention: head dim %d not supported (16, 32, 64, 128)", dh); return NEKO_EINVAL;
+  }
+#undef NEKO_ATT_FWD
+}
+
+int neko_attention_varlen_bwd(const uint16_t* qkv, const uint16_t* out, const uint16_t* dout, const float* lse, const int32_t* cu_seqlens,
+                              const int32_t* first_valid, uint16_t* dqkv, float* delta, int B, int T, int S_max, int S_width, int H, int dh,
+                              int out_f16, const neko_dropout* drop, void* stream) {
+  using namespace neko;
+  NEKO_REQUIRE(qkv && out && dout && lse && cu_seqlens && first_valid && dqkv && delta, "attention_varlen_bwd: null pointer");
+  NEKO_REQUIRE(B > 0 && T > 0 && H > 0 && S_max > 0 && S_max <= S_width, "attention_varlen_bwd: bad sizes");
+  NEKO_REQUIRE((reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(dout) & 15) == 0, "attention_varlen_bwd: misaligned");
+  NEKO_REQUIRE((long long)B * H * S_width < (1LL << 32), "attention_varlen_bwd: B*H*S_width exceeds the dropout row-id range");
+  cudaStream_t st = as_stream(stream);
+  const bf16* x = reinterpret_cast<const bf16*>(qkv);
+  const bf16* o = reinterpret_cast<const bf16*>(out);
+  const bf16* g = reinterpret_cast<const bf16*>(dout);
+  bf16* dx = reinterpret_cast<bf16*>(dqkv);
+  const DropCfg dc = drop_cfg(drop);
+#define NEKO_ATT_BWD(DH_) (dc.seed ? launch_bwd<DH_, true, true>(x, o, g, lse, delta, first_valid, cu_seqlens, dx, B, S_width, S_max, S_max, T, H, out_f16, dc, st) \
+                                   : launch_bwd<DH_, false, true>(x, o, g, lse, delta, first_valid, cu_seqlens, dx, B, S_width, S_max, S_max, T, H, out_f16, dc, st))
   switch (dh) {
     case 16: return NEKO_ATT_BWD(16);
     case 32: return NEKO_ATT_BWD(32);

@@ -117,26 +117,31 @@ __device__ __forceinline__ long long slot_token(const TokArgs& a, const neko_sam
   return id;
 }
 
+// PACKED: warps still walk (b, s) of the padded grid (s < seq_len); a valid position writes row row_base + (s - seq_off)
+// of the packed outputs and a padding position writes nothing.
+template <bool PACKED>
 __global__ void __launch_bounds__(256) tokenize_embed_kernel(TokArgs a) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  const int width = a.p.width;
+  const int width = PACKED ? a.p.seq_len : a.p.width;
   if (warp >= a.B * width) return;
   const int b = warp / width;
   const int s = warp - b * width;
   const neko_sample_desc sd = a.descs[b];
   const SlotInfo si = locate(sd, s, a.p.seq_len);
+  if (PACKED && si.kind == SLOT_PAD) return;
+  const int row = PACKED ? sd.row_base + (s - sd.seq_off) : warp;
   float tgt;
   const long long id = slot_token(a, sd, si, &tgt);
   if (lane == 0) {
-    a.tokens[warp] = id;
-    a.target_masks[warp] = tgt;
-    a.token_masks[warp] = (si.kind == SLOT_PAD) ? 0.0f : 1.0f;
+    a.tokens[row] = id;
+    a.target_masks[row] = tgt;
+    a.token_masks[row] = (si.kind == SLOT_PAD) ? 0.0f : 1.0f;
   }
   if (a.emb == nullptr) return;
 
   const int d = a.d;
-  float4* out = reinterpret_cast<float4*>(a.emb + (size_t)warp * d);
+  float4* out = reinterpret_cast<float4*>(a.emb + (size_t)row * d);
   const int nv = d >> 2;
   if (si.kind == SLOT_PAD) {
     for (int i = lane; i < nv; i += 32) out[i] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -183,18 +188,20 @@ struct EmbBwdArgs {
   float* d_patch_emb;
 };
 
+template <bool PACKED>
 __global__ void __launch_bounds__(256) embed_bwd_kernel(EmbBwdArgs a) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  const int width = a.p.width;
+  const int width = PACKED ? a.p.seq_len : a.p.width;
   if (warp >= a.B * width) return;
   const int b = warp / width;
   const int s = warp - b * width;
   const neko_sample_desc sd = a.descs[b];
   const SlotInfo si = locate(sd, s, a.p.seq_len);
   if (si.kind == SLOT_PAD) return;
+  const int row = PACKED ? sd.row_base + (s - sd.seq_off) : warp;
   const int d = a.d;
-  const float* g = a.d_emb + (size_t)warp * d;
+  const float* g = a.d_emb + (size_t)row * d;
   float* dst = nullptr;
   bool atomic = true;
   if (si.kind == SLOT_PATCH) {
@@ -205,7 +212,7 @@ __global__ void __launch_bounds__(256) embed_bwd_kernel(EmbBwdArgs a) {
   } else if (si.kind == SLOT_SEP) {
     dst = a.d_sep;
   } else {
-    const long long id = a.tokens[warp];
+    const long long id = a.tokens[row];
     if (id >= 0 && id < a.p.vocab) dst = a.d_embed_table + (size_t)id * d;
   }
   const bool add_pos = a.p.use_pos && si.kind >= SLOT_PATCH && si.kind <= SLOT_DOBS;
@@ -219,16 +226,11 @@ __global__ void __launch_bounds__(256) embed_bwd_kernel(EmbBwdArgs a) {
   }
 }
 
-}  // namespace neko
-
-extern "C" {
-
-int neko_tokenize_embed_fwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
-                            const float* fvals, const int32_t* ivals, const float* patch_emb,
-                            const float* embed_table, const float* pos_table, const float* sep_vec,
-                            int64_t* tokens, float* target_masks, float* token_masks,
-                            float* token_embeddings, int32_t* err_flag, void* stream) {
-  using namespace neko;
+template <bool PACKED>
+static int tokenize_embed(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp, const float* fvals,
+                          const int32_t* ivals, const float* patch_emb, const float* embed_table, const float* pos_table,
+                          const float* sep_vec, int64_t* tokens, float* target_masks, float* token_masks,
+                          float* token_embeddings, int32_t* err_flag, void* stream) {
   NEKO_REQUIRE(descs && hp && tokens && target_masks && token_masks, "tokenize: null pointer");
   NEKO_REQUIRE(B > 0 && hp->width >= hp->seq_len && hp->seq_len > 0, "tokenize: bad B/seq_len/width");
   if (token_embeddings) {
@@ -241,29 +243,63 @@ int neko_tokenize_embed_fwd(const neko_sample_desc* descs, int B, int d, const n
   a.fvals = fvals; a.ivals = ivals; a.patch_emb = patch_emb; a.embed_table = embed_table;
   a.pos_table = pos_table; a.sep_vec = sep_vec; a.tokens = tokens; a.target_masks = target_masks;
   a.token_masks = token_masks; a.emb = token_embeddings; a.err_flag = err_flag;
-  const long long warps = (long long)B * hp->width;
+  const long long warps = (long long)B * (PACKED ? hp->seq_len : hp->width);
   const int threads = 256;
   const long long blocks = (warps * 32 + threads - 1) / threads;
-  tokenize_embed_kernel<<<(unsigned)blocks, threads, 0, as_stream(stream)>>>(a);
+  tokenize_embed_kernel<PACKED><<<(unsigned)blocks, threads, 0, as_stream(stream)>>>(a);
   NEKO_LAUNCH_CHECK("tokenize_embed_kernel");
   return NEKO_OK;
 }
 
-int neko_embed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
-                   const int64_t* tokens, const float* d_token_embeddings, float* d_embed_table,
-                   float* d_pos_table, float* d_sep, float* d_patch_emb, void* stream) {
-  using namespace neko;
+template <bool PACKED>
+static int embed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp, const int64_t* tokens,
+                     const float* d_token_embeddings, float* d_embed_table, float* d_pos_table, float* d_sep,
+                     float* d_patch_emb, void* stream) {
   NEKO_REQUIRE(descs && hp && tokens && d_token_embeddings && d_embed_table && d_sep, "embed_bwd: null pointer");
   NEKO_REQUIRE(d_pos_table || !hp->use_pos, "embed_bwd: null d_pos_table");
   EmbBwdArgs a;
   a.descs = descs; a.B = B; a.d = d; a.p = *hp; a.tokens = tokens; a.d_emb = d_token_embeddings;
   a.d_embed_table = d_embed_table; a.d_pos_table = d_pos_table; a.d_sep = d_sep; a.d_patch_emb = d_patch_emb;
-  const long long warps = (long long)B * hp->width;
+  const long long warps = (long long)B * (PACKED ? hp->seq_len : hp->width);
   const int threads = 256;
   const long long blocks = (warps * 32 + threads - 1) / threads;
-  embed_bwd_kernel<<<(unsigned)blocks, threads, 0, as_stream(stream)>>>(a);
+  embed_bwd_kernel<PACKED><<<(unsigned)blocks, threads, 0, as_stream(stream)>>>(a);
   NEKO_LAUNCH_CHECK("embed_bwd_kernel");
   return NEKO_OK;
+}
+
+}  // namespace neko
+
+extern "C" {
+
+int neko_tokenize_embed_fwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
+                            const float* fvals, const int32_t* ivals, const float* patch_emb,
+                            const float* embed_table, const float* pos_table, const float* sep_vec,
+                            int64_t* tokens, float* target_masks, float* token_masks,
+                            float* token_embeddings, int32_t* err_flag, void* stream) {
+  return neko::tokenize_embed<false>(descs, B, d, hp, fvals, ivals, patch_emb, embed_table, pos_table, sep_vec, tokens,
+                                     target_masks, token_masks, token_embeddings, err_flag, stream);
+}
+
+int neko_tokenize_embed_packed_fwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
+                                   const float* fvals, const int32_t* ivals, const float* patch_emb,
+                                   const float* embed_table, const float* pos_table, const float* sep_vec,
+                                   int64_t* tokens, float* target_masks, float* token_masks,
+                                   float* token_embeddings, int32_t* err_flag, void* stream) {
+  return neko::tokenize_embed<true>(descs, B, d, hp, fvals, ivals, patch_emb, embed_table, pos_table, sep_vec, tokens,
+                                    target_masks, token_masks, token_embeddings, err_flag, stream);
+}
+
+int neko_embed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
+                   const int64_t* tokens, const float* d_token_embeddings, float* d_embed_table,
+                   float* d_pos_table, float* d_sep, float* d_patch_emb, void* stream) {
+  return neko::embed_bwd<false>(descs, B, d, hp, tokens, d_token_embeddings, d_embed_table, d_pos_table, d_sep, d_patch_emb, stream);
+}
+
+int neko_embed_packed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
+                          const int64_t* tokens, const float* d_token_embeddings, float* d_embed_table,
+                          float* d_pos_table, float* d_sep, float* d_patch_emb, void* stream) {
+  return neko::embed_bwd<true>(descs, B, d, hp, tokens, d_token_embeddings, d_embed_table, d_pos_table, d_sep, d_patch_emb, stream);
 }
 
 }  // extern "C"

@@ -158,6 +158,25 @@ def dropout_mask(rows: int, cols: int, drop: Dropout, device) -> torch.Tensor:
 
 
 # ------------------------------------------------------------------------------------------
+# tokenise / embed
+# ------------------------------------------------------------------------------------------
+def tokenize_embed_fwd(descs, B: int, d: int, prm: TokParams, fvals, ivals, patch_emb, embed_table, pos_table, sep_vec,
+                       tokens, target_masks, token_masks, token_embeddings, err_flag=None, packed: bool = False):
+    """Ids, masks and embeddings of a planned batch: [B*width] rows, or the packed [T] rows (no padding) when ``packed``."""
+    fn = load().neko_tokenize_embed_packed_fwd if packed else load().neko_tokenize_embed_fwd
+    check(fn(_p(descs), C.c_int(B), C.c_int(d), C.byref(prm), _p(fvals), _p(ivals), _p(patch_emb), _p(embed_table), _p(pos_table),
+             _p(sep_vec), _p(tokens), _p(target_masks), _p(token_masks), _p(token_embeddings), _p(err_flag), stream_ptr()),
+          "neko_tokenize_embed_packed_fwd" if packed else "neko_tokenize_embed_fwd")
+
+
+def embed_bwd(descs, B: int, d: int, prm: TokParams, tokens, d_emb, d_embed_table, d_pos_table, d_sep, d_patch_emb=None,
+              packed: bool = False):
+    fn = load().neko_embed_packed_bwd if packed else load().neko_embed_bwd
+    check(fn(_p(descs), C.c_int(B), C.c_int(d), C.byref(prm), _p(tokens), _p(d_emb), _p(d_embed_table), _p(d_pos_table), _p(d_sep),
+             _p(d_patch_emb), stream_ptr()), "neko_embed_packed_bwd" if packed else "neko_embed_bwd")
+
+
+# ------------------------------------------------------------------------------------------
 # attention
 # ------------------------------------------------------------------------------------------
 def attention_fwd(qkv: torch.Tensor, first_valid: torch.Tensor, H: int, S_valid: Optional[int] = None, out=None, lse=None,
@@ -193,6 +212,36 @@ def attention_bwd(qkv, out, dout, lse, first_valid, H: int, S_valid: Optional[in
     check(load().neko_attention_bwd(_p(qkv), _p(out), _p(dout), _p(lse), _p(first_valid), _p(dqkv), _p(delta), C.c_int(B),
                                     C.c_int(S), C.c_int(S if S_valid is None else S_valid), C.c_int(H), C.c_int(dh),
                                     C.c_int(int(out.dtype == torch.float16)), _dref(drop), stream_ptr()), "neko_attention_bwd")
+    return dqkv
+
+
+def attention_varlen_fwd(qkv: torch.Tensor, cu_seqlens: torch.Tensor, first_valid: torch.Tensor, H: int, S_max: int, S_width: int,
+                         out=None, lse=None, out_dtype: torch.dtype = torch.bfloat16, out2=None, drop=None):
+    """Packed causal attention: qkv [T, 3d], sample b = rows [cu_seqlens[b], cu_seqlens[b+1]); out [T, d], lse [H, T].
+    S_width / first_valid give the padded layout's dropout coordinates (include/neko_b200.h)."""
+    T, three_d = qkv.shape
+    d = three_d // 3
+    B = cu_seqlens.numel() - 1
+    if out is None:
+        out = torch.empty(T, d, device=qkv.device, dtype=out_dtype)
+    if lse is None:
+        lse = torch.empty(H, T, device=qkv.device, dtype=torch.float32)
+    check(load().neko_attention_varlen_fwd(_p(qkv), _p(cu_seqlens), _p(first_valid), _p(out), _p(out2), _p(lse), C.c_int(B), C.c_int(T),
+                                           C.c_int(S_max), C.c_int(S_width), C.c_int(H), C.c_int(d // H),
+                                           C.c_int(int(out.dtype == torch.float16)), _dref(drop), stream_ptr()), "neko_attention_varlen_fwd")
+    return out, lse
+
+
+def attention_varlen_bwd(qkv, out, dout, lse, cu_seqlens, first_valid, H: int, S_max: int, S_width: int, dqkv=None, delta=None, drop=None):
+    T, three_d = qkv.shape
+    B = cu_seqlens.numel() - 1
+    if dqkv is None:
+        dqkv = torch.empty_like(qkv)
+    if delta is None:
+        delta = torch.empty(H, T, device=qkv.device, dtype=torch.float32)
+    check(load().neko_attention_varlen_bwd(_p(qkv), _p(out), _p(dout), _p(lse), _p(cu_seqlens), _p(first_valid), _p(dqkv), _p(delta),
+                                           C.c_int(B), C.c_int(T), C.c_int(S_max), C.c_int(S_width), C.c_int(H), C.c_int(three_d // 3 // H),
+                                           C.c_int(int(out.dtype == torch.float16)), _dref(drop), stream_ptr()), "neko_attention_varlen_bwd")
     return dqkv
 
 

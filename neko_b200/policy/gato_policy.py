@@ -313,6 +313,12 @@ class GatoPolicy(nn.Module):
         # are exactly zero); 'dense' runs them over every position like the reference's autograd.  Identical gradients.
         self.head_mode = "rows"
         self.materialize_logits = True  # False: head evaluated on loss rows only, forward returns logits=None
+        # pack_sequences (needs materialize_logits = False): forward(inputs, compute_loss=True) and stage() lay the samples out
+        # back to back with no padding rows, so every row-proportional kernel runs on the valid tokens only (variable-length
+        # attention).  Same loss and gradients up to reassociation; pad_seq has no effect on them (right padding is causally
+        # invisible to valid rows).  Opt-in: the embedding / residual dropout masks are drawn at packed row coordinates, a
+        # different random stream from the padded layout's (the attention-dropout masks are the same).
+        self.pack_sequences = False
         self.lean_logits_f16 = True     # ... and, when gradients are wanted, those logits live in fp16 between head GEMM and fused CE
         self.mlp_proj_bf16 = False      # training forward: mlp down-projection on the bf16 activation twin (see _decoder)
         # 16-bit format of the FORWARD operands (activations fed to GEMMs, weight copy).  fp16 has 3 more mantissa
@@ -543,6 +549,7 @@ class GatoPolicy(nn.Module):
                                "descriptors and loss rows -- call loss.backward() first (or run the forward under torch.no_grad())")
         if self._staged_handle is not None and getattr(self._staged_handle, "staged", False):
             raise RuntimeError("stage(): the previously staged batch has not been consumed by forward() yet")
+        self._check_packing(compute_loss)
         st = self._plan(inputs, compute_loss)
         st.staged = True
         self._image_prefetch(st)
@@ -598,6 +605,7 @@ class GatoPolicy(nn.Module):
                     # forward, tokenize_input_dicts, predict_*.  Upload the staged plan again -- same layout, same seed.
                     self._upload_plan(state, state.drop_seed_host)
             else:
+                self._check_packing(compute_loss)
                 self._bwd_pending = False     # a new direct forward supersedes an abandoned step
                 state = self._plan(inputs, compute_loss)
             anchor = None
@@ -633,6 +641,11 @@ class GatoPolicy(nn.Module):
                 pos = torch.arange(B * S, device=self.device).view(B, S)[:, :-1].reshape(-1)[lm].to(torch.int32)
                 loss, _, _ = ops.masked_ce_fwd(full, self.vocab_size, pos, tokens.reshape(-1).contiguous())
         return logits, loss
+
+    def _check_packing(self, compute_loss):
+        if self.pack_sequences and compute_loss and self.materialize_logits:
+            raise ValueError("pack_sequences=True needs materialize_logits=False: the packed layout has no [B, S, V] logits "
+                             "to return (set materialize_logits = False, as the trainer does, or turn pack_sequences off)")
 
     def tokenize_input_dicts(self, inputs: list):
         """gato_policy.py:195-432 -> (token_embeddings fp32 [B,S,d], tokens int64 [B,S], token_target_masks fp32,
@@ -782,7 +795,9 @@ class GatoPolicy(nn.Module):
     # ------------------------------------------------------------------------------------------
     def _plan(self, inputs, compute_loss) -> _State:
         st = _State()
-        plan = build_plan(inputs, patch_size=self.patch_size, context_len=self.context_len, pad_seq=self.pad_seq)
+        # packing applies to loss-computing steps (tokenize_input_dicts, the predict_* loops and evaluation forwards stay padded)
+        packed = bool(self.pack_sequences and compute_loss and not self.materialize_logits)
+        plan = build_plan(inputs, patch_size=self.patch_size, context_len=self.context_len, pad_seq=self.pad_seq, packed=packed)
         st.plan = plan
         st.compute_loss = bool(compute_loss)
         # train-mode patch bins consume the global CPU RNG per image-bearing sample, rows first (embeddings.py:92-95)
@@ -810,12 +825,13 @@ class GatoPolicy(nn.Module):
 
     def _upload_plan(self, st: _State, seed):
         """The batch's single pinned -> device copy (descriptors, scalars, ids, loss rows, dropout seed header)."""
-        descs, fv, iv, first_valid, loss_rows, h2d, hdr = self._stager.upload(st.plan, seed)
+        descs, fv, iv, first_valid, loss_rows, cu_seqlens, h2d, hdr = self._stager.upload(st.plan, seed)
         st.descs, st.fvals, st.ivals, st.first_valid, st.loss_rows = descs, fv, iv, first_valid, loss_rows
+        st.cu_seqlens = cu_seqlens
         st.drop_seed = hdr[:2]
         st.drop_seed_host = seed
         st.stager_gen = self._stager.generation
-        self._last_drop = (st.drop_seed, st.plan.B, st.plan.width)
+        self._last_drop = (st.drop_seed, st.plan)
         st.h2d_bytes += h2d
 
     def _tok_params(self, plan: BatchPlan) -> TokParams:
@@ -931,7 +947,7 @@ class GatoPolicy(nn.Module):
     def _embed(self, st: _State):
         plan = st.plan
         d = self.embed_dim
-        N = plan.B * plan.width
+        N = plan.token_rows
         if not getattr(st, "in_graph", False):   # graph mode: _engine_forward refreshed the copies eagerly, version-checked
             self._refresh_bf16()
         if not getattr(st, "uploaded", False):
@@ -948,10 +964,9 @@ class GatoPolicy(nn.Module):
     def _launch_tokenize(self, st: _State):
         """The tokenise + embed + interleave + pad kernel alone (bench.py times it against the HBM roofline)."""
         plan, d, prm = st.plan, self.embed_dim, st.tok_params
-        check(load().neko_tokenize_embed_fwd(_p(st.descs), C.c_int(plan.B), C.c_int(d), C.byref(prm), _p(st.fvals), _p(st.ivals),
-                                             _p(st.patch_emb), _p(self.embed_token.weight), _p(self.pos_embed_observation.weight),
-                                             _p(self.separator_token), _p(st.tokens), _p(st.tmask), _p(st.mask), _p(st.x0), _p(None),
-                                             stream_ptr()), "neko_tokenize_embed_fwd")
+        ops.tokenize_embed_fwd(st.descs, plan.B, d, prm, st.fvals, st.ivals, st.patch_emb, self.embed_token.weight,
+                               self.pos_embed_observation.weight, self.separator_token, st.tokens, st.tmask, st.mask, st.x0,
+                               packed=plan.packed)
         self.launches += 1
 
     # -- dropout ------------------------------------------------------------------------------------
@@ -980,24 +995,37 @@ class GatoPolicy(nn.Module):
         ps = self._dropout_ps()
         if ps is None or getattr(self, "_last_drop", None) is None:
             return {}
-        seed, B, W = self._last_drop
+        seed, plan = self._last_drop
+        B, W = plan.B, plan.width
         d, H = self.embed_dim, self.heads
 
         def mult(stream, p, rows, cols):
             dr = Dropout.make(seed, stream, p)
             return ops.dropout_mask(rows, cols, dr, self.device).to(torch.float32) * dr.scale
 
+        if plan.packed:   # row masks were drawn at packed rows: scatter packed row row_base[b] + p to (b, first_valid[b] + p)
+            lengths = np.diff(plan.cu_seqlens)
+            dst = np.concatenate([b * W + plan.first_valid[b] + np.arange(lengths[b]) for b in range(B)])
+            dst = torch.from_numpy(dst).to(self.device)
+
+        def row_mult(stream, p):
+            if not plan.packed:
+                return mult(stream, p, B * W, d).view(B, W, d)
+            full = torch.zeros(B * W, d, device=self.device)
+            full[dst] = mult(stream, p, plan.token_rows, d)
+            return full.view(B, W, d)
+
         out = {}
         if ps[0] > 0:
-            out["embd"] = mult(0, ps[0], B * W, d).view(B, W, d)
+            out["embd"] = row_mult(0, ps[0])
         for i in range(self.layers):
             pa, pr, pm = ps[1 + 3 * i:4 + 3 * i]
             if pa > 0:
                 out[("attn", i)] = mult(4 * i + 1, pa, B * H * W, W).view(B, H, W, W)
             if pr > 0:
-                out[("resid_attn", i)] = mult(4 * i + 2, pr, B * W, d).view(B, W, d)
+                out[("resid_attn", i)] = row_mult(4 * i + 2, pr)
             if pm > 0:
-                out[("resid_mlp", i)] = mult(4 * i + 3, pm, B * W, d).view(B, W, d)
+                out[("resid_mlp", i)] = row_mult(4 * i + 3, pm)
         return out
 
     def _drop_site(self, st: _State, stream: int, p: float):
@@ -1010,7 +1038,8 @@ class GatoPolicy(nn.Module):
         """L pre-LN blocks + ln_f (trajectory_gpt2.py:322-358, 779).  x fp32 [N,d] -> hf bf16 [N,d]."""
         gate = bool(self.transformer.config.gate)
         d, H = self.embed_dim, self.heads
-        N = B * W
+        N = x.shape[0]            # B * W, or the T rows of a packed batch
+        packed = getattr(st, "plan", None) is not None and st.plan.packed
         eps = self.transformer.config.layer_norm_epsilon
         fdt = self.fwd_dtype
         dual = keep and fdt != torch.bfloat16   # backward GEMMs need bf16 copies of the saved activations
@@ -1037,9 +1066,12 @@ class GatoPolicy(nn.Module):
             qkv = self._buf("qkv" + tag, (N, 3 * d), torch.bfloat16)
             ops.gemm(ln1, self._wview(pre + "attn.c_attn.weight"), b_mn=True, epilogue=ops.EPI_BF16, out=qkv, bias=blk.attn.c_attn.bias)
             att, att_b = pair("att", tag, (N, d))
-            lse = self._buf("lse" + tag, (B, H, W), torch.float32)
+            lse = self._buf("lse" + tag, (H, N) if packed else (B, H, W), torch.float32)
             kv = getattr(st, "kv", None)
-            if kv is not None and kv.decoding:
+            if packed:
+                ops.attention_varlen_fwd(qkv, st.cu_seqlens, first_valid, H, S_valid, W, att, lse, out2=att_b if dual else None,
+                                         drop=self._drop_site(st, 4 * i + 1, blk.attn.attn_dropout.p))
+            elif kv is not None and kv.decoding:
                 # KV-cached decode: N == 1; append this position's key / value, attend over the cache
                 kv.k[i, kv.len].copy_(qkv[0, d:2 * d])
                 kv.v[i, kv.len].copy_(qkv[0, 2 * d:])
@@ -1140,7 +1172,7 @@ class GatoPolicy(nn.Module):
         p = st.plan
         return (p.B, p.seq_len, p.width, p.descs.tobytes(), tuple((g.height, g.width, g.is_u8, g.n_frames) for g in p.image_groups),
                 len(p.precomputed_patch), st.compute_loss, st.need_grad, self.training, self.materialize_logits, self.head_mode,
-                self.fwd_dtype, st.row_bins is not None, self._dropout_ps(), self.lean_logits_f16, self.mlp_proj_bf16)
+                self.fwd_dtype, st.row_bins is not None, self._dropout_ps(), self.lean_logits_f16, self.mlp_proj_bf16, p.packed)
 
     def _engine_forward(self, st: _State):
         if not self.use_cuda_graphs:
@@ -1198,7 +1230,7 @@ class GatoPolicy(nn.Module):
     def _forward_compute(self, st: _State):
         plan = st.plan
         B, W, d, V = plan.B, plan.width, self.embed_dim, self.vocab_size
-        N = B * W
+        N = plan.token_rows
         self._generation += 1
         st.generation = self._generation
         keep = st.need_grad
@@ -1308,7 +1340,7 @@ class GatoPolicy(nn.Module):
             raise RuntimeError("nothing to differentiate: forward ran with compute_loss=False or selected no loss rows")
         plan = st.plan
         B, W, d, V, Vp, H = plan.B, plan.width, self.embed_dim, self.vocab_size, self._Vp, self.heads
-        N = B * W
+        N = plan.token_rows
         n_rows = st.n_rows
         sync = getattr(self, "_grad_sync", None)
         if sync is not None and getattr(sync, "mode", "overlap") == "tail":
@@ -1420,9 +1452,14 @@ class GatoPolicy(nn.Module):
             datt = self._buf("datt", (N, d), torch.bfloat16)
             ops.gemm(dxb, Wb(pre + "attn.c_proj.weight"), epilogue=ops.EPI_BF16, out=datt)
             dqkv = self._buf("dqkv", (N, 3 * d), torch.bfloat16)
-            delta = self._buf("delta", (B, H, W), torch.float32)
-            ops.attention_bwd(qkv.view(B, W, 3 * d), att.view(B, W, d), datt.view(B, W, d), lse, st.first_valid, H, plan.seq_len,
-                              dqkv.view(B, W, 3 * d), delta, drop=D(4 * i + 1, blk.attn.attn_dropout.p))
+            if plan.packed:
+                delta = self._buf("delta", (H, N), torch.float32)
+                ops.attention_varlen_bwd(qkv, att, datt, lse, st.cu_seqlens, st.first_valid, H, plan.seq_len, W, dqkv, delta,
+                                         drop=D(4 * i + 1, blk.attn.attn_dropout.p))
+            else:
+                delta = self._buf("delta", (B, H, W), torch.float32)
+                ops.attention_bwd(qkv.view(B, W, 3 * d), att.view(B, W, d), datt.view(B, W, d), lse, st.first_valid, H, plan.seq_len,
+                                  dqkv.view(B, W, 3 * d), delta, drop=D(4 * i + 1, blk.attn.attn_dropout.p))
             ops.gemm(ln1, dqkv, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "attn.c_attn.weight"), accumulate=acc,
                      M=d, N=3 * d, K=N)
             ops.colsum(dqkv, G(pre + "attn.c_attn.bias"), accumulate=True)
@@ -1442,9 +1479,8 @@ class GatoPolicy(nn.Module):
         if plan.n_patch_rows and getattr(st, "img_groups", None):
             dpe = self._buf("d_patch_emb", (plan.n_patch_rows, d), torch.float32)
             dpe.zero_()
-        check(load().neko_embed_bwd(_p(st.descs), C.c_int(B), C.c_int(d), C.byref(st.tok_params), _p(st.tokens), _p(dx),
-                                    _p(G("embed_token.weight")), _p(G("pos_embed_observation.weight")), _p(G("separator_token")),
-                                    _p(dpe), stream_ptr()), "neko_embed_bwd")
+        ops.embed_bwd(st.descs, B, d, st.tok_params, st.tokens, dx, G("embed_token.weight"), G("pos_embed_observation.weight"),
+                      G("separator_token"), dpe, packed=plan.packed)
         self.launches += 1
         if dpe is not None:
             self._image_backward(st, dpe, acc)

@@ -40,11 +40,18 @@ class BatchPlan:
     n_f: int
     n_i: int
     first_valid: np.ndarray  # int32 [B] = seq_off
-    loss_rows: np.ndarray    # int32 [n_rows] flat positions b*width+s
+    loss_rows: np.ndarray    # int32 [n_rows] flat positions b*width+s (packed: row_base[b]+s-seq_off)
     n_valid_tokens: int
     image_groups: List[ImageGroup]
     n_patch_rows: int
     precomputed_patch: List[Tuple[int, torch.Tensor]]  # (patch_off, image_embeddings [T,P,d])
+    packed: bool = False     # samples back to back, no padding rows (see build_plan)
+    cu_seqlens: np.ndarray = None  # int32 [B+1]: exclusive prefix sum of the sample lengths (packed row_base, then the total)
+
+    @property
+    def token_rows(self) -> int:
+        """Rows of the token-major activations: B * width padded, n_valid_tokens packed."""
+        return self.n_valid_tokens if self.packed else self.B * self.width
 
 
 def _is_present(d: dict, k: str) -> bool:
@@ -69,10 +76,14 @@ def _loss_sel(T: int, n_patches: int, n_text: int, n_obs: int, tpt: int) -> np.n
     return sel
 
 
-def build_plan(inputs: Sequence[dict], *, patch_size: int, context_len: int, pad_seq: bool) -> BatchPlan:
+def build_plan(inputs: Sequence[dict], *, patch_size: int, context_len: int, pad_seq: bool, packed: bool = False) -> BatchPlan:
     """Host half of tokenize_input_dicts (gato_policy.py:195-432): shapes only -- one 16-int descriptor per sample, the
     flat value lists, left-padding offsets and the loss rows.  Runs once per step on the host, so the per-sample work is
-    kept to plain Python ints and list appends; descriptors become one int32 array at the end."""
+    kept to plain Python ints and list appends; descriptors become one int32 array at the end.
+
+    ``packed``: sample b occupies rows [row_base[b], row_base[b] + L_b) of a [T = n_valid_tokens] layout with no padding rows
+    (row_base = exclusive prefix sum of the lengths, stored in the descriptor).  seq_len, width and first_valid keep their
+    padded values: the attention kernels take their dropout coordinates from them."""
     B = len(inputs)
     assert B > 0, "empty batch"
     fvals: List[torch.Tensor] = []
@@ -210,16 +221,22 @@ def build_plan(inputs: Sequence[dict], *, patch_size: int, context_len: int, pad
     width = context_len if (pad_seq and context_len > S) else S
     first_valid = (S - lengths).astype(np.int32)
     desc[:, 7] = first_valid
+    cu_seqlens = np.zeros(B + 1, dtype=np.int32)
+    np.cumsum(lengths, out=cu_seqlens[1:])
+    if packed:
+        desc[:, 14] = cu_seqlens[:B]
     rows = []
     for b in range(B):
-        # loss row s: token s valid (s >= off) and target mask at s+1 set, s+1 < S
+        # loss row s: token s valid (s >= off) and target mask at s+1 set, s+1 < S.  The selected offsets stop before the
+        # sample's last token, so the target row + 1 stays inside the sample in the packed layout too.
         sel = _loss_sel(int(desc[b, 0]), int(desc[b, 1]), int(desc[b, 2]), int(n_obs[b]), int(tpt[b]))
-        rows.append(sel + (b * width + int(first_valid[b])))
+        rows.append(sel + (int(cu_seqlens[b]) if packed else b * width + int(first_valid[b])))
     loss_rows = np.concatenate(rows).astype(np.int32, copy=False) if rows else np.zeros(0, dtype=np.int32)
     raw = desc.view(np.uint8).reshape(-1)
     return BatchPlan(B=B, seq_len=S, width=width, descs=raw, fvals=fvals, ivals=ivals, n_f=n_f, n_i=n_i,
                      first_valid=first_valid, loss_rows=loss_rows, n_valid_tokens=int(lengths.sum()),
-                     image_groups=groups, n_patch_rows=n_patch_rows, precomputed_patch=pre_patch)
+                     image_groups=groups, n_patch_rows=n_patch_rows, precomputed_patch=pre_patch, packed=packed,
+                     cu_seqlens=cu_seqlens)
 
 
 class Stager:
@@ -251,7 +268,7 @@ class Stager:
     HEADER = 256  # bytes at offset 0 of the staging buffer: per-step scalars (dropout seed words)
 
     def upload(self, plan: BatchPlan, header: Optional[np.ndarray] = None):
-        """Returns device views: descs(u8), fvals(f32), ivals(i32), first_valid(i32), loss_rows(i32), the
+        """Returns device views: descs(u8), fvals(f32), ivals(i32), first_valid(i32), loss_rows(i32), cu_seqlens(i32), the
         number of host->device bytes moved and the int32 view of the header region."""
         def al(n):
             return (n + 255) // 256 * 256
@@ -259,7 +276,7 @@ class Stager:
         host_i = all(not t.is_cuda for t in plan.ivals)
         # every region always exists in the (pointer-stable) device buffer, whatever the source of the values: CUDA
         # graphs captured on this batch shape keep reading the same addresses
-        sizes = [plan.descs.nbytes, plan.n_f * 4, plan.n_i * 4, plan.first_valid.nbytes, plan.loss_rows.nbytes]
+        sizes = [plan.descs.nbytes, plan.n_f * 4, plan.n_i * 4, plan.first_valid.nbytes, plan.loss_rows.nbytes, plan.cu_seqlens.nbytes]
         offs = np.cumsum([self.HEADER] + [al(s) for s in sizes])
         total = int(offs[-1])
         self._ensure(total)
@@ -283,13 +300,14 @@ class Stager:
         pin[offs[3]:offs[3] + sizes[3]] = torch.from_numpy(plan.first_valid.view(np.uint8))
         if sizes[4]:
             pin[offs[4]:offs[4] + sizes[4]] = torch.from_numpy(plan.loss_rows.view(np.uint8))
+        pin[offs[5]:offs[5] + sizes[5]] = torch.from_numpy(plan.cu_seqlens.view(np.uint8))
         if host_f and host_i:
             dev[:total].copy_(pin[:total], non_blocking=True)
             h2d = total
         else:
             dev[:self.HEADER].copy_(pin[:self.HEADER], non_blocking=True)
             h2d += self.HEADER
-            for i in range(5):
+            for i in range(6):
                 if sizes[i] and not ((i == 1 and not host_f) or (i == 2 and not host_i)):
                     dev[offs[i]:offs[i] + sizes[i]].copy_(pin[offs[i]:offs[i] + sizes[i]], non_blocking=True)
                     h2d += sizes[i]
@@ -303,4 +321,5 @@ class Stager:
         descs = dev[offs[0]:offs[0] + sizes[0]]
         fv = view(1, torch.float32)
         iv = view(2, torch.int32)
-        return descs, fv, iv, view(3, torch.int32), view(4, torch.int32), h2d, dev[:self.HEADER].view(torch.int32)
+        return (descs, fv, iv, view(3, torch.int32), view(4, torch.int32), view(5, torch.int32), h2d,
+                dev[:self.HEADER].view(torch.int32))

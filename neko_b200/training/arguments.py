@@ -74,6 +74,7 @@ class TrainingArgs:
     # synthetic-data additions of this repo (no datasets / simulators offline)
     synthetic: str = "cfg2"
     disable_cuda_graphs: bool = False   # replay forward / backward from CUDA graphs per batch shape (neko_b200 engine knob)
+    pack_sequences: bool = False        # padding-free steps: samples back to back, variable-length attention (neko_b200 engine knob)
     seed: int = 1234
 
 

@@ -43,6 +43,7 @@ def main():
               "flag only switches its own matmul/softmax path to F.scaled_dot_product_attention (trajectory_gpt2.py:241-250)")
     model.materialize_logits = False   # the trainer discards logits (trainer.py:178)
     model.use_cuda_graphs = not args.disable_cuda_graphs
+    model.pack_sequences = args.pack_sequences
     torch.manual_seed(args.seed + rank)     # per-rank dropout masks, patch-position draws and multinomial remainders
     sync = None
     if world > 1:
