@@ -153,7 +153,7 @@ enum neko_epilogue {
   NEKO_EPI_F32 = 1,             /* C fp32 = acc (+bias) (+= C when accumulate)                  */
   NEKO_EPI_GELU_BF16 = 2,       /* C 16-bit = acc+bias (pre-activation), C2 16-bit = gelu_erf() */
   NEKO_EPI_RESID_F32 = 3,       /* C fp32 = acc + bias + aux_f32[m,n]   (residual add)          */
-  NEKO_EPI_DGELU_BF16 = 4,      /* C 16-bit = acc * gelu_erf'(aux_bf16[m,n])                    */
+  NEKO_EPI_DGELU_BF16 = 4,      /* C 16-bit = acc * gelu_erf'(aux_bf16[m,n]); bias must be NULL */
   NEKO_EPI_RESID_F32_BF16 = 5   /* as 3, plus C2 16-bit copy of the result                      */
 };
 /* 16-bit operands / outputs are bf16 unless the matching flag selects IEEE fp16 (same tensor-core rate,
@@ -187,6 +187,22 @@ typedef struct neko_gemm_desc {
 } neko_gemm_desc;
 
 int neko_gemm(const neko_gemm_desc* host_desc, void* stream);
+
+/* The schedule neko_gemm would launch for this descriptor (same argument checks, same NEKO_GEMM_* environment knobs),
+ * computed on the host without launching anything. */
+typedef struct neko_gemm_plan_info {
+  int32_t BN;                   /* tile width: 128, 192 or 256 columns                          */
+  int32_t pair;                 /* 1: cta_group::2 CTA pair (256-row tile), 0: single CTA (128)  */
+  int32_t splits;               /* split-K factor (fp32 reduce-add into C when > 1)              */
+  int32_t epi_warps;            /* epilogue warps per CTA: 8 or 16                              */
+  int32_t streamk;              /* 1: stream-K work distribution (needs the workspace)          */
+  int32_t tma_store;            /* 1: outputs through shared-memory staging + TMA stores, 0: direct stores */
+  int32_t tma_aux;              /* 1: RESID_F32 / DGELU aux operand through TMA boxes, 0: per-thread loads */
+  int32_t vec_ok;               /* 1: 16-byte epilogue accesses, 0: per-element (scalar) path   */
+  int32_t n_fast;               /* tile rasterisation walks N first                             */
+  int32_t stages;               /* shared-memory ring depth of the main loop                    */
+} neko_gemm_plan_info;
+int neko_gemm_plan(const neko_gemm_desc* host_desc, neko_gemm_plan_info* out);
 /* Bytes of neko_gemm_desc.workspace that cover every problem on this device (148 partial 128 x 256 fp32 tiles + counters). */
 int64_t neko_gemm_workspace_bytes(void);
 

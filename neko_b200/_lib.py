@@ -42,7 +42,11 @@ class Dropout(C.Structure):
         if seed_tensor is None or thr <= 0:
             return cls(seed=None, stream=0, thr16=0, scale=1.0, reserved=0)
         thr = min(thr, 65535)
-        return cls(seed=seed_tensor.data_ptr(), stream=int(stream), thr16=thr, scale=65536.0 / (65536.0 - thr), reserved=0)
+        d = cls(seed=seed_tensor.data_ptr(), stream=int(stream), thr16=thr, scale=65536.0 / (65536.0 - thr), reserved=0)
+        # the kernels read the seed through this pointer: the descriptor keeps its tensor alive, so a temporary seed
+        # (Dropout.make(torch.tensor(...), ...)) is not freed and its memory reused by the time a kernel reads it
+        d._seed_tensor = seed_tensor
+        return d
 
 
 class GemmDesc(C.Structure):
@@ -53,6 +57,12 @@ class GemmDesc(C.Structure):
                 ("C", C.c_void_p), ("ldc", C.c_int64), ("C2", C.c_void_p), ("ldc2", C.c_int64),
                 ("C3", C.c_void_p), ("ldc3", C.c_int64), ("bias", C.c_void_p), ("aux", C.c_void_p), ("ld_aux", C.c_int64),
                 ("drop", Dropout), ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64)]
+
+
+class GemmPlanInfo(C.Structure):
+    """neko_gemm_plan_info (include/neko_b200.h)."""
+    _fields_ = [(n, C.c_int32) for n in (
+        "BN", "pair", "splits", "epi_warps", "streamk", "tma_store", "tma_aux", "vec_ok", "n_fast", "stages")]
 
 
 EPI_BF16, EPI_F32, EPI_GELU_BF16, EPI_RESID_F32, EPI_DGELU_BF16, EPI_RESID_F32_BF16 = range(6)

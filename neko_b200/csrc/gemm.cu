@@ -944,8 +944,20 @@ extern "C" int64_t neko_gemm_workspace_bytes(void) {
   return (int64_t)neko::sm_count() * 128 * 256 * 4 + 4096;
 }
 
-extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
-  using namespace neko;
+namespace neko {
+
+// Everything neko_gemm decides before it launches: the kernel parameters (minus the tensor-map-backed pointers that only the
+// launch needs) and the host-side choices.  neko_gemm_plan reports it without launching.
+struct GemmPlan {
+  GemmParams p;
+  int epi16;         // 16 epilogue warps (else 8)
+  long long mb;      // row blocks of the chosen tile height (128, or 256 for a pair)
+  int stage_bytes;   // one ring stage: A box + this CTA's B box
+  int sms;           // persistent grid cap
+};
+
+// Argument checks and schedule selection of one neko_gemm call.  Launches nothing, touches no device memory.
+static int plan_gemm(const neko_gemm_desc* gd, GemmPlan& pl) {
   NEKO_REQUIRE(gd != nullptr, "gemm: null descriptor");
   const int M = gd->M, N = gd->N, K = gd->K, a_mn = gd->a_mn, b_mn = gd->b_mn, epilogue = gd->epilogue;
   const int accumulate = gd->accumulate, flags = gd->flags;
@@ -965,8 +977,11 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
     NEKO_REQUIRE(aux != nullptr, "gemm: epilogue %d needs aux", epilogue);
   NEKO_REQUIRE(!accumulate || epilogue == NEKO_EPI_F32, "gemm: accumulate is only defined for NEKO_EPI_F32");
   NEKO_REQUIRE(C3 == nullptr || epilogue == NEKO_EPI_GELU_BF16, "gemm: C3 is only defined for NEKO_EPI_GELU_BF16");
+  // C = acc * gelu'(aux): the TMA-aux epilogue has no bias term, the per-thread ones would add it before the multiply
+  NEKO_REQUIRE(bias == nullptr || epilogue != NEKO_EPI_DGELU_BF16, "gemm: NEKO_EPI_DGELU_BF16 takes no bias");
 
-  GemmParams p;
+  GemmParams& p = pl.p;
+  memset(&p, 0, sizeof(p));
   p.M = M; p.N = N; p.K = K;
   p.a_mn = a_mn ? 1 : 0; p.b_mn = b_mn ? 1 : 0;
   p.epi = epilogue; p.accumulate = accumulate; p.flags = flags;
@@ -982,6 +997,7 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
   // a 227 KB CTA queued behind a long-running communication CTA would stall its whole statically partitioned share of tiles)
   static const int sms_cap = getenv("NEKO_GEMM_SMS") ? atoi(getenv("NEKO_GEMM_SMS")) : 0;
   const int sms = (sms_cap > 1 && sms_cap < sm_count()) ? (sms_cap & ~1) : sm_count();
+  pl.sms = sms;
   const int kblocks = (K + BK - 1) / BK;
   const bool can_split = (epilogue == NEKO_EPI_F32) && (bias == nullptr);
   // CTA pairs pay off where the main loop dominates (measured per shape, profiles/r01_gemm_shapes.md): plain fp32
@@ -1017,6 +1033,7 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
     }
   }
   const long long mb_ = (M + (p.pair ? 2 * BM : BM) - 1) / (p.pair ? 2 * BM : BM);
+  pl.mb = mb_;
   if (const char* force = getenv("NEKO_GEMM_BN")) {
     const int v = atoi(force);
     if (v == 128 || v == 256 || (v == 192 && !(p.pair && b_mn))) p.BN = v;
@@ -1029,14 +1046,9 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
   if (const char* force = getenv("NEKO_GEMM_NFAST")) p.n_fast = atoi(force) ? 1 : 0;
   p.kb_per_split = (kblocks + p.splits - 1) / p.splits;
   p.splits = (kblocks + p.kb_per_split - 1) / p.kb_per_split;  // no empty split
-  if (p.splits > 1 && !accumulate) {  // (also correct for the reduce-add TMA path)
-    // partial sums are RED-added: start from zero
-    cudaError_t e = cudaMemset2DAsync(C, (size_t)ldc * sizeof(float), 0, (size_t)N * sizeof(float), (size_t)M, as_stream(stream));
-    if (e != cudaSuccess) return check_cuda(e, "cudaMemset2DAsync(gemm split-K)");
-  }
   const int bnl = p.pair ? p.BN / 2 : p.BN;  // B rows staged per CTA
-  const int stage_bytes = BM * BK * 2 + bnl * BK * 2;
-  p.stages = (SMEM_BUDGET - 1024 - 512 - STAGING_BYTES) / stage_bytes;
+  pl.stage_bytes = BM * BK * 2 + bnl * BK * 2;
+  p.stages = (SMEM_BUDGET - 1024 - 512 - STAGING_BYTES) / pl.stage_bytes;
   if (p.stages > 8) p.stages = 8;
   const bool out_bf16 = (epilogue == NEKO_EPI_BF16 || epilogue == NEKO_EPI_GELU_BF16 || epilogue == NEKO_EPI_DGELU_BF16);
   auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
@@ -1052,37 +1064,15 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
   const int c_esz = out_bf16 ? 2 : 4;
   p.tma_store = (tma_ok(C, ldc, c_esz) && tma_ok(C2, ldc2, 2) && tma_ok(C3, ldc3, 2)) ? 1 : 0;
   if (getenv("NEKO_GEMM_DIRECT_STORE")) p.tma_store = 0;
-  CUtensorMap ma, mb, mc, mc2, mc3, maux;
-  memset(&mc, 0, sizeof(mc)); memset(&mc2, 0, sizeof(mc2)); memset(&mc3, 0, sizeof(mc3)); memset(&maux, 0, sizeof(maux));
-  int rc;
   // the auxiliary operand of the residual / GELU' epilogues through TMA boxes (same staging slots as the output)
   static const bool no_tma_aux = getenv("NEKO_GEMM_NO_TMA_AUX") != nullptr;
   p.tma_aux = 0;
   if (p.tma_store && !no_tma_aux && p.splits == 1 && (epilogue == NEKO_EPI_RESID_F32 || epilogue == NEKO_EPI_DGELU_BF16)) {
     const int aesz = (epilogue == NEKO_EPI_RESID_F32) ? 4 : 2;
-    if (tma_ok(aux, ld_aux, aesz) && (bias == nullptr || al16(bias))) {
-      rc = make_map(&maux, aux, (unsigned long long)N, (unsigned long long)M, (unsigned long long)ld_aux, 32, 32, aesz == 4 ? 2 : 3);
-      if (rc != NEKO_OK) return rc;
-      p.tma_aux = 1;
-    }
-  }
-  if (p.tma_store) {
-    const int ckind = out_bf16 ? ((flags & NEKO_GEMM_C_F16) ? 4 : 3) : 2;
-    rc = make_map(&mc, C, (unsigned long long)N, (unsigned long long)M, (unsigned long long)ldc, 32, 32, ckind);
-    if (rc != NEKO_OK) return rc;
-    if (C2) {
-      rc = make_map(&mc2, C2, (unsigned long long)N, (unsigned long long)M, (unsigned long long)ldc2, 32, 32, (flags & NEKO_GEMM_C2_F16) ? 4 : 3);
-      if (rc != NEKO_OK) return rc;
-    }
-    if (C3) {
-      rc = make_map(&mc3, C3, (unsigned long long)N, (unsigned long long)M, (unsigned long long)ldc3, 32, 32, 3);
-      if (rc != NEKO_OK) return rc;
-    }
+    if (tma_ok(aux, ld_aux, aesz) && (bias == nullptr || al16(bias))) p.tma_aux = 1;
   }
   // stream-K (see WorkIter): worth it when the tile count is a poor multiple of the worker count -- the N = 768 projections and
   // dgrads at the cfg2 token count run 90 pair tiles on 74 pairs, i.e. two rounds for 1.2 rounds of work
-  CUtensorMap mws;
-  memset(&mws, 0, sizeof(mws));
   p.streamk = 0; p.sk_acc = nullptr; p.sk_flags = nullptr;
   {
     const long long workers = p.pair ? sms / 2 : sms;
@@ -1099,19 +1089,88 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
     if (want && gd->workspace && gd->workspace_bytes >= need && (reinterpret_cast<uintptr_t>(gd->workspace) & 127) == 0) {
       p.sk_acc = static_cast<float*>(gd->workspace);
       p.sk_flags = reinterpret_cast<unsigned*>(static_cast<char*>(gd->workspace) + acc_bytes);
-      rc = make_map(&mws, p.sk_acc, (unsigned long long)p.BN, (unsigned long long)(workers * tm), (unsigned long long)p.BN, 32, 32, 2);
-      if (rc != NEKO_OK) return rc;
       p.streamk = 1;
     }
   }
-  if (!p.a_mn) rc = make_map(&ma, A, (unsigned long long)K, (unsigned long long)M, (unsigned long long)lda, BK, BM, (flags & NEKO_GEMM_A_F16) ? 1 : 0);
-  else         rc = make_map(&ma, A, (unsigned long long)M, (unsigned long long)K, (unsigned long long)lda, 64, BK, (flags & NEKO_GEMM_A_F16) ? 1 : 0);
+  // epilogue warps: 16 where the epilogue, not the main loop, bounds the launch (NEKO_GEMM_EPI16=0/1 forces; BN = 192 has no
+  // 4-way column split)
+  const int epi16_env = getenv("NEKO_GEMM_EPI16") ? atoi(getenv("NEKO_GEMM_EPI16")) : -1;   // read per call: tools/gemm_sweep.py flips it
+  bool epi16 = (epilogue == NEKO_EPI_GELU_BF16);   // measured (profiles/r02_gemm_epi16_sweep.txt): 58 -> 54 us for c_fc, neutral or worse elsewhere
+  if (epi16_env >= 0) epi16 = epi16_env != 0;
+  if (p.BN == 192) epi16 = false;
+  pl.epi16 = epi16 ? 1 : 0;
+  return NEKO_OK;
+}
+
+}  // namespace neko
+
+extern "C" int neko_gemm_plan(const neko_gemm_desc* gd, neko_gemm_plan_info* out) {
+  using namespace neko;
+  NEKO_REQUIRE(out != nullptr, "gemm_plan: null output");
+  GemmPlan pl;
+  const int rc = plan_gemm(gd, pl);
   if (rc != NEKO_OK) return rc;
-  if (!p.b_mn) rc = make_map(&mb, B, (unsigned long long)K, (unsigned long long)N, (unsigned long long)ldb, BK, (unsigned)bnl, (flags & NEKO_GEMM_B_F16) ? 1 : 0);
-  else         rc = make_map(&mb, B, (unsigned long long)N, (unsigned long long)K, (unsigned long long)ldb, 64, BK, (flags & NEKO_GEMM_B_F16) ? 1 : 0);
+  out->BN = pl.p.BN;
+  out->pair = pl.p.pair;
+  out->splits = pl.p.splits;
+  out->epi_warps = pl.epi16 ? 16 : 8;
+  out->streamk = pl.p.streamk;
+  out->tma_store = pl.p.tma_store;
+  out->tma_aux = pl.p.tma_aux;
+  out->vec_ok = pl.p.vec_ok;
+  out->n_fast = pl.p.n_fast;
+  out->stages = pl.p.stages;
+  return NEKO_OK;
+}
+
+extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
+  using namespace neko;
+  GemmPlan pl;
+  int rc = plan_gemm(gd, pl);
+  if (rc != NEKO_OK) return rc;
+  GemmParams& p = pl.p;
+  const int M = p.M, N = p.N, K = p.K, flags = p.flags;
+  const bool out_bf16 = (p.epi == NEKO_EPI_BF16 || p.epi == NEKO_EPI_GELU_BF16 || p.epi == NEKO_EPI_DGELU_BF16);
+  if (p.splits > 1 && !p.accumulate) {  // (also correct for the reduce-add TMA path)
+    // partial sums are RED-added: start from zero
+    cudaError_t e = cudaMemset2DAsync(p.C, (size_t)p.ldc * sizeof(float), 0, (size_t)N * sizeof(float), (size_t)M, as_stream(stream));
+    if (e != cudaSuccess) return check_cuda(e, "cudaMemset2DAsync(gemm split-K)");
+  }
+  CUtensorMap ma, mb, mc, mc2, mc3, maux;
+  memset(&mc, 0, sizeof(mc)); memset(&mc2, 0, sizeof(mc2)); memset(&mc3, 0, sizeof(mc3)); memset(&maux, 0, sizeof(maux));
+  if (p.tma_aux) {
+    rc = make_map(&maux, p.aux, (unsigned long long)N, (unsigned long long)M, (unsigned long long)p.ld_aux, 32, 32, p.epi == NEKO_EPI_RESID_F32 ? 2 : 3);
+    if (rc != NEKO_OK) return rc;
+  }
+  if (p.tma_store) {
+    const int ckind = out_bf16 ? ((flags & NEKO_GEMM_C_F16) ? 4 : 3) : 2;
+    rc = make_map(&mc, p.C, (unsigned long long)N, (unsigned long long)M, (unsigned long long)p.ldc, 32, 32, ckind);
+    if (rc != NEKO_OK) return rc;
+    if (p.C2) {
+      rc = make_map(&mc2, p.C2, (unsigned long long)N, (unsigned long long)M, (unsigned long long)p.ldc2, 32, 32, (flags & NEKO_GEMM_C2_F16) ? 4 : 3);
+      if (rc != NEKO_OK) return rc;
+    }
+    if (p.C3) {
+      rc = make_map(&mc3, p.C3, (unsigned long long)N, (unsigned long long)M, (unsigned long long)p.ldc3, 32, 32, 3);
+      if (rc != NEKO_OK) return rc;
+    }
+  }
+  CUtensorMap mws;
+  memset(&mws, 0, sizeof(mws));
+  if (p.streamk) {
+    const long long workers = p.pair ? pl.sms / 2 : pl.sms, tm = p.pair ? 2 * BM : BM;
+    rc = make_map(&mws, p.sk_acc, (unsigned long long)p.BN, (unsigned long long)(workers * tm), (unsigned long long)p.BN, 32, 32, 2);
+    if (rc != NEKO_OK) return rc;
+  }
+  const int bnl = p.pair ? p.BN / 2 : p.BN;  // B rows staged per CTA
+  if (!p.a_mn) rc = make_map(&ma, gd->A, (unsigned long long)K, (unsigned long long)M, (unsigned long long)gd->lda, BK, BM, (flags & NEKO_GEMM_A_F16) ? 1 : 0);
+  else         rc = make_map(&ma, gd->A, (unsigned long long)M, (unsigned long long)K, (unsigned long long)gd->lda, 64, BK, (flags & NEKO_GEMM_A_F16) ? 1 : 0);
+  if (rc != NEKO_OK) return rc;
+  if (!p.b_mn) rc = make_map(&mb, gd->B, (unsigned long long)K, (unsigned long long)N, (unsigned long long)gd->ldb, BK, (unsigned)bnl, (flags & NEKO_GEMM_B_F16) ? 1 : 0);
+  else         rc = make_map(&mb, gd->B, (unsigned long long)N, (unsigned long long)K, (unsigned long long)gd->ldb, 64, BK, (flags & NEKO_GEMM_B_F16) ? 1 : 0);
   if (rc != NEKO_OK) return rc;
 
-  const size_t smem = (size_t)p.stages * stage_bytes + STAGING_BYTES + 1024 /*alignment slack*/ + 512 /*barriers*/;
+  const size_t smem = (size_t)p.stages * pl.stage_bytes + STAGING_BYTES + 1024 /*alignment slack*/ + 512 /*barriers*/;
   static std::once_flag attr_once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(attr_once, [] {
@@ -1121,14 +1180,10 @@ extern "C" int neko_gemm(const neko_gemm_desc* gd, void* stream) {
       if (attr_err == cudaSuccess) attr_err = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BUDGET);
   });
   if (attr_err != cudaSuccess) return check_cuda(attr_err, "cudaFuncSetAttribute(gemm)");
-  // epilogue warps: 16 where the epilogue, not the main loop, bounds the launch (NEKO_GEMM_EPI16=0/1 forces; BN = 192 has no
-  // 4-way column split)
-  const int epi16_env = getenv("NEKO_GEMM_EPI16") ? atoi(getenv("NEKO_GEMM_EPI16")) : -1;   // read per call: tools/gemm_sweep.py flips it
-  bool epi16 = (epilogue == NEKO_EPI_GELU_BF16);   // measured (profiles/r02_gemm_epi16_sweep.txt): 58 -> 54 us for c_fc, neutral or worse elsewhere
-  if (epi16_env >= 0) epi16 = epi16_env != 0;
-  if (p.BN == 192) epi16 = false;
+  const bool epi16 = pl.epi16 != 0;
+  const int sms = pl.sms;
   const int threads = 64 + 32 * (epi16 ? 16 : 8);
-  const long long units = mb_ * ((N + p.BN - 1) / p.BN) * p.splits;   // stream-K: tiles >= workers, so the grid below is the full one
+  const long long units = pl.mb * ((N + p.BN - 1) / p.BN) * p.splits;   // stream-K: tiles >= workers, so the grid below is the full one
   if (p.pair) {
     const int pairs = sms / 2;
     const int grid = 2 * (int)(units < pairs ? units : pairs);

@@ -12,7 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import (EPI_BF16, EPI_DGELU_BF16, EPI_F32, EPI_GELU_BF16, EPI_RESID_F32, EPI_RESID_F32_BF16,  # noqa: F401
-                   Dropout, GemmDesc, SampleDesc, TokParams, _p, check, load, stream_ptr)
+                   Dropout, GemmDesc, GemmPlanInfo, SampleDesc, TokParams, _p, check, load, stream_ptr)
 
 
 _16BIT = (torch.bfloat16, torch.float16)
@@ -48,15 +48,8 @@ def _gemm_workspace(device):
     return ws
 
 
-def gemm(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: bool = False, epilogue: int = EPI_BF16,
-         out: Optional[torch.Tensor] = None, out2: Optional[torch.Tensor] = None, out3: Optional[torch.Tensor] = None,
-         bias: Optional[torch.Tensor] = None, aux: Optional[torch.Tensor] = None, accumulate: bool = False,
-         M: Optional[int] = None, N: Optional[int] = None, K: Optional[int] = None,
-         out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False):
-    """C[M,N] = epilogue(sum_k A[m,k] B[n,k]).
-
-    a: 16-bit [M,K] (a_mn=False) or [K,M] (a_mn=True); b: same format, [N,K] or [K,N]; rows may be strided
-    (stride(0) is the leading dimension)."""
+def _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop, gelu_tanh):
+    """neko_gemm_desc of one gemm() / gemm_plan() call, allocating the outputs that were not given."""
     _cuda(a, b, out, out2, out3, bias, aux)
     assert a.dtype in _16BIT and b.dtype == a.dtype, "A and B must share one 16-bit format"
     assert a.stride(1) == 1 and b.stride(1) == 1
@@ -86,17 +79,45 @@ def gemm(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: bool = F
     ws = _gemm_workspace(a.device)
     if ws is not None:
         gd.workspace, gd.workspace_bytes = ws.data_ptr(), ws.numel()
+    return gd, out, out2
+
+
+def gemm(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: bool = False, epilogue: int = EPI_BF16,
+         out: Optional[torch.Tensor] = None, out2: Optional[torch.Tensor] = None, out3: Optional[torch.Tensor] = None,
+         bias: Optional[torch.Tensor] = None, aux: Optional[torch.Tensor] = None, accumulate: bool = False,
+         M: Optional[int] = None, N: Optional[int] = None, K: Optional[int] = None,
+         out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False):
+    """C[M,N] = epilogue(sum_k A[m,k] B[n,k]).
+
+    a: 16-bit [M,K] (a_mn=False) or [K,M] (a_mn=True); b: same format, [N,K] or [K,N]; rows may be strided
+    (stride(0) is the leading dimension)."""
+    gd, out, out2 = _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop,
+                               gelu_tanh)
     if GEMM_TIMING is not None:  # bench.py: CUDA events around every tensor-core launch (roofline.achieved)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         check(load().neko_gemm(C.byref(gd), stream_ptr()), "neko_gemm")
         e1.record()
-        GEMM_TIMING.append((e0, e1, 2.0 * M * N * K, (M, N, K, int(a_mn), int(b_mn), epilogue)))
+        GEMM_TIMING.append((e0, e1, 2.0 * gd.M * gd.N * gd.K, (gd.M, gd.N, gd.K, int(a_mn), int(b_mn), epilogue)))
     else:
         check(load().neko_gemm(C.byref(gd), stream_ptr()), "neko_gemm")
     if out2 is not None and epilogue in (EPI_GELU_BF16, EPI_RESID_F32_BF16):
         return out, out2
     return out
+
+
+def gemm_plan(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: bool = False, epilogue: int = EPI_BF16,
+              out: Optional[torch.Tensor] = None, out2: Optional[torch.Tensor] = None, out3: Optional[torch.Tensor] = None,
+              bias: Optional[torch.Tensor] = None, aux: Optional[torch.Tensor] = None, accumulate: bool = False,
+              M: Optional[int] = None, N: Optional[int] = None, K: Optional[int] = None,
+              out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False) -> dict:
+    """The schedule gemm() would launch with the same arguments (neko_gemm_plan_info as a dict); launches nothing.
+    Raises NekoError where gemm() would reject the arguments."""
+    gd, _, _ = _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop,
+                          gelu_tanh)
+    info = GemmPlanInfo()
+    check(load().neko_gemm_plan(C.byref(gd), C.byref(info)), "neko_gemm_plan")
+    return {name: getattr(info, name) for name, _ in GemmPlanInfo._fields_}
 
 
 # ------------------------------------------------------------------------------------------

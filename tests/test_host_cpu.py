@@ -47,20 +47,35 @@ def test_integration_doc_names_every_entry_point():
 def test_struct_layouts_match_header(tmp_path):
     """ctypes mirrors vs the C header, as a C compiler lays the structs out."""
     import subprocess
-    from neko_b200._lib import Dropout, GemmDesc, SampleDesc, TokParams, HEADER
+    from neko_b200._lib import Dropout, GemmDesc, GemmPlanInfo, SampleDesc, TokParams, HEADER
     assert ctypes.sizeof(SampleDesc) == 64
     assert ctypes.sizeof(TokParams) == 40
     assert ctypes.sizeof(Dropout) == 24
     assert ctypes.sizeof(GemmDesc) == 8 * 4 + 13 * 8 + 24 + 16
+    assert ctypes.sizeof(GemmPlanInfo) == 10 * 4
     src = tmp_path / "sizes.c"
-    src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "neko_b200.h"\nint main(void){printf("%zu %zu %zu %zu %zu %zu %zu",'
+    src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "neko_b200.h"\nint main(void){printf("%zu %zu %zu %zu %zu %zu %zu %zu",'
                    'sizeof(neko_sample_desc), sizeof(neko_tok_params), sizeof(neko_dropout), sizeof(neko_gemm_desc),'
-                   'offsetof(neko_gemm_desc, drop), offsetof(neko_gemm_desc, aux), offsetof(neko_gemm_desc, workspace));return 0;}\n')
+                   'offsetof(neko_gemm_desc, drop), offsetof(neko_gemm_desc, aux), offsetof(neko_gemm_desc, workspace),'
+                   'sizeof(neko_gemm_plan_info));return 0;}\n')
     exe = tmp_path / "sizes"
     subprocess.run(["gcc", "-I", os.path.dirname(HEADER), str(src), "-o", str(exe)], check=True)
     got = [int(v) for v in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.split()]
     assert got == [ctypes.sizeof(SampleDesc), ctypes.sizeof(TokParams), ctypes.sizeof(Dropout), ctypes.sizeof(GemmDesc),
-                   GemmDesc.drop.offset, GemmDesc.aux.offset, GemmDesc.workspace.offset]
+                   GemmDesc.drop.offset, GemmDesc.aux.offset, GemmDesc.workspace.offset, ctypes.sizeof(GemmPlanInfo)]
+
+
+def test_dropout_descriptor_keeps_its_seed_alive():
+    """The kernels read the seed through the descriptor's pointer: a temporary seed tensor must outlive the call that
+    made the descriptor (else its memory is reused before the kernel reads it)."""
+    import gc
+    import weakref
+    from neko_b200._lib import Dropout
+    dr = Dropout.make(torch.tensor([9, 10], dtype=torch.int32), 6, 0.25)
+    gc.collect()
+    seed = weakref.ref(dr._seed_tensor)
+    assert seed() is not None and dr.seed == seed().data_ptr()
+    assert Dropout.make(None, 6, 0.25).seed is None and Dropout.make(torch.tensor([1, 2]), 6, 0.0).seed is None
 
 
 def test_no_cpu_fallback():
