@@ -217,9 +217,15 @@ int64_t neko_gemm_workspace_bytes(void);
 int neko_attention_fwd(const uint16_t* qkv, const int32_t* first_valid, uint16_t* out,
                        uint16_t* out2_bf16 /* nullable second copy */, float* lse, int B, int S, int S_valid,
                        int H, int dh, int out_f16, const neko_dropout* drop, void* stream);
+/* The forward kernel neko_attention_fwd would run for these arguments (same argument checks, same NEKO_ATTN_TC knob),
+ * decided on the host without launching anything: 0 = mma.sync kernel, 1 = tcgen05 kernel, < 0 = the call is rejected. */
+int neko_attention_fwd_path(const uint16_t* qkv, const int32_t* first_valid, const uint16_t* out,
+                            const uint16_t* out2_bf16, const float* lse, int B, int S, int S_valid, int H, int dh,
+                            int out_f16, const neko_dropout* drop);
 /* Single-query attention against a key/value cache (KV-cached decode for the predict_* loops, gato_policy.py:452-476 --
  * the reference re-runs the whole context per generated token).  q bf16 [H*dh] (the new position's query), k_cache /
- * v_cache bf16 [len, H*dh] (all visible keys incl. the new one), out 16-bit [H*dh]. */
+ * v_cache bf16 [len, H*dh] (all visible keys incl. the new one), out 16-bit [H*dh].  len <= 8192; dh even and dividing 128;
+ * q and k_cache 4-byte aligned. */
 int neko_attention_decode(const uint16_t* q, const uint16_t* k_cache, const uint16_t* v_cache, int len, int H, int dh,
                           uint16_t* out, int out_f16, void* stream);
 /* dqkv bf16 [B,S,3*H*dh]; delta fp32 [B,H,S] is caller-provided scratch. */

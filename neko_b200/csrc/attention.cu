@@ -764,8 +764,20 @@ __global__ void __launch_bounds__(128) attn_decode_kernel(const bf16* __restrict
 }
 
 // tcgen05 forward (attention_tc.cu): 0 = ran, 1 = shape not covered, < 0 = error
+bool attention_fwd_tc_eligible(const void* qkv, const void* out, const void* out2, int H, int dh);
 int attention_fwd_tc(const bf16* qkv, const int32_t* fv, bf16* out, bf16* out2, float* lse, int B, int S, int S_valid, int H, int dh, int out_f16,
                      DropCfg drop, cudaStream_t st);
+
+// argument checks of neko_attention_fwd, shared with neko_attention_fwd_path
+static int attention_fwd_args(const uint16_t* qkv, const int32_t* first_valid, const uint16_t* out, const float* lse, int B, int S,
+                              int S_valid, int H, int dh) {
+  NEKO_REQUIRE(qkv && first_valid && out && lse, "attention_fwd: null pointer");
+  NEKO_REQUIRE(B > 0 && S > 0 && H > 0 && S_valid > 0 && S_valid <= S, "attention_fwd: bad sizes");
+  NEKO_REQUIRE((reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, "attention_fwd: misaligned");
+  NEKO_REQUIRE((long long)B * H * S < (1LL << 32), "attention_fwd: B*H*S exceeds the dropout row-id range");
+  NEKO_REQUIRE(dh == 16 || dh == 32 || dh == 64 || dh == 128, "attention: head dim %d not supported (16, 32, 64, 128)", dh);
+  return NEKO_OK;
+}
 
 }  // namespace neko
 
@@ -774,10 +786,8 @@ extern "C" {
 int neko_attention_fwd(const uint16_t* qkv, const int32_t* first_valid, uint16_t* out, uint16_t* out2_bf16, float* lse, int B, int S,
                        int S_valid, int H, int dh, int out_f16, const neko_dropout* drop, void* stream) {
   using namespace neko;
-  NEKO_REQUIRE(qkv && first_valid && out && lse, "attention_fwd: null pointer");
-  NEKO_REQUIRE(B > 0 && S > 0 && H > 0 && S_valid > 0 && S_valid <= S, "attention_fwd: bad sizes");
-  NEKO_REQUIRE((reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, "attention_fwd: misaligned");
-  NEKO_REQUIRE((long long)B * H * S < (1LL << 32), "attention_fwd: B*H*S exceeds the dropout row-id range");
+  const int rc = attention_fwd_args(qkv, first_valid, out, lse, B, S, S_valid, H, dh);
+  if (rc != NEKO_OK) return rc;
   const bf16* x = reinterpret_cast<const bf16*>(qkv);
   bf16* o = reinterpret_cast<bf16*>(out);
   bf16* o2 = reinterpret_cast<bf16*>(out2_bf16);
@@ -799,11 +809,23 @@ int neko_attention_fwd(const uint16_t* qkv, const int32_t* first_valid, uint16_t
 #undef NEKO_ATT_FWD
 }
 
+int neko_attention_fwd_path(const uint16_t* qkv, const int32_t* first_valid, const uint16_t* out, const uint16_t* out2_bf16, const float* lse,
+                            int B, int S, int S_valid, int H, int dh, int out_f16, const neko_dropout* drop) {
+  using namespace neko;
+  (void)out_f16;
+  (void)drop;
+  const int rc = attention_fwd_args(qkv, first_valid, out, lse, B, S, S_valid, H, dh);
+  if (rc != NEKO_OK) return rc;
+  return attention_fwd_tc_eligible(qkv, out, out2_bf16, H, dh) ? 1 : 0;
+}
+
 int neko_attention_decode(const uint16_t* q, const uint16_t* k_cache, const uint16_t* v_cache, int len, int H, int dh, uint16_t* out,
                           int out_f16, void* stream) {
   using namespace neko;
   NEKO_REQUIRE(q && k_cache && v_cache && out, "attention_decode: null pointer");
   NEKO_REQUIRE(len > 0 && len <= 8192 && H > 0 && dh > 0 && dh <= 128 && dh % 2 == 0 && 128 % dh == 0, "attention_decode: bad sizes (len=%d dh=%d)", len, dh);
+  // q and the key rows are read as pairs of bf16 (32-bit loads)
+  NEKO_REQUIRE((reinterpret_cast<uintptr_t>(q) & 3) == 0 && (reinterpret_cast<uintptr_t>(k_cache) & 3) == 0, "attention_decode: misaligned");
   const size_t smem = (size_t)(len + 128) * sizeof(float);
   attn_decode_kernel<<<H, 128, smem, as_stream(stream)>>>(reinterpret_cast<const bf16*>(q), reinterpret_cast<const bf16*>(k_cache),
                                                          reinterpret_cast<const bf16*>(v_cache), len, H * dh, dh, 1.0f / sqrtf((float)dh), out,
@@ -820,6 +842,7 @@ int neko_attention_bwd(const uint16_t* qkv, const uint16_t* out, const uint16_t*
   NEKO_REQUIRE(B > 0 && S > 0 && H > 0 && S_valid > 0 && S_valid <= S, "attention_bwd: bad sizes");
   NEKO_REQUIRE((reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
                (reinterpret_cast<uintptr_t>(dout) & 15) == 0, "attention_bwd: misaligned");
+  NEKO_REQUIRE((long long)B * H * S < (1LL << 32), "attention_bwd: B*H*S exceeds the dropout row-id range");
   cudaStream_t st = as_stream(stream);
   const bf16* x = reinterpret_cast<const bf16*>(qkv);
   const bf16* o = reinterpret_cast<const bf16*>(out);

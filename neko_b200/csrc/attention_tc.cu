@@ -353,18 +353,24 @@ static int launch_fwd_tc(const CUtensorMap& map, const int32_t* fv, bf16* out, b
   return NEKO_OK;
 }
 
-// returns NEKO_OK when the tensor-core path ran, 1 when the shape is not covered (caller falls back), < 0 on error
-int attention_fwd_tc(const bf16* qkv, const int32_t* fv, bf16* out, bf16* out2, float* lse, int B, int S, int S_valid, int H, int dh, int out_f16,
-                     DropCfg drop, cudaStream_t st) {
+// true when neko_attention_fwd takes the tcgen05 path for these arguments (host only, launches nothing)
+bool attention_fwd_tc_eligible(const void* qkv, const void* out, const void* out2, int H, int dh) {
   // Opt-in (NEKO_ATTN_TC=1, read per call so tests can toggle it): at the BASELINE head dim 32 the op is bound by exp /
   // barrier latency, not by the tensor pipe, and the mma.sync kernel with 4-6 resident CTAs per SM is faster
   // (41 us vs 57 us per launch at cfg2, profiles/r01_ncu_attn_tc.txt; DESIGN.md section 4).
   const char* on = getenv("NEKO_ATTN_TC");
-  if (!(on && atoi(on) != 0)) return 1;
-  if (!(dh == 64 || (dh == 32 && H % 2 == 0))) return 1;
+  if (!(on && atoi(on) != 0)) return false;
+  if (!(dh == 64 || (dh == 32 && H % 2 == 0))) return false;
   const int d = H * dh;
-  if ((reinterpret_cast<uintptr_t>(qkv) & 15) || (reinterpret_cast<uintptr_t>(out) & 15) || (out2 && (reinterpret_cast<uintptr_t>(out2) & 15)) || d % 8)
-    return 1;
+  return !((reinterpret_cast<uintptr_t>(qkv) & 15) || (reinterpret_cast<uintptr_t>(out) & 15) || (out2 && (reinterpret_cast<uintptr_t>(out2) & 15)) ||
+           d % 8);
+}
+
+// returns NEKO_OK when the tensor-core path ran, 1 when the shape is not covered (caller falls back), < 0 on error
+int attention_fwd_tc(const bf16* qkv, const int32_t* fv, bf16* out, bf16* out2, float* lse, int B, int S, int S_valid, int H, int dh, int out_f16,
+                     DropCfg drop, cudaStream_t st) {
+  if (!attention_fwd_tc_eligible(qkv, out, out2, H, dh)) return 1;
+  const int d = H * dh;
   CUtensorMap map;
   int rc = make_map(&map, qkv, 3ull * d, (unsigned long long)B * S, 3ull * d, 64, ATC_BLK, 0);
   if (rc != NEKO_OK) return rc;

@@ -215,6 +215,24 @@ def attention_fwd(qkv: torch.Tensor, first_valid: torch.Tensor, H: int, S_valid:
     return out, lse
 
 
+def attention_fwd_path(qkv: torch.Tensor, first_valid: torch.Tensor, H: int, S_valid: Optional[int] = None, out=None, lse=None,
+                       out_dtype: torch.dtype = torch.bfloat16, out2=None, drop=None) -> str:
+    """The forward kernel attention_fwd() would run with the same arguments: "mma" (mma.sync) or "tc" (tcgen05);
+    launches nothing.  Raises NekoError where attention_fwd() would reject the arguments."""
+    B, S, three_d = qkv.shape
+    d = three_d // 3
+    if out is None:
+        out = torch.empty(B, S, d, device=qkv.device, dtype=out_dtype)
+    if lse is None:
+        lse = torch.empty(B, H, S, device=qkv.device, dtype=torch.float32)
+    rc = load().neko_attention_fwd_path(_p(qkv), _p(first_valid), _p(out), _p(out2), _p(lse), C.c_int(B), C.c_int(S),
+                                        C.c_int(S if S_valid is None else S_valid), C.c_int(H), C.c_int(d // H),
+                                        C.c_int(int(out.dtype == torch.float16)), _dref(drop))
+    if rc < 0:
+        check(rc, "neko_attention_fwd_path")
+    return ("mma", "tc")[rc]
+
+
 def attention_decode(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tensor, length: int, H: int, out: torch.Tensor):
     """One new query against `length` cached keys / values (bf16 [>=length, d])."""
     d = q.numel()
