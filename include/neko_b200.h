@@ -165,6 +165,8 @@ enum neko_epilogue {
 #define NEKO_GEMM_C_F16 4
 #define NEKO_GEMM_C2_F16 8
 #define NEKO_GEMM_GELU_TANH 16 /* GELU / GELU' epilogues use the tanh form (HF "gelu_new", pretrained GPT-2) instead of erf */
+#define NEKO_GEMM_DETERMINISTIC 32 /* bitwise reproducible: splits = 1 and no stream-K whatever NEKO_GEMM_SPLITS / NEKO_GEMM_STREAMK
+                                    * say, so each element is summed by one CTA in k order (the result does not depend on the grid) */
 
 typedef struct neko_gemm_desc {
   int32_t M, N, K;
@@ -335,6 +337,62 @@ int neko_adamw_step(float* param, const float* grad, float* exp_avg, float* exp_
                     float lr, float beta1, float beta2, float eps, float weight_decay, int step,
                     const float* grad_sumsq, float max_norm, float grad_div,
                     uint16_t* w_f16, uint16_t* w_bf16, int64_t n_cast, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Ordered reductions (deterministic training mode, DESIGN.md "Deterministic training mode").  Each entry point computes what
+ * its default twin computes, but every floating-point sum has a fixed order that depends on the problem shape only -- not on
+ * the grid, the SM count, NEKO_*_CTAS caps or timing -- so the result is bitwise reproducible.  It differs from the default
+ * twin by reassociation only.  Scratch memory comes from `workspace` (device, at least *_workspace_bytes bytes, no
+ * initialisation needed; 256-byte aligned for the sorting entry points, 16-byte for the others); nothing is allocated or
+ * synchronised, so the calls can be captured in a CUDA graph.  The *_workspace_bytes queries return the size, or a negative
+ * NEKO_E* code.  Argument checks return NEKO_EINVAL before any CUDA call; the sorting entry points (embed, patch_pos) query
+ * the radix sort's scratch size before they compare it with workspace_bytes.
+ * NEKO_ORDERED_CTAS (environment) caps the grid of these kernels; it changes no result.
+ * ------------------------------------------------------------------------------------------- */
+/* neko_layernorm_bwd with dgamma / dbeta / dx_colsum summed over fixed 64-row blocks (block partials in the workspace, then
+ * folded in a fixed order, one writer per element).  d % 4 == 0, d <= 2048; x, dx_resid, gamma 16-byte and dy, dx_bf16
+ * 8-byte aligned.  dx_resid and dx_bf16 are computed row by row exactly as the warp-per-row default kernel does. */
+int64_t neko_layernorm_bwd_ordered_workspace_bytes(int N, int d);
+int neko_layernorm_bwd_ordered(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean,
+                               const float* rstd, float* dx_resid, uint16_t* dx_bf16, float* dgamma, float* dbeta,
+                               float* dx_colsum, int N, int d, const neko_dropout* branch_drop, void* workspace,
+                               int64_t workspace_bytes, void* stream);
+/* neko_colsum_bf16 over fixed 64-row blocks. */
+int64_t neko_colsum_bf16_ordered_workspace_bytes(int M, int N);
+int neko_colsum_bf16_ordered(const uint16_t* X, int64_t ld, int M, int N, float* out, int accumulate, void* workspace,
+                             int64_t workspace_bytes, void* stream);
+/* neko_embed_bwd / neko_embed_packed_bwd as a sorted scatter-add: (table row, source row) keys are built on the device and
+ * radix-sorted (stable), and every embed_token / pos_embed_observation row and the separator is summed by one writer in
+ * ascending source-row order.  d_patch_emb rows are copied.  Ids outside [0, vocab) and position slots >= ctx_rows are
+ * skipped.  Gradient buffers 16-byte aligned.  One workspace size covers both layouts. */
+int64_t neko_embed_bwd_ordered_workspace_bytes(int B, const neko_tok_params* host_params);
+int neko_embed_bwd_ordered(const neko_sample_desc* descs, int B, int d, const neko_tok_params* host_params,
+                           const int64_t* tokens, const float* d_token_embeddings, float* d_embed_table, float* d_pos_table,
+                           float* d_sep, float* d_patch_emb, void* workspace, int64_t workspace_bytes, void* stream);
+int neko_embed_packed_bwd_ordered(const neko_sample_desc* descs, int B, int d, const neko_tok_params* host_params,
+                                  const int64_t* tokens, const float* d_token_embeddings, float* d_embed_table,
+                                  float* d_pos_table, float* d_sep, float* d_patch_emb, void* workspace,
+                                  int64_t workspace_bytes, void* stream);
+/* neko_patch_resblock_bwd with the patches cut into fixed chunks of 8: each chunk stores its weight / GroupNorm gradient
+ * partials to a workspace slot, and the slots are folded in a fixed order. */
+int64_t neko_patch_resblock_bwd_ordered_workspace_bytes(int n_img, int Himg, int Wimg, int patch);
+int neko_patch_resblock_bwd_ordered(const void* images, int is_u8, int n_img, int Himg, int Wimg, int patch,
+                                    int C, int groups, const float* conv1_w, const float* conv1_b,
+                                    const float* gn_w, const float* gn_b, const float* conv2_w,
+                                    const float* gn_stats, const uint16_t* d_patches_bf16,
+                                    float* d_conv1_w, float* d_conv1_b, float* d_gn_w, float* d_gn_b,
+                                    float* d_conv2_w, float* d_conv2_b, void* workspace, int64_t workspace_bytes,
+                                    void* stream);
+/* neko_patch_pos_bwd as a sorted scatter-add (d % 4 == 0).  n_row_bins / n_col_bins: rows of d_row_tab / d_col_tab; bins
+ * outside them are skipped. */
+int64_t neko_patch_pos_bwd_ordered_workspace_bytes(int P, int n_row_bins, int n_col_bins);
+int neko_patch_pos_bwd_ordered(const float* dx, int P, int d, const int32_t* row_bin, const int32_t* col_bin,
+                               float* d_row_tab, int n_row_bins, float* d_col_tab, int n_col_bins, void* workspace,
+                               int64_t workspace_bytes, void* stream);
+/* neko_sumsq_f32 over fixed 8192-element blocks, then one CTA folds the block partials in a fixed order. */
+int64_t neko_sumsq_f32_ordered_workspace_bytes(int64_t n);
+int neko_sumsq_f32_ordered(const float* x, int64_t n, float* out_accum, void* workspace, int64_t workspace_bytes,
+                           void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Data-parallel gradient all-reduce over NVLink peer memory (replaces the DDP bucket all-reduce the reference gets from

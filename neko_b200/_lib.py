@@ -88,7 +88,7 @@ def load():
     lib.neko_last_error.restype = C.c_char_p
     for name in declared_symbols():
         fn = getattr(lib, name)  # AttributeError here = header / library mismatch
-        if name == "neko_gemm_workspace_bytes":
+        if name == "neko_gemm_workspace_bytes" or name.endswith("_workspace_bytes"):
             fn.restype = C.c_int64
         elif name != "neko_last_error":
             fn.restype = C.c_int

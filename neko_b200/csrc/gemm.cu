@@ -999,7 +999,10 @@ static int plan_gemm(const neko_gemm_desc* gd, GemmPlan& pl) {
   const int sms = (sms_cap > 1 && sms_cap < sm_count()) ? (sms_cap & ~1) : sm_count();
   pl.sms = sms;
   const int kblocks = (K + BK - 1) / BK;
-  const bool can_split = (epilogue == NEKO_EPI_F32) && (bias == nullptr);
+  // NEKO_GEMM_DETERMINISTIC: every output element is summed by one CTA in k order, whatever the tile shape (no split-K, no
+  // stream-K; the NEKO_GEMM_SPLITS / NEKO_GEMM_STREAMK forcing is ignored).
+  const bool deterministic = (flags & NEKO_GEMM_DETERMINISTIC) != 0;
+  const bool can_split = (epilogue == NEKO_EPI_F32) && (bias == nullptr) && !deterministic;
   // CTA pairs pay off where the main loop dominates (measured per shape, profiles/r01_gemm_shapes.md): plain fp32
   // outputs (LM head, weight gradients) and wide 16-bit outputs; narrow-N and epilogue-heavy launches stay single-CTA.
   // (tools/gemm_sweep.py: at K >= 2048 the 256 x 256 pair tile also wins for N = 768 despite filling only 1.2 waves.)
@@ -1086,6 +1089,7 @@ static int plan_gemm(const neko_gemm_desc* gd, GemmPlan& pl) {
                 tiles_sk % workers != 0 && (double)(rounds * workers) >= 1.12 * (double)tiles_sk && rounds <= 4;
     if (sk_env == 0) want = false;
     if (sk_env < 0) want = false;          // default off until measured (NEKO_GEMM_STREAMK=1 enables)
+    if (deterministic) want = false;
     if (want && gd->workspace && gd->workspace_bytes >= need && (reinterpret_cast<uintptr_t>(gd->workspace) & 127) == 0) {
       p.sk_acc = static_cast<float*>(gd->workspace);
       p.sk_flags = reinterpret_cast<unsigned*>(static_cast<char*>(gd->workspace) + acc_bytes);

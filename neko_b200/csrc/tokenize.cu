@@ -9,6 +9,7 @@
 // sample descriptor, computes the id (lane-uniform), then streams the d-float row with 128-bit
 // loads/stores.  Algorithmic bytes per token: d*4 (table row) + d*4 (output row) + 16 (id + masks).
 #include "common.cuh"
+#include "ordered.cuh"
 
 namespace neko {
 
@@ -268,9 +269,112 @@ static int embed_bwd(const neko_sample_desc* descs, int B, int d, const neko_tok
   return NEKO_OK;
 }
 
+// Ordered backward (deterministic mode): one warp per grid position writes two sort keys -- [0, n) the table row (embed_token
+// row id, or vocab for the separator), [n, 2n) the position-table row (vocab + 1 + j) -- with the position's gradient row as
+// value; positions without a target get the sentinel key.  Patch rows are copied (one writer per row).  The sorted segments
+// are then summed in ascending source-row order (ordered.cu).
+template <bool PACKED>
+__global__ void __launch_bounds__(256) embed_keys_kernel(EmbBwdArgs a, unsigned* __restrict__ keys, int* __restrict__ vals) {
+  const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  const int width = PACKED ? a.p.seq_len : a.p.width;
+  const long long n = (long long)a.B * width;
+  if (warp >= n) return;
+  const int b = (int)(warp / width);
+  const int s = (int)(warp - (long long)b * width);
+  const neko_sample_desc sd = a.descs[b];
+  const SlotInfo si = locate(sd, s, a.p.seq_len);
+  const unsigned sentinel = (unsigned)(a.p.vocab + 1 + a.p.ctx_rows);
+  unsigned tk = sentinel, pk = sentinel;
+  int row = 0;
+  if (si.kind != SLOT_PAD) {
+    row = PACKED ? sd.row_base + (s - sd.seq_off) : (int)warp;
+    if (si.kind == SLOT_PATCH) {
+      if (a.d_patch_emb) {
+        const float4* g = reinterpret_cast<const float4*>(a.d_emb + (size_t)row * a.d);
+        float4* dst = reinterpret_cast<float4*>(a.d_patch_emb + ((size_t)sd.patch_off + (size_t)si.t * sd.n_patches + si.k) * a.d);
+        for (int i = lane; i < (a.d >> 2); i += 32) dst[i] = g[i];
+      }
+    } else if (si.kind == SLOT_SEP) {
+      tk = (unsigned)a.p.vocab;
+    } else {
+      const long long id = a.tokens[row];
+      if (id >= 0 && id < a.p.vocab) tk = (unsigned)id;
+    }
+    if (a.p.use_pos && si.kind >= SLOT_PATCH && si.kind <= SLOT_DOBS && si.j < a.p.ctx_rows) pk = (unsigned)(a.p.vocab + 1 + si.j);
+  }
+  if (lane == 0) {
+    keys[warp] = tk; vals[warp] = row;
+    keys[n + warp] = pk; vals[n + warp] = row;
+  }
+}
+
+static int embed_ord_check(const neko_tok_params* hp, int B) {
+  NEKO_REQUIRE(hp && B > 0 && hp->seq_len > 0 && hp->width >= hp->seq_len && hp->vocab > 0 && hp->ctx_rows >= 0,
+               "embed_bwd_ordered: bad B / seq_len / width / vocab / ctx_rows");
+  NEKO_REQUIRE((long long)B * hp->width <= (1LL << 29) && (long long)hp->vocab + hp->ctx_rows < (1LL << 30),
+               "embed_bwd_ordered: problem too large");
+  return NEKO_OK;
+}
+
+template <bool PACKED>
+static int embed_bwd_ordered(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp, const int64_t* tokens,
+                             const float* d_token_embeddings, float* d_embed_table, float* d_pos_table, float* d_sep,
+                             float* d_patch_emb, void* workspace, int64_t workspace_bytes, void* stream) {
+  NEKO_REQUIRE(descs && hp && tokens && d_token_embeddings && d_embed_table && d_sep && workspace, "embed_bwd_ordered: null pointer");
+  NEKO_REQUIRE(d_pos_table || !hp->use_pos, "embed_bwd_ordered: null d_pos_table");
+  int rc = embed_ord_check(hp, B);
+  if (rc != NEKO_OK) return rc;
+  NEKO_REQUIRE(d > 0 && d % 4 == 0, "embed_bwd_ordered: embed_dim must be a multiple of 4 (got %d)", d);
+  auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+  NEKO_REQUIRE(al16(d_token_embeddings) && al16(d_embed_table) && al16(d_pos_table) && al16(d_sep) && al16(d_patch_emb) &&
+               (reinterpret_cast<uintptr_t>(workspace) & 255) == 0,
+               "embed_bwd_ordered: gradient buffers must be 16-byte aligned, the workspace 256-byte aligned");
+  const long long n = (long long)B * (PACKED ? hp->seq_len : hp->width);
+  const int end_bit = key_bits((unsigned)(hp->vocab + 1 + hp->ctx_rows));
+  SortWs s;
+  rc = sort_ws_layout(2 * n, end_bit, workspace, s);
+  if (rc != NEKO_OK) return rc;
+  NEKO_REQUIRE(workspace_bytes >= (int64_t)s.total, "embed_bwd_ordered: workspace of %lld bytes, need %lld", (long long)workspace_bytes,
+               (long long)s.total);
+  EmbBwdArgs a;
+  a.descs = descs; a.B = B; a.d = d; a.p = *hp; a.tokens = tokens; a.d_emb = d_token_embeddings;
+  a.d_embed_table = d_embed_table; a.d_pos_table = d_pos_table; a.d_sep = d_sep; a.d_patch_emb = d_patch_emb;
+  embed_keys_kernel<PACKED><<<(unsigned)((n * 32 + 255) / 256), 256, 0, as_stream(stream)>>>(a, s.kin, s.vin);
+  NEKO_LAUNCH_CHECK("embed_keys_kernel");
+  SegDst dst{};
+  dst.p[0] = d_embed_table; dst.p[1] = d_sep; dst.p[2] = d_pos_table;
+  dst.off[0] = 0; dst.off[1] = hp->vocab; dst.off[2] = hp->vocab + 1; dst.off[3] = hp->vocab + 1 + hp->ctx_rows;
+  return sort_and_segsum(s, 2 * n, end_bit, d_token_embeddings, d, dst, as_stream(stream));
+}
+
 }  // namespace neko
 
 extern "C" {
+
+int64_t neko_embed_bwd_ordered_workspace_bytes(int B, const neko_tok_params* host_params) {
+  using namespace neko;
+  const int rc = embed_ord_check(host_params, B);
+  if (rc != NEKO_OK) return rc;
+  SortWs s;
+  const int r2 = sort_ws_layout(2LL * B * host_params->width, key_bits((unsigned)(host_params->vocab + 1 + host_params->ctx_rows)), nullptr, s);
+  if (r2 != NEKO_OK) return r2;
+  return (int64_t)s.total;
+}
+
+int neko_embed_bwd_ordered(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp, const int64_t* tokens,
+                           const float* d_token_embeddings, float* d_embed_table, float* d_pos_table, float* d_sep, float* d_patch_emb,
+                           void* workspace, int64_t workspace_bytes, void* stream) {
+  return neko::embed_bwd_ordered<false>(descs, B, d, hp, tokens, d_token_embeddings, d_embed_table, d_pos_table, d_sep, d_patch_emb,
+                                        workspace, workspace_bytes, stream);
+}
+
+int neko_embed_packed_bwd_ordered(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp, const int64_t* tokens,
+                                  const float* d_token_embeddings, float* d_embed_table, float* d_pos_table, float* d_sep,
+                                  float* d_patch_emb, void* workspace, int64_t workspace_bytes, void* stream) {
+  return neko::embed_bwd_ordered<true>(descs, B, d, hp, tokens, d_token_embeddings, d_embed_table, d_pos_table, d_sep, d_patch_emb,
+                                       workspace, workspace_bytes, stream);
+}
 
 int neko_tokenize_embed_fwd(const neko_sample_desc* descs, int B, int d, const neko_tok_params* hp,
                             const float* fvals, const int32_t* ivals, const float* patch_emb,

@@ -62,6 +62,16 @@ class GradSynchronizer:
         # of the mix produces text tokens): averaging zeros is a no-op, so they are left out of the all-reduce
         self.skip_ranges: List[Tuple[int, int]] = []
 
+    def require_deterministic(self):
+        """Deterministic training mode (GatoPolicy.deterministic): every rank must end with the same bits on every run.  The
+        p2p exchanges sum the ranks in a fixed order; NCCL's all-reduce promises no order, so it is refused."""
+        if self.world > 1 and self.backend != "p2p":
+            raise ValueError(f"deterministic mode needs the p2p data-parallel backend (got {self.backend!r}): NCCL's all-reduce "
+                             "does not sum the ranks in a fixed order, so runs would not be bitwise reproducible")
+        if self.world > 1 and self.nccl_tail:
+            raise ValueError("deterministic mode cannot be combined with NEKO_DP_NCCL_TAIL=1: the tail of the exchange would go "
+                             "through NCCL, whose all-reduce does not sum the ranks in a fixed order")
+
     # -- hook called by the backward engine -----------------------------------------------------------
     def on_range_ready(self, lo: int, hi: int):
         if not self.enabled or self.world == 1:
@@ -494,6 +504,8 @@ def attach(policy, group=None, bucket_bytes: int = 64 << 20, no_text_tokens: boo
     last, non-overlappable bucket -- then have zero gradient everywhere and are left out of the all-reduce, like the
     never-used ``transformer.wte``.  The result is identical to the dense all-reduce."""
     sync = GradSynchronizer(policy._grad_arena, group=group, bucket_bytes=bucket_bytes, mode=mode, compress=compress, backend=backend)
+    if getattr(policy, "deterministic", False):
+        sync.require_deterministic()
     if sync.backend == "p2p" and sync.world > 1:
         sync._p2p = _P2PState(policy._grad_arena, group)     # collective: map the peers' arenas now, not inside backward
     if no_text_tokens:

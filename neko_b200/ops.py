@@ -16,7 +16,7 @@ from ._lib import (EPI_BF16, EPI_DGELU_BF16, EPI_F32, EPI_GELU_BF16, EPI_RESID_F
 
 
 _16BIT = (torch.bfloat16, torch.float16)
-GEMM_A_F16, GEMM_B_F16, GEMM_C_F16, GEMM_C2_F16, GEMM_GELU_TANH = 1, 2, 4, 8, 16
+GEMM_A_F16, GEMM_B_F16, GEMM_C_F16, GEMM_C2_F16, GEMM_GELU_TANH, GEMM_DETERMINISTIC = 1, 2, 4, 8, 16, 32
 GEMM_TIMING = None  # list collecting (start_event, end_event, flops) per launch when set by bench.py
 
 
@@ -48,7 +48,8 @@ def _gemm_workspace(device):
     return ws
 
 
-def _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop, gelu_tanh):
+def _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop, gelu_tanh,
+               deterministic=False):
     """neko_gemm_desc of one gemm() / gemm_plan() call, allocating the outputs that were not given."""
     _cuda(a, b, out, out2, out3, bias, aux)
     assert a.dtype in _16BIT and b.dtype == a.dtype, "A and B must share one 16-bit format"
@@ -69,6 +70,7 @@ def _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulat
     flags |= GEMM_C_F16 if out.dtype == torch.float16 else 0
     flags |= GEMM_C2_F16 if (out2 is not None and out2.dtype == torch.float16) else 0
     flags |= GEMM_GELU_TANH if gelu_tanh else 0   # GELU / GELU' epilogues: tanh form ("gelu_new")
+    flags |= GEMM_DETERMINISTIC if deterministic else 0   # no split-K / stream-K: bitwise reproducible
     gd = GemmDesc(M=M, N=N, K=K, a_mn=int(a_mn), b_mn=int(b_mn), epilogue=epilogue, accumulate=int(accumulate), flags=flags,
                   A=a.data_ptr(), lda=a.stride(0), B=b.data_ptr(), ldb=b.stride(0), C=out.data_ptr(), ldc=out.stride(0),
                   C2=_ptr(out2), ldc2=out2.stride(0) if out2 is not None else 0,
@@ -86,13 +88,14 @@ def gemm(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: bool = F
          out: Optional[torch.Tensor] = None, out2: Optional[torch.Tensor] = None, out3: Optional[torch.Tensor] = None,
          bias: Optional[torch.Tensor] = None, aux: Optional[torch.Tensor] = None, accumulate: bool = False,
          M: Optional[int] = None, N: Optional[int] = None, K: Optional[int] = None,
-         out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False):
-    """C[M,N] = epilogue(sum_k A[m,k] B[n,k]).
+         out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False,
+         deterministic: bool = False):
+    """C[M,N] = epilogue(sum_k A[m,k] B[n,k]).  deterministic: NEKO_GEMM_DETERMINISTIC (one CTA sums each element in k order).
 
     a: 16-bit [M,K] (a_mn=False) or [K,M] (a_mn=True); b: same format, [N,K] or [K,N]; rows may be strided
     (stride(0) is the leading dimension)."""
     gd, out, out2 = _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop,
-                               gelu_tanh)
+                               gelu_tanh, deterministic)
     if GEMM_TIMING is not None:  # bench.py: CUDA events around every tensor-core launch (roofline.achieved)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
@@ -110,11 +113,12 @@ def gemm_plan(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: boo
               out: Optional[torch.Tensor] = None, out2: Optional[torch.Tensor] = None, out3: Optional[torch.Tensor] = None,
               bias: Optional[torch.Tensor] = None, aux: Optional[torch.Tensor] = None, accumulate: bool = False,
               M: Optional[int] = None, N: Optional[int] = None, K: Optional[int] = None,
-              out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False) -> dict:
+              out_dtype: torch.dtype = torch.bfloat16, drop: Optional[Dropout] = None, gelu_tanh: bool = False,
+              deterministic: bool = False) -> dict:
     """The schedule gemm() would launch with the same arguments (neko_gemm_plan_info as a dict); launches nothing.
     Raises NekoError where gemm() would reject the arguments."""
     gd, _, _ = _gemm_args(a, b, a_mn, b_mn, epilogue, out, out2, out3, bias, aux, accumulate, M, N, K, out_dtype, drop,
-                          gelu_tanh)
+                          gelu_tanh, deterministic)
     info = GemmPlanInfo()
     check(load().neko_gemm_plan(C.byref(gd), C.byref(info)), "neko_gemm_plan")
     return {name: getattr(info, name) for name, _ in GemmPlanInfo._fields_}
@@ -387,3 +391,86 @@ def adamw_step(param, grad, exp_avg, exp_avg_sq, lr, beta1, beta2, eps, weight_d
                                  C.c_float(beta1), C.c_float(beta2), C.c_float(eps), C.c_float(weight_decay), C.c_int(step),
                                  _p(grad_sumsq), C.c_float(max_norm), C.c_float(grad_div), _p(w_f16), _p(w_bf16), C.c_int64(n_cast),
                                  stream_ptr()), "neko_adamw_step")
+
+
+# ------------------------------------------------------------------------------------------
+# ordered reductions (deterministic training mode): same results as their default twins up to reassociation, with every sum in
+# a fixed order.  `ws` is a device tensor of at least the matching *_workspace_bytes() bytes.
+# ------------------------------------------------------------------------------------------
+def _ws_bytes(rc: int, what: str) -> int:
+    if rc < 0:
+        check(int(rc), what)
+    return int(rc)
+
+
+def layernorm_bwd_ordered_workspace_bytes(N: int, d: int) -> int:
+    return _ws_bytes(load().neko_layernorm_bwd_ordered_workspace_bytes(C.c_int(N), C.c_int(d)), "neko_layernorm_bwd_ordered_workspace_bytes")
+
+
+def layernorm_bwd_ordered(dy_bf16, x, gamma, mean, rstd, dx_resid, dgamma, dbeta, ws, dx_bf16=None, dx_colsum=None, branch_drop=None):
+    N, d = x.shape
+    check(load().neko_layernorm_bwd_ordered(_p(dy_bf16), _p(x), _p(gamma), _p(mean), _p(rstd), _p(dx_resid), _p(dx_bf16), _p(dgamma),
+                                            _p(dbeta), _p(dx_colsum), C.c_int(N), C.c_int(d), _dref(branch_drop), _p(ws),
+                                            C.c_int64(ws.numel() * ws.element_size()), stream_ptr()), "neko_layernorm_bwd_ordered")
+
+
+def colsum_ordered_workspace_bytes(M: int, N: int) -> int:
+    return _ws_bytes(load().neko_colsum_bf16_ordered_workspace_bytes(C.c_int(M), C.c_int(N)), "neko_colsum_bf16_ordered_workspace_bytes")
+
+
+def colsum_ordered(x_bf16: torch.Tensor, out: torch.Tensor, ws: torch.Tensor, accumulate: bool = False):
+    M, N = x_bf16.shape
+    check(load().neko_colsum_bf16_ordered(_p(x_bf16), C.c_int64(x_bf16.stride(0)), C.c_int(M), C.c_int(N), _p(out),
+                                          C.c_int(int(accumulate)), _p(ws), C.c_int64(ws.numel() * ws.element_size()), stream_ptr()),
+          "neko_colsum_bf16_ordered")
+    return out
+
+
+def embed_bwd_ordered_workspace_bytes(B: int, prm: TokParams) -> int:
+    return _ws_bytes(load().neko_embed_bwd_ordered_workspace_bytes(C.c_int(B), C.byref(prm)), "neko_embed_bwd_ordered_workspace_bytes")
+
+
+def embed_bwd_ordered(descs, B: int, d: int, prm: TokParams, tokens, d_emb, d_embed_table, d_pos_table, d_sep, ws, d_patch_emb=None,
+                      packed: bool = False):
+    fn = load().neko_embed_packed_bwd_ordered if packed else load().neko_embed_bwd_ordered
+    check(fn(_p(descs), C.c_int(B), C.c_int(d), C.byref(prm), _p(tokens), _p(d_emb), _p(d_embed_table), _p(d_pos_table), _p(d_sep),
+             _p(d_patch_emb), _p(ws), C.c_int64(ws.numel() * ws.element_size()), stream_ptr()),
+          "neko_embed_packed_bwd_ordered" if packed else "neko_embed_bwd_ordered")
+
+
+def patch_resblock_bwd_ordered_workspace_bytes(n_img: int, height: int, width: int, patch: int) -> int:
+    return _ws_bytes(load().neko_patch_resblock_bwd_ordered_workspace_bytes(C.c_int(n_img), C.c_int(height), C.c_int(width), C.c_int(patch)),
+                     "neko_patch_resblock_bwd_ordered_workspace_bytes")
+
+
+def patch_resblock_bwd_ordered(images, is_u8: bool, n_img: int, height: int, width: int, patch: int, C_mid: int, groups: int, conv1_w,
+                               conv1_b, gn_w, gn_b, conv2_w, gn_stats, d_patches_bf16, d_conv1_w, d_conv1_b, d_gn_w, d_gn_b, d_conv2_w,
+                               d_conv2_b, ws):
+    check(load().neko_patch_resblock_bwd_ordered(_p(images), C.c_int(int(is_u8)), C.c_int(n_img), C.c_int(height), C.c_int(width),
+                                                 C.c_int(patch), C.c_int(C_mid), C.c_int(groups), _p(conv1_w), _p(conv1_b), _p(gn_w),
+                                                 _p(gn_b), _p(conv2_w), _p(gn_stats), _p(d_patches_bf16), _p(d_conv1_w), _p(d_conv1_b),
+                                                 _p(d_gn_w), _p(d_gn_b), _p(d_conv2_w), _p(d_conv2_b), _p(ws),
+                                                 C.c_int64(ws.numel() * ws.element_size()), stream_ptr()),
+          "neko_patch_resblock_bwd_ordered")
+
+
+def patch_pos_bwd_ordered_workspace_bytes(P: int, n_row_bins: int, n_col_bins: int) -> int:
+    return _ws_bytes(load().neko_patch_pos_bwd_ordered_workspace_bytes(C.c_int(P), C.c_int(n_row_bins), C.c_int(n_col_bins)),
+                     "neko_patch_pos_bwd_ordered_workspace_bytes")
+
+
+def patch_pos_bwd_ordered(dx, row_bin, col_bin, d_row_tab, d_col_tab, ws):
+    P, d = dx.shape
+    check(load().neko_patch_pos_bwd_ordered(_p(dx), C.c_int(P), C.c_int(d), _p(row_bin), _p(col_bin), _p(d_row_tab),
+                                            C.c_int(d_row_tab.shape[0]), _p(d_col_tab), C.c_int(d_col_tab.shape[0]), _p(ws),
+                                            C.c_int64(ws.numel() * ws.element_size()), stream_ptr()), "neko_patch_pos_bwd_ordered")
+
+
+def sumsq_ordered_workspace_bytes(n: int) -> int:
+    return _ws_bytes(load().neko_sumsq_f32_ordered_workspace_bytes(C.c_int64(n)), "neko_sumsq_f32_ordered_workspace_bytes")
+
+
+def sumsq_ordered(x: torch.Tensor, out: torch.Tensor, ws: torch.Tensor):
+    check(load().neko_sumsq_f32_ordered(_p(x), C.c_int64(x.numel()), _p(out), _p(ws), C.c_int64(ws.numel() * ws.element_size()),
+                                        stream_ptr()), "neko_sumsq_f32_ordered")
+    return out

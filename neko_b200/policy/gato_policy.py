@@ -16,6 +16,7 @@ Design (see DESIGN.md):
 from __future__ import annotations
 
 import ctypes as C
+import gc
 import math
 import weakref
 from typing import Dict, List, Optional, Union
@@ -35,9 +36,20 @@ def _pad_to(n: int, m: int) -> int:
     return (n + m - 1) // m * m
 
 
+def _before_capture():
+    """Run before every CUDA-graph capture.  A dropped graph entry (workspace epoch change, cache eviction, a policy that went
+    out of scope) keeps its CUDAGraph alive in a reference cycle (entry <-> captured state) until the cyclic collector runs;
+    if that happens in the middle of a capture, destroying the graph there invalidates the capture.  torch no longer collects
+    before a capture, so collect here, then drain the device."""
+    gc.collect()
+    torch.cuda.synchronize()
+
+
 # --------------------------------------------------------------------------------------------------
 # parameter containers with the reference's module tree (trajectory_gpt2.py:120-359, 535-550)
 # --------------------------------------------------------------------------------------------------
+
+
 class _Conv1D(nn.Module):
     """HF Conv1D: weight [in, out], y = x @ W + b; N(0, 0.02) / zeros (trajectory_gpt2.py:375-386)."""
 
@@ -319,6 +331,11 @@ class GatoPolicy(nn.Module):
         # invisible to valid rows).  Opt-in: the embedding / residual dropout masks are drawn at packed row coordinates, a
         # different random stream from the padded layout's (the attention-dropout masks are the same).
         self.pack_sequences = False
+        # deterministic: every floating-point reduction of a training step runs in a fixed order that depends on the inputs and
+        # shapes only (ordered column sums, sorted embedding scatter, chunked patch backward, GEMMs without split-K / stream-K,
+        # ordered gradient norm), so two runs with the same seed give the same bits whatever the grid, SM count or timing
+        # (DESIGN.md "Deterministic training mode").  Differs from the default mode by reassociation only.
+        self.deterministic = False
         self.lean_logits_f16 = True     # ... and, when gradients are wanted, those logits live in fp16 between head GEMM and fused CE
         self.mlp_proj_bf16 = False      # training forward: mlp down-projection on the bf16 activation twin (see _decoder)
         # 16-bit format of the FORWARD operands (activations fed to GEMMs, weight copy).  fp16 has 3 more mantissa
@@ -532,6 +549,30 @@ class GatoPolicy(nn.Module):
             self._ws[name] = t
             self._ws_epoch = getattr(self, "_ws_epoch", 0) + 1   # captured graphs hold raw pointers: invalidate them
         return t[:n].view(*shape)
+
+    # -- deterministic mode: the ordered twins of the reducing kernels --------------------------------
+    def _ordered_ws(self, nbytes: int) -> torch.Tensor:
+        """Scratch of the ordered reductions: one buffer for all of them (they run in stream order).  The eager first sight
+        of a plan grows it to the step's largest need, so captured graphs see one stable pointer."""
+        return self._buf("ordered_ws", (max(int(nbytes), 256),), torch.uint8)
+
+    def _gemm(self, *args, **kw):
+        return ops.gemm(*args, deterministic=self.deterministic, **kw)
+
+    def _ln_bwd(self, dy, x, gamma, mean, rstd, dx, dgamma, dbeta, dxb, dx_colsum=None, branch_drop=None):
+        if self.deterministic:
+            ws = self._ordered_ws(ops.layernorm_bwd_ordered_workspace_bytes(*x.shape))
+            ops.layernorm_bwd_ordered(dy, x, gamma, mean, rstd, dx, dgamma, dbeta, ws, dx_bf16=dxb, dx_colsum=dx_colsum,
+                                      branch_drop=branch_drop)
+        else:
+            ops.layernorm_bwd(dy, x, gamma, mean, rstd, dx, dgamma, dbeta, dxb, dx_colsum=dx_colsum, branch_drop=branch_drop)
+
+    def _colsum(self, x_bf16, out):
+        """out += column sums of x_bf16 (bias gradients)."""
+        if self.deterministic:
+            ops.colsum_ordered(x_bf16, out, self._ordered_ws(ops.colsum_ordered_workspace_bytes(*x_bf16.shape)), accumulate=True)
+        else:
+            ops.colsum(x_bf16, out, accumulate=True)
 
     # ------------------------------------------------------------------------------------------
     # public API
@@ -912,11 +953,11 @@ class GatoPolicy(nn.Module):
                   "neko_patch_resblock_fwd")
             out = pe[row0:row0 + P]
             if self.fwd_dtype == torch.float16:
-                ops.gemm(patches, self._wview("image_embedding.post_embedding_projection.weight"), epilogue=ops.EPI_F32,
-                         out=out, bias=ie.post_embedding_projection.bias)
+                self._gemm(patches, self._wview("image_embedding.post_embedding_projection.weight"), epilogue=ops.EPI_F32,
+                           out=out, bias=ie.post_embedding_projection.bias)
             else:
-                ops.gemm(patches_b, self._wview("image_embedding.post_embedding_projection.weight", bwd=True), epilogue=ops.EPI_F32,
-                         out=out, bias=ie.post_embedding_projection.bias)
+                self._gemm(patches_b, self._wview("image_embedding.post_embedding_projection.weight", bwd=True), epilogue=ops.EPI_F32,
+                           out=out, bias=ie.post_embedding_projection.bias)
             self.launches += 2
             st.img_groups.append((gi, g, buf, patches_b, stats, row0, P))
             if st.dev_row_bins is not None:
@@ -1064,7 +1105,7 @@ class GatoPolicy(nn.Module):
             r1 = self._buf("r1" + tag, (N,), torch.float32)
             ops.layernorm_fwd(x, blk.ln_1.weight, blk.ln_1.bias, eps, ln1, m1, r1, y2=ln1_b if dual else None)
             qkv = self._buf("qkv" + tag, (N, 3 * d), torch.bfloat16)
-            ops.gemm(ln1, self._wview(pre + "attn.c_attn.weight"), b_mn=True, epilogue=ops.EPI_BF16, out=qkv, bias=blk.attn.c_attn.bias)
+            self._gemm(ln1, self._wview(pre + "attn.c_attn.weight"), b_mn=True, epilogue=ops.EPI_BF16, out=qkv, bias=blk.attn.c_attn.bias)
             att, att_b = pair("att", tag, (N, d))
             lse = self._buf("lse" + tag, (H, N) if packed else (B, H, W), torch.float32)
             kv = getattr(st, "kv", None)
@@ -1083,8 +1124,8 @@ class GatoPolicy(nn.Module):
                     kv.k[i, :W].copy_(qkv[:W, d:2 * d])
                     kv.v[i, :W].copy_(qkv[:W, 2 * d:])
             x1 = self._buf(f"x.{2 * i + 1}" if keep else "x.b", (N, d), torch.float32)
-            ops.gemm(att, self._wview(pre + "attn.c_proj.weight"), b_mn=True, epilogue=ops.EPI_RESID_F32, out=x1, aux=x,
-                     bias=blk.attn.c_proj.bias, drop=self._drop_site(st, 4 * i + 2, blk.attn.resid_dropout.p))
+            self._gemm(att, self._wview(pre + "attn.c_proj.weight"), b_mn=True, epilogue=ops.EPI_RESID_F32, out=x1, aux=x,
+                       bias=blk.attn.c_proj.bias, drop=self._drop_site(st, 4 * i + 2, blk.attn.resid_dropout.p))
             ln2, ln2_b = pair("ln2", tag, (N, d))
             m2 = self._buf("m2" + tag, (N,), torch.float32)
             r2 = self._buf("r2" + tag, (N,), torch.float32)
@@ -1097,23 +1138,23 @@ class GatoPolicy(nn.Module):
             # the bf16 twin (and the bf16 weight copy) and the fp16 tensor is never written.
             lowp = dual and self.mlp_proj_bf16 and not gate
             if lowp:
-                ops.gemm(ln2, self._wview(pre + "mlp.c_fc.weight"), b_mn=True, epilogue=ops.EPI_GELU_BF16, out=fpre, out2=fact_b,
-                         bias=blk.mlp.c_fc.bias, gelu_tanh=self._gelu_tanh)
+                self._gemm(ln2, self._wview(pre + "mlp.c_fc.weight"), b_mn=True, epilogue=ops.EPI_GELU_BF16, out=fpre, out2=fact_b,
+                           bias=blk.mlp.c_fc.bias, gelu_tanh=self._gelu_tanh)
             elif not gate:
-                ops.gemm(ln2, self._wview(pre + "mlp.c_fc.weight"), b_mn=True, epilogue=ops.EPI_GELU_BF16, out=fpre, out2=fact,
-                         out3=fact_b if dual else None, bias=blk.mlp.c_fc.bias, gelu_tanh=self._gelu_tanh)
+                self._gemm(ln2, self._wview(pre + "mlp.c_fc.weight"), b_mn=True, epilogue=ops.EPI_GELU_BF16, out=fpre, out2=fact,
+                           out3=fact_b if dual else None, bias=blk.mlp.c_fc.bias, gelu_tanh=self._gelu_tanh)
             else:   # geglu: h = gelu(c_fc(x)) * gated_layer(x)   (trajectory_gpt2.py:267-276; nn.Linear weight is [out, in])
                 gelu_o = self._buf("fgelu", (N, 4 * d), fdt)
-                ops.gemm(ln2, self._wview(pre + "mlp.c_fc.weight"), b_mn=True, epilogue=ops.EPI_GELU_BF16, out=fpre, out2=gelu_o,
-                         bias=blk.mlp.c_fc.bias)
+                self._gemm(ln2, self._wview(pre + "mlp.c_fc.weight"), b_mn=True, epilogue=ops.EPI_GELU_BF16, out=fpre, out2=gelu_o,
+                           bias=blk.mlp.c_fc.bias)
                 fgate = self._buf("fgate" + tag, (N, 4 * d), torch.bfloat16)
-                ops.gemm(ln2, self._wview(pre + "mlp.gated_layer.weight"), epilogue=ops.EPI_BF16, out=fgate,
-                         bias=blk.mlp.gated_layer.bias)
+                self._gemm(ln2, self._wview(pre + "mlp.gated_layer.weight"), epilogue=ops.EPI_BF16, out=fgate,
+                           bias=blk.mlp.gated_layer.bias)
                 ops.geglu_fwd(gelu_o, fgate, fact, fact_b if dual else None)
                 self.launches += 2
             x2 = self._buf(f"x.{2 * i + 2}" if keep else "x.a", (N, d), torch.float32)
-            ops.gemm(fact_b if lowp else fact, self._wview(pre + "mlp.c_proj.weight", bwd=lowp), b_mn=True, epilogue=ops.EPI_RESID_F32,
-                     out=x2, aux=x1, bias=blk.mlp.c_proj.bias, drop=self._drop_site(st, 4 * i + 3, blk.mlp.dropout.p))
+            self._gemm(fact_b if lowp else fact, self._wview(pre + "mlp.c_proj.weight", bwd=lowp), b_mn=True, epilogue=ops.EPI_RESID_F32,
+                       out=x2, aux=x1, bias=blk.mlp.c_proj.bias, drop=self._drop_site(st, 4 * i + 3, blk.mlp.dropout.p))
             self.launches += 7
             if keep:
                 acts.append((x, ln1_b, m1, r1, qkv, att_b, lse, x1, ln2_b, m2, r2, fpre, fact_b, fgate))
@@ -1134,10 +1175,10 @@ class GatoPolicy(nn.Module):
         cross entropy, which reads V*2 instead of V*4 bytes per row (csrc/ce.cu: ce_fused_f16_kernel)."""
         if f16:
             logits = self._buf("logits_rows_f16", (n_rows, self._Vp), torch.float16)
-            ops.gemm(hf, self._wview("predict_token.weight", rows=self._Vp), epilogue=ops.EPI_BF16, out=logits, N=self._Vp)
+            self._gemm(hf, self._wview("predict_token.weight", rows=self._Vp), epilogue=ops.EPI_BF16, out=logits, N=self._Vp)
         else:
             logits = torch.empty(n_rows, self._Vp, dtype=torch.float32, device=self.device)
-            ops.gemm(hf, self._wview("predict_token.weight", rows=self._Vp), epilogue=ops.EPI_F32, out=logits, N=self._Vp)
+            self._gemm(hf, self._wview("predict_token.weight", rows=self._Vp), epilogue=ops.EPI_F32, out=logits, N=self._Vp)
         self.launches += 1
         return logits
 
@@ -1172,7 +1213,8 @@ class GatoPolicy(nn.Module):
         p = st.plan
         return (p.B, p.seq_len, p.width, p.descs.tobytes(), tuple((g.height, g.width, g.is_u8, g.n_frames) for g in p.image_groups),
                 len(p.precomputed_patch), st.compute_loss, st.need_grad, self.training, self.materialize_logits, self.head_mode,
-                self.fwd_dtype, st.row_bins is not None, self._dropout_ps(), self.lean_logits_f16, self.mlp_proj_bf16, p.packed)
+                self.fwd_dtype, st.row_bins is not None, self._dropout_ps(), self.lean_logits_f16, self.mlp_proj_bf16,
+                self.deterministic, p.packed)
 
     def _engine_forward(self, st: _State):
         if not self.use_cuda_graphs:
@@ -1195,7 +1237,7 @@ class GatoPolicy(nn.Module):
             st.graph_entry = None
             return out
         if "fwd" not in ent:                  # second sight: capture
-            torch.cuda.synchronize()
+            _before_capture()
             l0 = self.launches
             gph = torch.cuda.CUDAGraph()
             if self._graph_pool is None:
@@ -1318,7 +1360,7 @@ class GatoPolicy(nn.Module):
             acc = (acc, bool(sync.enabled))    # no_sync() micro-steps replay a graph without the all-reduces
         gb = ent["bwd"].get(acc)
         if gb is None:
-            torch.cuda.synchronize()
+            _before_capture()
             l0 = self.launches
             gph = torch.cuda.CUDAGraph()
             self._capturing = True
@@ -1346,6 +1388,8 @@ class GatoPolicy(nn.Module):
         if sync is not None and getattr(sync, "mode", "overlap") == "tail":
             sync = None
         if sync is not None:
+            if self.deterministic:
+                sync.require_deterministic()
             sync.begin_step()
         if acc_override is None:
             acc = self._begin_grads(bool(plan.n_patch_rows and getattr(st, 'img_groups', None)))
@@ -1370,11 +1414,11 @@ class GatoPolicy(nn.Module):
                 ops.masked_ce_bwd(st.logits_full, V, st.loss_rows, st.tokens, st.row_lse, gscale, dl, flags=flags)
             hc = self._buf("hf_rows_b", (n_rows, d), torch.bfloat16)
             ops.gather_rows(st.hf, st.loss_rows, d, hc)
-            ops.gemm(dl, hc, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G("predict_token.weight"), accumulate=acc,
-                     M=V, N=d, K=n_rows)
+            self._gemm(dl, hc, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G("predict_token.weight"), accumulate=acc,
+                       M=V, N=d, K=n_rows)
             # K = the padded vocabulary (818 k-blocks), a handful of output tiles: fp32 output lets the kernel split K
             dhc32 = self._buf("dhf_rows_f32", (n_rows, d), torch.float32)
-            ops.gemm(dl, Wb("predict_token.weight", rows=Vp), b_mn=True, epilogue=ops.EPI_F32, out=dhc32, M=n_rows, N=d, K=Vp)
+            self._gemm(dl, Wb("predict_token.weight", rows=Vp), b_mn=True, epilogue=ops.EPI_F32, out=dhc32, M=n_rows, N=d, K=Vp)
             dhc = self._buf("dhf_rows", (n_rows, d), torch.bfloat16)
             ops.cast_bf16(dhc32, dhc)
             dhf = self._buf("dhf", (N, d), torch.bfloat16)
@@ -1385,11 +1429,11 @@ class GatoPolicy(nn.Module):
             dl = self._buf("dlogits", (N, Vp), torch.bfloat16)
             dl.zero_()
             ops.masked_ce_bwd(st.logits_full, V, st.loss_rows, st.tokens, st.row_lse, gscale, dl)
-            ops.gemm(dl, st.hf, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G("predict_token.weight"), accumulate=acc,
-                     M=V, N=d, K=N)
+            self._gemm(dl, st.hf, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G("predict_token.weight"), accumulate=acc,
+                       M=V, N=d, K=N)
             # K = the padded vocabulary (818 k-blocks) but only 360 output tiles: fp32 output lets the kernel split K
             dhf32 = self._buf("dhf_f32", (N, d), torch.float32)
-            ops.gemm(dl, Wb("predict_token.weight", rows=Vp), b_mn=True, epilogue=ops.EPI_F32, out=dhf32, M=N, N=d, K=Vp)
+            self._gemm(dl, Wb("predict_token.weight", rows=Vp), b_mn=True, epilogue=ops.EPI_F32, out=dhf32, M=N, N=d, K=Vp)
             dhf = self._buf("dhf", (N, d), torch.bfloat16)
             ops.cast_bf16(dhf32, dhf)
             self.launches += 6
@@ -1407,8 +1451,8 @@ class GatoPolicy(nn.Module):
         # residual branch below this LN (branch_drop); the fp32 dx keeps the undropped residual-path gradient.
         D = lambda s, pp: self._drop_site(st, s, pp)  # noqa: E731
         hL = self.transformer.h[self.layers - 1]
-        ops.layernorm_bwd(dhf, st.x_last, lnf.weight, st.mf, st.rf, dx, G("transformer.ln_f.weight"), G("transformer.ln_f.bias"), dxb,
-                          dx_colsum=G(last + "mlp.c_proj.bias"), branch_drop=D(4 * (self.layers - 1) + 3, hL.mlp.dropout.p))
+        self._ln_bwd(dhf, st.x_last, lnf.weight, st.mf, st.rf, dx, G("transformer.ln_f.weight"), G("transformer.ln_f.bias"), dxb,
+                     dx_colsum=G(last + "mlp.c_proj.bias"), branch_drop=D(4 * (self.layers - 1) + 3, hL.mlp.dropout.p))
         self.launches += 2
         self._notify("transformer.ln_f.weight", "transformer.ln_f.bias")
 
@@ -1418,39 +1462,39 @@ class GatoPolicy(nn.Module):
             pre = f"transformer.h.{i}."
             (x0, ln1, m1, r1, qkv, att, lse, x1, ln2, m2, r2, fpre, fact, fgate) = st.acts[i]
             # MLP: x2 = x1 + gelu(ln2 @ Wfc + b) @ Wproj + b
-            ops.gemm(fact, dxb, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "mlp.c_proj.weight"), accumulate=acc,
-                     M=4 * d, N=d, K=N)
+            self._gemm(fact, dxb, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "mlp.c_proj.weight"), accumulate=acc,
+                       M=4 * d, N=d, K=N)
             dpre = self._buf("dfpre", (N, 4 * d), torch.bfloat16)
             dln = self._buf("dln", (N, d), torch.bfloat16)
             if fgate is None:
-                ops.gemm(dxb, Wb(pre + "mlp.c_proj.weight"), epilogue=ops.EPI_DGELU_BF16, out=dpre, aux=fpre, gelu_tanh=self._gelu_tanh)
+                self._gemm(dxb, Wb(pre + "mlp.c_proj.weight"), epilogue=ops.EPI_DGELU_BF16, out=dpre, aux=fpre, gelu_tanh=self._gelu_tanh)
             else:   # geglu: dh -> (d_gate, d_pre); the gate Linear gets its own wgrad / bias grad / dgrad
                 dh4 = self._buf("dfh", (N, 4 * d), torch.bfloat16)
-                ops.gemm(dxb, Wb(pre + "mlp.c_proj.weight"), epilogue=ops.EPI_BF16, out=dh4)
+                self._gemm(dxb, Wb(pre + "mlp.c_proj.weight"), epilogue=ops.EPI_BF16, out=dh4)
                 dgate = self._buf("dfgate", (N, 4 * d), torch.bfloat16)
                 ops.geglu_bwd(dh4, fpre, fgate, dgate, dpre)
-                ops.gemm(dgate, ln2, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "mlp.gated_layer.weight"),
-                         accumulate=True, M=4 * d, N=d, K=N)
-                ops.colsum(dgate, G(pre + "mlp.gated_layer.bias"), accumulate=True)
+                self._gemm(dgate, ln2, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "mlp.gated_layer.weight"),
+                           accumulate=True, M=4 * d, N=d, K=N)
+                self._colsum(dgate, G(pre + "mlp.gated_layer.bias"))
                 self.launches += 4
-            ops.gemm(ln2, dpre, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "mlp.c_fc.weight"), accumulate=acc,
-                     M=d, N=4 * d, K=N)
-            ops.colsum(dpre, G(pre + "mlp.c_fc.bias"), accumulate=True)
+            self._gemm(ln2, dpre, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "mlp.c_fc.weight"), accumulate=acc,
+                       M=d, N=4 * d, K=N)
+            self._colsum(dpre, G(pre + "mlp.c_fc.bias"))
             if fgate is None:
-                ops.gemm(dpre, Wb(pre + "mlp.c_fc.weight"), epilogue=ops.EPI_BF16, out=dln)
+                self._gemm(dpre, Wb(pre + "mlp.c_fc.weight"), epilogue=ops.EPI_BF16, out=dln)
             else:   # d ln2 = d_pre . Wfc^T + d_gate . Wg: two GEMMs into one fp32 buffer, then the 16-bit copy
                 dln32 = self._buf("dln_f32", (N, d), torch.float32)
-                ops.gemm(dpre, Wb(pre + "mlp.c_fc.weight"), epilogue=ops.EPI_F32, out=dln32)
-                ops.gemm(dgate, Wb(pre + "mlp.gated_layer.weight"), b_mn=True, epilogue=ops.EPI_F32, out=dln32, accumulate=True)
+                self._gemm(dpre, Wb(pre + "mlp.c_fc.weight"), epilogue=ops.EPI_F32, out=dln32)
+                self._gemm(dgate, Wb(pre + "mlp.gated_layer.weight"), b_mn=True, epilogue=ops.EPI_F32, out=dln32, accumulate=True)
                 ops.cast_bf16(dln32, dln)
                 self.launches += 2
-            ops.layernorm_bwd(dln, x1, blk.ln_2.weight, m2, r2, dx, G(pre + "ln_2.weight"), G(pre + "ln_2.bias"), dxb,
-                              dx_colsum=G(pre + "attn.c_proj.bias"), branch_drop=D(4 * i + 2, blk.attn.resid_dropout.p))
+            self._ln_bwd(dln, x1, blk.ln_2.weight, m2, r2, dx, G(pre + "ln_2.weight"), G(pre + "ln_2.bias"), dxb,
+                         dx_colsum=G(pre + "attn.c_proj.bias"), branch_drop=D(4 * i + 2, blk.attn.resid_dropout.p))
             # attention: x1 = x0 + attn(ln1 @ Wqkv + b) @ Wproj + b
-            ops.gemm(att, dxb, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "attn.c_proj.weight"), accumulate=acc,
-                     M=d, N=d, K=N)
+            self._gemm(att, dxb, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "attn.c_proj.weight"), accumulate=acc,
+                       M=d, N=d, K=N)
             datt = self._buf("datt", (N, d), torch.bfloat16)
-            ops.gemm(dxb, Wb(pre + "attn.c_proj.weight"), epilogue=ops.EPI_BF16, out=datt)
+            self._gemm(dxb, Wb(pre + "attn.c_proj.weight"), epilogue=ops.EPI_BF16, out=datt)
             dqkv = self._buf("dqkv", (N, 3 * d), torch.bfloat16)
             if plan.packed:
                 delta = self._buf("delta", (H, N), torch.float32)
@@ -1460,13 +1504,13 @@ class GatoPolicy(nn.Module):
                 delta = self._buf("delta", (B, H, W), torch.float32)
                 ops.attention_bwd(qkv.view(B, W, 3 * d), att.view(B, W, d), datt.view(B, W, d), lse, st.first_valid, H, plan.seq_len,
                                   dqkv.view(B, W, 3 * d), delta, drop=D(4 * i + 1, blk.attn.attn_dropout.p))
-            ops.gemm(ln1, dqkv, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "attn.c_attn.weight"), accumulate=acc,
-                     M=d, N=3 * d, K=N)
-            ops.colsum(dqkv, G(pre + "attn.c_attn.bias"), accumulate=True)
-            ops.gemm(dqkv, Wb(pre + "attn.c_attn.weight"), epilogue=ops.EPI_BF16, out=dln)
-            ops.layernorm_bwd(dln, x0, blk.ln_1.weight, m1, r1, dx, G(pre + "ln_1.weight"), G(pre + "ln_1.bias"), dxb,
-                              dx_colsum=G(f"transformer.h.{i - 1}.mlp.c_proj.bias") if i > 0 else None,
-                              branch_drop=D(4 * (i - 1) + 3, self.transformer.h[i - 1].mlp.dropout.p) if i > 0 else None)
+            self._gemm(ln1, dqkv, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G(pre + "attn.c_attn.weight"), accumulate=acc,
+                       M=d, N=3 * d, K=N)
+            self._colsum(dqkv, G(pre + "attn.c_attn.bias"))
+            self._gemm(dqkv, Wb(pre + "attn.c_attn.weight"), epilogue=ops.EPI_BF16, out=dln)
+            self._ln_bwd(dln, x0, blk.ln_1.weight, m1, r1, dx, G(pre + "ln_1.weight"), G(pre + "ln_1.bias"), dxb,
+                         dx_colsum=G(f"transformer.h.{i - 1}.mlp.c_proj.bias") if i > 0 else None,
+                         branch_drop=D(4 * (i - 1) + 3, self.transformer.h[i - 1].mlp.dropout.p) if i > 0 else None)
             self.launches += 14
             self._notify(pre + "mlp.c_proj.weight", pre + "ln_1.bias")
 
@@ -1479,8 +1523,13 @@ class GatoPolicy(nn.Module):
         if plan.n_patch_rows and getattr(st, "img_groups", None):
             dpe = self._buf("d_patch_emb", (plan.n_patch_rows, d), torch.float32)
             dpe.zero_()
-        ops.embed_bwd(st.descs, B, d, st.tok_params, st.tokens, dx, G("embed_token.weight"), G("pos_embed_observation.weight"),
-                      G("separator_token"), dpe, packed=plan.packed)
+        if self.deterministic:
+            ws = self._ordered_ws(ops.embed_bwd_ordered_workspace_bytes(B, st.tok_params))
+            ops.embed_bwd_ordered(st.descs, B, d, st.tok_params, st.tokens, dx, G("embed_token.weight"), G("pos_embed_observation.weight"),
+                                  G("separator_token"), ws, dpe, packed=plan.packed)
+        else:
+            ops.embed_bwd(st.descs, B, d, st.tok_params, st.tokens, dx, G("embed_token.weight"), G("pos_embed_observation.weight"),
+                          G("separator_token"), dpe, packed=plan.packed)
         self.launches += 1
         if dpe is not None:
             self._image_backward(st, dpe, acc)
@@ -1498,7 +1547,12 @@ class GatoPolicy(nn.Module):
         pp = "image_embedding.patch_embedding."
         for (gi, g, buf, patches, stats, row0, P) in st.img_groups:
             gslice = dpe[row0:row0 + P]
-            if st.row_bins is not None:
+            if st.row_bins is not None and self.deterministic:
+                rt = G("image_embedding.patch_pos_encoding.height_pos_embedding.weight")
+                ct = G("image_embedding.patch_pos_encoding.width_pos_embedding.weight")
+                ws = self._ordered_ws(ops.patch_pos_bwd_ordered_workspace_bytes(P, rt.shape[0], ct.shape[0]))
+                ops.patch_pos_bwd_ordered(gslice, st.dev_row_bins[row0:row0 + P], st.dev_col_bins[row0:row0 + P], rt, ct, ws)
+            elif st.row_bins is not None:
                 check(lib.neko_patch_pos_bwd(_p(gslice), C.c_int(P), C.c_int(d), _p(st.dev_row_bins[row0:row0 + P]),
                                              _p(st.dev_col_bins[row0:row0 + P]),
                                              _p(G("image_embedding.patch_pos_encoding.height_pos_embedding.weight")),
@@ -1506,11 +1560,19 @@ class GatoPolicy(nn.Module):
                       "neko_patch_pos_bwd")
             gb = self._buf(f"dpe_bf16_{gi}", (P, d), torch.bfloat16)
             ops.cast_bf16(gslice, gb)
-            ops.colsum(gb, G("image_embedding.post_embedding_projection.bias"), accumulate=True)
-            ops.gemm(gb, patches, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G("image_embedding.post_embedding_projection.weight"),
-                     accumulate=True, M=d, N=patches.shape[1], K=P)
+            self._colsum(gb, G("image_embedding.post_embedding_projection.bias"))
+            self._gemm(gb, patches, a_mn=True, b_mn=True, epilogue=ops.EPI_F32, out=G("image_embedding.post_embedding_projection.weight"),
+                       accumulate=True, M=d, N=patches.shape[1], K=P)
             dpatch = self._buf(f"dpatches{gi}", (P, patches.shape[1]), torch.bfloat16)
-            ops.gemm(gb, self._wview("image_embedding.post_embedding_projection.weight", bwd=True), b_mn=True, epilogue=ops.EPI_BF16, out=dpatch)
+            self._gemm(gb, self._wview("image_embedding.post_embedding_projection.weight", bwd=True), b_mn=True, epilogue=ops.EPI_BF16, out=dpatch)
+            if self.deterministic:
+                ws = self._ordered_ws(ops.patch_resblock_bwd_ordered_workspace_bytes(g.n_frames, g.height, g.width, self.patch_size))
+                ops.patch_resblock_bwd_ordered(buf, g.is_u8, g.n_frames, g.height, g.width, self.patch_size, rb.mid_channels, rb.num_groups,
+                                               rb.conv1.weight, rb.conv1.bias, rb.gn2.weight, rb.gn2.bias, rb.conv2.weight, stats, dpatch,
+                                               G(pp + "conv1.weight"), G(pp + "conv1.bias"), G(pp + "gn2.weight"), G(pp + "gn2.bias"),
+                                               G(pp + "conv2.weight"), G(pp + "conv2.bias"), ws)
+                self.launches += 6
+                continue
             check(lib.neko_patch_resblock_bwd(_p(buf), C.c_int(int(g.is_u8)), C.c_int(g.n_frames), C.c_int(g.height), C.c_int(g.width),
                                               C.c_int(self.patch_size), C.c_int(rb.mid_channels), C.c_int(rb.num_groups),
                                               _p(rb.conv1.weight), _p(rb.conv1.bias), _p(rb.gn2.weight), _p(rb.gn2.bias),

@@ -75,6 +75,7 @@ class TrainingArgs:
     synthetic: str = "cfg2"
     disable_cuda_graphs: bool = False   # replay forward / backward from CUDA graphs per batch shape (neko_b200 engine knob)
     pack_sequences: bool = False        # padding-free steps: samples back to back, variable-length attention (neko_b200 engine knob)
+    deterministic: bool = False         # bitwise-reproducible steps: fixed-order reductions in place of float atomics (engine knob)
     seed: int = 1234
 
 

@@ -91,7 +91,11 @@ class FusedAdamW:
             # ranges without a gradient hold zeros (GatoPolicy._begin_grads clears them each cycle): the norm over the whole
             # arena equals clip_grad_norm_ over the parameters that have one
             self.sumsq.zero_()
-            ops.sumsq(p._grad_arena, self.sumsq)
+            if getattr(p, "deterministic", False):   # fixed-order sum: the clip factor is bitwise reproducible
+                n = p._grad_arena.numel()
+                ops.sumsq_ordered(p._grad_arena, self.sumsq, p._buf("ordered_ws", (ops.sumsq_ordered_workspace_bytes(n),), torch.uint8))
+            else:
+                ops.sumsq(p._grad_arena, self.sumsq)
             ss = self.sumsq
         # the update also rewrites the 16-bit operand copies of the GEMM weights (fp16 forward / bf16 backward), so the
         # next forward starts without a cast kernel

@@ -44,6 +44,7 @@ def main():
     model.materialize_logits = False   # the trainer discards logits (trainer.py:178)
     model.use_cuda_graphs = not args.disable_cuda_graphs
     model.pack_sequences = args.pack_sequences
+    model.deterministic = args.deterministic   # before dp.attach: it refuses an exchange without a fixed summation order
     torch.manual_seed(args.seed + rank)     # per-rank dropout masks, patch-position draws and multinomial remainders
     sync = None
     if world > 1:
