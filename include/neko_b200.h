@@ -126,6 +126,7 @@ int neko_embed_packed_bwd(const neko_sample_desc* descs, int B, int d, const nek
 
 /* ---------------------------------------------------------------------------------------------
  * LayerNorm (ln_1 / ln_2 / ln_f, trajectory_gpt2.py:323,353,779). x fp32 [N,d] -> y bf16 (fp16 if out_f16).
+ * d % 4 == 0, d <= 2048; rows are dense (pitch d).  x, gamma, beta 16-byte aligned; y, y2 8-byte aligned.
  * ------------------------------------------------------------------------------------------- */
 int neko_layernorm_fwd(const float* x, const float* gamma, const float* beta, uint16_t* y_16,
                        uint16_t* y2_bf16 /* nullable second copy */, float* mean, float* rstd, int N, int d,
@@ -134,10 +135,27 @@ int neko_layernorm_fwd(const float* x, const float* gamma, const float* beta, ui
  * fp32 [d] are accumulated (caller zeroes them).  dx_colsum (nullable, fp32 [d], accumulated): column sums
  * of the bf16 copy = the bias gradient of the Conv1D whose output was added into this residual.
  * branch_drop (nullable): the residual branch that produced x went through dropout (x = x_prev + dropout(branch)); the
- * bf16 copy and dx_colsum then carry mask * scale * dx_resid, i.e. the gradient entering that branch. */
+ * bf16 copy and dx_colsum then carry mask * scale * dx_resid, i.e. the gradient entering that branch.
+ * x, dx_resid, gamma 16-byte aligned; dy, dx_bf16 8-byte aligned (the alignment neko_layernorm_bwd_ordered requires).
+ * Kernel: warp-per-row when d % 128 == 0 and d <= 1024; otherwise a column-owner kernel over NEKO_LN_CTAS row ranges
+ * (default 2 per SM; values below 1 keep the default): staged (cp.async.bulk ring) when d % 8 == 0, dy is 16-byte
+ * aligned and the ring has >= 2 stages, else register.  NEKO_LN_BWD_COLUMNS / NEKO_LN_BWD_REGISTER (read once per
+ * process) force the column-owner / register kernels. */
 int neko_layernorm_bwd(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean,
                        const float* rstd, float* dx_resid, uint16_t* dx_bf16, float* dgamma,
                        float* dbeta, float* dx_colsum, int N, int d, const neko_dropout* branch_drop, void* stream);
+/* The backward kernel neko_layernorm_bwd would run for these arguments (same argument checks, same environment knobs),
+ * decided on the host without launching anything: 0 = warp-per-row, 1 = staged, 2 = register, < 0 = the call is
+ * rejected.  out (nullable) receives the launch shape. */
+typedef struct neko_layernorm_bwd_path_info {
+  int32_t grid;                 /* CTAs launched                                                   */
+  int32_t rows_per_cta;         /* column-owner kernels: consecutive rows per CTA; 0 for warp-per-row (grid-stride rows) */
+  int32_t stages;               /* staged kernel: shared-memory ring depth (2..4); 0 otherwise      */
+} neko_layernorm_bwd_path_info;
+int neko_layernorm_bwd_path(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean,
+                            const float* rstd, const float* dx_resid, const uint16_t* dx_bf16, const float* dgamma,
+                            const float* dbeta, const float* dx_colsum, int N, int d, const neko_dropout* branch_drop,
+                            neko_layernorm_bwd_path_info* out);
 
 /* ---------------------------------------------------------------------------------------------
  * Dense GEMM on tcgen05 tensor cores (HF Conv1D addmm trajectory_gpt2.py:222,253,274,277;
@@ -254,6 +272,8 @@ int neko_attention_varlen_bwd(const uint16_t* qkv, const uint16_t* out, const ui
 #define NEKO_CE_LOGITS_COMPACT 1   /* logits row r (not rows[r]) holds position rows[r]            */
 #define NEKO_CE_DLOGITS_COMPACT 2  /* dlogits row r (not rows[r]) receives position rows[r]         */
 #define NEKO_CE_ZERO_PAD 4         /* bwd also zeroes dlogits columns V..ld_dlogits of the rows it writes */
+/* A target outside [0, V) (e.g. -1) is not an error: nothing outside the row is read, the row's loss is 0 (it still counts
+ * in the mean's n_rows), and its gradient row is softmax * g / n_rows with no one-hot term. */
 int neko_masked_ce_fwd(const float* logits, int64_t ld_logits, int V, const int32_t* rows, int n_rows,
                        const int64_t* tokens, float* row_lse, float* row_loss, float* loss, int flags,
                        void* stream);

@@ -65,6 +65,11 @@ class GemmPlanInfo(C.Structure):
         "BN", "pair", "splits", "epi_warps", "streamk", "tma_store", "tma_aux", "vec_ok", "n_fast", "stages")]
 
 
+class LnBwdPathInfo(C.Structure):
+    """neko_layernorm_bwd_path_info (include/neko_b200.h)."""
+    _fields_ = [(n, C.c_int32) for n in ("grid", "rows_per_cta", "stages")]
+
+
 EPI_BF16, EPI_F32, EPI_GELU_BF16, EPI_RESID_F32, EPI_DGELU_BF16, EPI_RESID_F32_BF16 = range(6)
 
 _lib = None

@@ -229,8 +229,8 @@ extern "C" {
 
 static int cast_impl(const float* src, uint16_t* dst, int64_t n, int f16, void* stream) {
   using namespace neko;
-  NEKO_REQUIRE(src && dst && n >= 0, "cast: bad arguments");
-  if (n == 0) return NEKO_OK;
+  if (n == 0) return NEKO_OK;   // an empty tensor may have no storage (null pointers): nothing to do
+  NEKO_REQUIRE(src && dst && n > 0, "cast: bad arguments");
   NEKO_REQUIRE((reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(dst) & 7) == 0, "cast: misaligned buffers");
   long long blocks = (n / 4 + 255) / 256;
   const long long cap = (long long)sm_count() * 16;
@@ -246,8 +246,8 @@ int neko_cast_f32_to_f16(const float* src, uint16_t* dst, int64_t n, void* strea
 
 int neko_cast_f32_to_f16_bf16(const float* src, uint16_t* dst_f16, uint16_t* dst_bf16, int64_t n, void* stream) {
   using namespace neko;
-  NEKO_REQUIRE(src && dst_f16 && dst_bf16 && n >= 0, "cast: bad arguments");
   if (n == 0) return NEKO_OK;
+  NEKO_REQUIRE(src && dst_f16 && dst_bf16 && n > 0, "cast: bad arguments");
   NEKO_REQUIRE((reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(dst_f16) & 7) == 0 &&
                (reinterpret_cast<uintptr_t>(dst_bf16) & 7) == 0, "cast: misaligned buffers");
   long long blocks = (n / 4 + 255) / 256;

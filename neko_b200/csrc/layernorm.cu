@@ -421,6 +421,60 @@ __global__ void __launch_bounds__(256, 2) layernorm_bwd_rows_kernel(const bf16* 
 
 }  // namespace neko
 
+namespace neko {
+
+static bool ln_al(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; }
+
+// Argument checks and kernel choice of neko_layernorm_bwd, shared with neko_layernorm_bwd_path so that the query reports
+// exactly what a launch runs.  Touches no device state beyond sm_count().
+struct LnBwdPlan {
+  int kernel;          // 0 warp-per-row, 1 staged, 2 register (column-owner kernels)
+  int grid, threads, rows_per_cta, stages;
+  size_t smem;
+};
+
+static int ln_bwd_plan(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean, const float* rstd,
+                       const float* dx_resid, const uint16_t* dx_bf16, const float* dgamma, const float* dbeta, int N, int d,
+                       LnBwdPlan& p) {
+  NEKO_REQUIRE(dy_bf16 && x && gamma && mean && rstd && dx_resid && dgamma && dbeta, "layernorm_bwd: null pointer");
+  NEKO_REQUIRE(N > 0 && d > 0 && d % 4 == 0 && d <= LN_MAX_D, "layernorm_bwd: need d %% 4 == 0 and d <= %d (got %d)", LN_MAX_D, d);
+  NEKO_REQUIRE(ln_al(x, 16) && ln_al(dx_resid, 16) && ln_al(gamma, 16) && ln_al(dy_bf16, 8) && ln_al(dx_bf16, 8),
+               "layernorm_bwd: x, dx_resid and gamma must be 16-byte aligned, dy and dx_bf16 8-byte aligned");
+  // warp-per-row variant (default): d = 128 * NV with NV <= 8
+  static const bool force_cols = getenv("NEKO_LN_BWD_COLUMNS") != nullptr;
+  if (!force_cols && d % 128 == 0 && d <= 1024) {
+    int grid = 2 * sm_count();                                       // two CTAs per SM
+    const int rows_per_grid = grid * 8;
+    if (N < rows_per_grid) grid = (N + 7) / 8;
+    p = LnBwdPlan{0, grid, 256, 0, 0, (size_t)(1 + 8 * 3) * d * sizeof(float)};   // gamma + 8 warps x 3 accumulator rows
+    return NEKO_OK;
+  }
+  // column-owner kernels: one float4 column group per thread, a CTA owns rows_per_cta consecutive rows.
+  // ~2 CTAs per SM: enough loads in flight (12 per thread), few enough CTAs that the final atomics stay cheap
+  int ctas = sm_count() * 2;
+  if (const char* e = getenv("NEKO_LN_CTAS")) {   // values below 1 (or not a number) keep the default
+    const int v = atoi(e);
+    if (v >= 1) ctas = v;
+  }
+  int rows_per_cta = (N + ctas - 1) / ctas;
+  rows_per_cta = ((rows_per_cta + LNB_ROWS - 1) / LNB_ROWS) * LNB_ROWS;
+  ctas = (N + rows_per_cta - 1) / rows_per_cta;
+  const int threads = ((d / 4 + 31) / 32) * 32;
+  // staged variant: ring of `stages` row blocks (40 d bytes each) in shared memory, two CTAs per SM
+  const size_t stage_bytes = (size_t)LNB_ROWS * d * 10;
+  int stages = (int)((100 * 1024) / stage_bytes);
+  if (stages > 4) stages = 4;
+  static const bool force_reg = getenv("NEKO_LN_BWD_REGISTER") != nullptr;
+  if (stages >= 2 && d % 8 == 0 && ln_al(dy_bf16, 16) && !force_reg) {
+    p = LnBwdPlan{1, ctas, threads, rows_per_cta, stages, stage_bytes * stages};
+    return NEKO_OK;
+  }
+  p = LnBwdPlan{2, ctas, threads, rows_per_cta, 0, 0};
+  return NEKO_OK;
+}
+
+}  // namespace neko
+
 extern "C" {
 
 int neko_layernorm_fwd(const float* x, const float* gamma, const float* beta, uint16_t* y_bf16, uint16_t* y2_bf16, float* mean,
@@ -428,6 +482,8 @@ int neko_layernorm_fwd(const float* x, const float* gamma, const float* beta, ui
   using namespace neko;
   NEKO_REQUIRE(x && gamma && beta && y_bf16 && mean && rstd, "layernorm_fwd: null pointer");
   NEKO_REQUIRE(N > 0 && d > 0 && d % 4 == 0 && d <= LN_MAX_D, "layernorm_fwd: need d %% 4 == 0 and d <= %d (got %d)", LN_MAX_D, d);
+  NEKO_REQUIRE(ln_al(x, 16) && ln_al(gamma, 16) && ln_al(beta, 16) && ln_al(y_bf16, 8) && ln_al(y2_bf16, 8),
+               "layernorm_fwd: x, gamma and beta must be 16-byte aligned, y and y2 8-byte aligned");
   const int threads = 256;
   const long long blocks = ((long long)N * 32 + threads - 1) / threads;
 #define NEKO_LN_FWD(NV) launch_pdl(layernorm_fwd_kernel<NV>, dim3((unsigned)blocks), dim3(threads), 0, as_stream(stream), x, gamma, beta, y_bf16, y2_bf16, mean, rstd, N, d, eps, out_f16)
@@ -439,35 +495,39 @@ int neko_layernorm_fwd(const float* x, const float* gamma, const float* beta, ui
   return NEKO_OK;
 }
 
+int neko_layernorm_bwd_path(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean, const float* rstd,
+                            const float* dx_resid, const uint16_t* dx_bf16, const float* dgamma, const float* dbeta,
+                            const float* dx_colsum, int N, int d, const neko_dropout* branch_drop, neko_layernorm_bwd_path_info* out) {
+  using namespace neko;
+  (void)dx_colsum;
+  (void)branch_drop;
+  LnBwdPlan p;
+  const int rc = ln_bwd_plan(dy_bf16, x, gamma, mean, rstd, dx_resid, dx_bf16, dgamma, dbeta, N, d, p);
+  if (rc != NEKO_OK) return rc;
+  if (out) {
+    out->grid = p.grid;
+    out->rows_per_cta = p.rows_per_cta;
+    out->stages = p.stages;
+  }
+  return p.kernel;
+}
+
 int neko_layernorm_bwd(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean, const float* rstd,
                        float* dx_resid, uint16_t* dx_bf16, float* dgamma, float* dbeta, float* dx_colsum, int N, int d,
                        const neko_dropout* branch_drop, void* stream) {
   using namespace neko;
-  NEKO_REQUIRE(dy_bf16 && x && gamma && mean && rstd && dx_resid && dgamma && dbeta, "layernorm_bwd: null pointer");
-  NEKO_REQUIRE(N > 0 && d > 0 && d % 4 == 0 && d <= LN_MAX_D, "layernorm_bwd: need d %% 4 == 0 and d <= %d (got %d)", LN_MAX_D, d);
-  const int threads = ((d / 4 + 31) / 32) * 32;  // one float4 column group per thread
-  // ~2 CTAs per SM: enough loads in flight (12 per thread), few enough CTAs that the final atomics stay cheap
-  int ctas = sm_count() * 2;
-  if (const char* e = getenv("NEKO_LN_CTAS")) ctas = atoi(e);
-  int rows_per_cta = (N + ctas - 1) / ctas;
-  rows_per_cta = ((rows_per_cta + LNB_ROWS - 1) / LNB_ROWS) * LNB_ROWS;
-  ctas = (N + rows_per_cta - 1) / rows_per_cta;
-  // warp-per-row variant (default): d = 128 * NV with NV <= 8
-  static const bool force_cols = getenv("NEKO_LN_BWD_COLUMNS") != nullptr;
-  if (!force_cols && d % 128 == 0 && d <= 1024 && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dx_resid)) & 15) == 0 &&
-      (reinterpret_cast<uintptr_t>(dy_bf16) & 7) == 0 && (!dx_bf16 || (reinterpret_cast<uintptr_t>(dx_bf16) & 7) == 0)) {
+  LnBwdPlan p;
+  const int rc = ln_bwd_plan(dy_bf16, x, gamma, mean, rstd, dx_resid, dx_bf16, dgamma, dbeta, N, d, p);
+  if (rc != NEKO_OK) return rc;
+  const DropCfg dc = drop_cfg(branch_drop);
+  if (p.kernel == 0) {
     const int nv = d / 128;
-    const size_t smem_r = (size_t)(1 + 8 * 3) * d * sizeof(float);   // gamma + 8 warps x 3 accumulator rows
-    int grid = 2 * sm_count();                                       // two CTAs per SM
-    const int rows_per_grid = grid * 8;
-    if (N < rows_per_grid) grid = (N + 7) / 8;
-    const DropCfg dc = drop_cfg(branch_drop);
 #define NEKO_LNB_ROWS(NV_) { static bool attr_##NV_ = false;                                                                      \
       if (!attr_##NV_) {                                                                                                          \
         cudaError_t e_ = cudaFuncSetAttribute(layernorm_bwd_rows_kernel<NV_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 104 * 1024); \
         if (e_ != cudaSuccess) return check_cuda(e_, "cudaFuncSetAttribute(layernorm_bwd_rows)");                                    \
         attr_##NV_ = true; } }                                                                                                      \
-    launch_pdl(layernorm_bwd_rows_kernel<NV_>, dim3(grid), dim3(256), smem_r, as_stream(stream), \
+    launch_pdl(layernorm_bwd_rows_kernel<NV_>, dim3(p.grid), dim3(p.threads), p.smem, as_stream(stream), \
                                       reinterpret_cast<const bf16*>(dy_bf16), x, gamma, mean, rstd, dx_resid, reinterpret_cast<bf16*>(dx_bf16), \
                                       dgamma, dbeta, dx_colsum, N, d, dc)
     switch (nv) {
@@ -484,27 +544,20 @@ int neko_layernorm_bwd(const uint16_t* dy_bf16, const float* x, const float* gam
     NEKO_LAUNCH_CHECK("layernorm_bwd_rows_kernel");
     return NEKO_OK;
   }
-  // staged variant: ring of `stages` row blocks (40 d bytes each) in shared memory, two CTAs per SM
-  const size_t stage_bytes = (size_t)LNB_ROWS * d * 10;
-  int stages = (int)((100 * 1024) / stage_bytes);
-  if (stages > 4) stages = 4;
-  static const bool force_reg = getenv("NEKO_LN_BWD_REGISTER") != nullptr;
-  const bool aligned = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dx_resid) | reinterpret_cast<uintptr_t>(dy_bf16)) & 15) == 0;
-  if (stages >= 2 && d % 8 == 0 && aligned && !force_reg) {
-    const size_t smem = stage_bytes * stages;
+  if (p.kernel == 1) {
     static size_t attr_smem = 0;
-    if (smem > attr_smem) {
-      cudaError_t e = cudaFuncSetAttribute(layernorm_bwd_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (p.smem > attr_smem) {
+      cudaError_t e = cudaFuncSetAttribute(layernorm_bwd_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
       if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(layernorm_bwd_staged)");
-      attr_smem = smem;
+      attr_smem = p.smem;
     }
-    launch_pdl(layernorm_bwd_staged_kernel, dim3(ctas), dim3(threads), smem, as_stream(stream), reinterpret_cast<const bf16*>(dy_bf16), x, gamma,
-               mean, rstd, dx_resid, reinterpret_cast<bf16*>(dx_bf16), dgamma, dbeta, dx_colsum, N, d, rows_per_cta, stages, drop_cfg(branch_drop));
+    launch_pdl(layernorm_bwd_staged_kernel, dim3(p.grid), dim3(p.threads), p.smem, as_stream(stream), reinterpret_cast<const bf16*>(dy_bf16), x,
+               gamma, mean, rstd, dx_resid, reinterpret_cast<bf16*>(dx_bf16), dgamma, dbeta, dx_colsum, N, d, p.rows_per_cta, p.stages, dc);
     NEKO_LAUNCH_CHECK("layernorm_bwd_staged_kernel");
     return NEKO_OK;
   }
-  launch_pdl(layernorm_bwd_kernel, dim3(ctas), dim3(threads), 0, as_stream(stream), reinterpret_cast<const bf16*>(dy_bf16), x, gamma, mean, rstd,
-             dx_resid, reinterpret_cast<bf16*>(dx_bf16), dgamma, dbeta, dx_colsum, N, d, rows_per_cta, drop_cfg(branch_drop));
+  launch_pdl(layernorm_bwd_kernel, dim3(p.grid), dim3(p.threads), 0, as_stream(stream), reinterpret_cast<const bf16*>(dy_bf16), x, gamma, mean, rstd,
+             dx_resid, reinterpret_cast<bf16*>(dx_bf16), dgamma, dbeta, dx_colsum, N, d, p.rows_per_cta, dc);
   NEKO_LAUNCH_CHECK("layernorm_bwd_kernel");
   return NEKO_OK;
 }

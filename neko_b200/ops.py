@@ -12,7 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import (EPI_BF16, EPI_DGELU_BF16, EPI_F32, EPI_GELU_BF16, EPI_RESID_F32, EPI_RESID_F32_BF16,  # noqa: F401
-                   Dropout, GemmDesc, GemmPlanInfo, SampleDesc, TokParams, _p, check, load, stream_ptr)
+                   Dropout, GemmDesc, GemmPlanInfo, LnBwdPathInfo, SampleDesc, TokParams, _p, check, load, stream_ptr)
 
 
 _16BIT = (torch.bfloat16, torch.float16)
@@ -127,6 +127,21 @@ def gemm_plan(a: torch.Tensor, b: torch.Tensor, *, a_mn: bool = False, b_mn: boo
 # ------------------------------------------------------------------------------------------
 # LayerNorm
 # ------------------------------------------------------------------------------------------
+def _dense(dtypes, **ts):
+    """The kernels index rows as if dense: a strided view would be read as the wrong rows."""
+    for name, t in ts.items():
+        if t is not None:
+            assert t.dtype in dtypes[name], f"{name}: dtype {t.dtype}, expected one of {dtypes[name]}"
+            assert t.is_contiguous(), f"{name} must be contiguous"
+
+
+_LN_FWD_DT = dict(x=(torch.float32,), gamma=(torch.float32,), beta=(torch.float32,), y=_16BIT, y2=(torch.bfloat16,),
+                  mean=(torch.float32,), rstd=(torch.float32,))
+_LN_BWD_DT = dict(dy=(torch.bfloat16,), x=(torch.float32,), gamma=(torch.float32,), mean=(torch.float32,), rstd=(torch.float32,),
+                  dx_resid=(torch.float32,), dgamma=(torch.float32,), dbeta=(torch.float32,), dx_bf16=(torch.bfloat16,),
+                  dx_colsum=(torch.float32,))
+
+
 def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float = 1e-5, y=None, mean=None, rstd=None,
                   out_dtype: torch.dtype = torch.bfloat16, y2=None):
     _cuda(x, gamma, beta)
@@ -137,6 +152,7 @@ def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps:
         mean = torch.empty(N, device=x.device, dtype=torch.float32)
     if rstd is None:
         rstd = torch.empty(N, device=x.device, dtype=torch.float32)
+    _dense(_LN_FWD_DT, x=x, gamma=gamma, beta=beta, y=y, y2=y2, mean=mean, rstd=rstd)
     check(load().neko_layernorm_fwd(_p(x), _p(gamma), _p(beta), _p(y), _p(y2), _p(mean), _p(rstd), C.c_int(N), C.c_int(d),
                                     C.c_float(eps), C.c_int(int(y.dtype == torch.float16)), stream_ptr()), "neko_layernorm_fwd")
     return y, mean, rstd
@@ -148,9 +164,26 @@ def _dref(drop):
 
 def layernorm_bwd(dy_bf16, x, gamma, mean, rstd, dx_resid, dgamma, dbeta, dx_bf16=None, dx_colsum=None, branch_drop=None):
     N, d = x.shape
+    _dense(_LN_BWD_DT, dy=dy_bf16, x=x, gamma=gamma, mean=mean, rstd=rstd, dx_resid=dx_resid, dgamma=dgamma, dbeta=dbeta,
+           dx_bf16=dx_bf16, dx_colsum=dx_colsum)
     check(load().neko_layernorm_bwd(_p(dy_bf16), _p(x), _p(gamma), _p(mean), _p(rstd), _p(dx_resid), _p(dx_bf16),
                                     _p(dgamma), _p(dbeta), _p(dx_colsum), C.c_int(N), C.c_int(d), _dref(branch_drop), stream_ptr()),
           "neko_layernorm_bwd")
+
+
+LN_BWD_KERNELS = ("rows", "staged", "register")
+
+
+def layernorm_bwd_path(dy_bf16, x, gamma, mean, rstd, dx_resid, dgamma, dbeta, dx_bf16=None, dx_colsum=None, branch_drop=None) -> dict:
+    """The kernel layernorm_bwd() would run with the same arguments ("rows" = warp-per-row, "staged", "register") and its
+    launch shape; launches nothing.  Raises NekoError where layernorm_bwd() would reject the arguments."""
+    N, d = x.shape
+    info = LnBwdPathInfo()
+    rc = load().neko_layernorm_bwd_path(_p(dy_bf16), _p(x), _p(gamma), _p(mean), _p(rstd), _p(dx_resid), _p(dx_bf16), _p(dgamma),
+                                        _p(dbeta), _p(dx_colsum), C.c_int(N), C.c_int(d), _dref(branch_drop), C.byref(info))
+    if rc < 0:
+        check(rc, "neko_layernorm_bwd_path")
+    return dict(kernel=LN_BWD_KERNELS[rc], grid=info.grid, rows_per_cta=info.rows_per_cta, stages=info.stages)
 
 
 def geglu_fwd(act: torch.Tensor, gate: torch.Tensor, out: torch.Tensor, out_bf16: Optional[torch.Tensor] = None):
