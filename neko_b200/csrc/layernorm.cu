@@ -7,6 +7,7 @@
 #include <stdlib.h>
 #include "common.cuh"
 #include "dropout.cuh"
+#include "ordered.cuh"
 
 namespace neko {
 
@@ -72,6 +73,19 @@ __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const float* __restr
 // live in 12 registers per thread for the whole kernel (one global atomicAdd per column per CTA at the end).
 constexpr int LNB_ROWS = 4;
 
+// the column-owner kernels' final flush: one atomicAdd per column and CTA
+__device__ __forceinline__ void ln_cols_flush(int c4, const float4& ag, const float4& ab, const float4& ac, float* dgamma, float* dbeta,
+                                              float* dx_colsum) {
+  float* pg = dgamma + 4 * c4;
+  float* pb = dbeta + 4 * c4;
+  atomicAdd(pg, ag.x); atomicAdd(pg + 1, ag.y); atomicAdd(pg + 2, ag.z); atomicAdd(pg + 3, ag.w);
+  atomicAdd(pb, ab.x); atomicAdd(pb + 1, ab.y); atomicAdd(pb + 2, ab.z); atomicAdd(pb + 3, ab.w);
+  if (dx_colsum) {
+    float* pc = dx_colsum + 4 * c4;
+    atomicAdd(pc, ac.x); atomicAdd(pc + 1, ac.y); atomicAdd(pc + 2, ac.z); atomicAdd(pc + 3, ac.w);
+  }
+}
+
 __global__ void __launch_bounds__(512) layernorm_bwd_kernel(const bf16* __restrict__ dy, const float* __restrict__ x,
                                                             const float* __restrict__ gamma, const float* __restrict__ mean,
                                                             const float* __restrict__ rstd, float* __restrict__ dx_resid,
@@ -106,66 +120,11 @@ __global__ void __launch_bounds__(512) layernorm_bwd_kernel(const bf16* __restri
       mu[r] = (row < row1) ? __ldg(mean + row) : 0.f;
       rs[r] = (row < row1) ? __ldg(rstd + row) : 0.f;
     }
-    float s[2 * LNB_ROWS];
-    float4 gy[LNB_ROWS], xh[LNB_ROWS];
-#pragma unroll
-    for (int r = 0; r < LNB_ROWS; ++r) {
-      const float2 d01 = unpack_bf16x2(dv[r].x), d23 = unpack_bf16x2(dv[r].y);
-      xh[r] = make_float4((xv[r].x - mu[r]) * rs[r], (xv[r].y - mu[r]) * rs[r], (xv[r].z - mu[r]) * rs[r], (xv[r].w - mu[r]) * rs[r]);
-      gy[r] = make_float4(d01.x * g.x, d01.y * g.y, d23.x * g.z, d23.y * g.w);
-      s[r] = (gy[r].x + gy[r].y) + (gy[r].z + gy[r].w);
-      s[LNB_ROWS + r] = (gy[r].x * xh[r].x + gy[r].y * xh[r].y) + (gy[r].z * xh[r].z + gy[r].w * xh[r].w);
-      // column sums of dy and dy * xhat
-      ab.x += d01.x; ab.y += d01.y; ab.z += d23.x; ab.w += d23.y;
-      ag.x += d01.x * xh[r].x; ag.y += d01.y * xh[r].y; ag.z += d23.x * xh[r].z; ag.w += d23.y * xh[r].w;
-    }
-#pragma unroll
-    for (int i = 0; i < 2 * LNB_ROWS; ++i) s[i] = warp_sum(s[i]);
-    if (lane == 0) {
-#pragma unroll
-      for (int i = 0; i < 2 * LNB_ROWS; ++i) red[parity][wid][i] = s[i];
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 2 * LNB_ROWS; ++i) {
-      float t = 0.f;
-      for (int w = 0; w < nwarps; ++w) t += red[parity][w][i];
-      s[i] = t * inv_d;
-    }
-#pragma unroll
-    for (int r = 0; r < LNB_ROWS; ++r) {
-      const int row = rb + r;
-      if (act && row < row1) {
-        const float m1 = s[r], m2 = s[LNB_ROWS + r];
-        float4 o = rv[r];
-        o.x += rs[r] * (gy[r].x - m1 - xh[r].x * m2);
-        o.y += rs[r] * (gy[r].y - m1 - xh[r].y * m2);
-        o.z += rs[r] * (gy[r].z - m1 - xh[r].z * m2);
-        o.w += rs[r] * (gy[r].w - m1 - xh[r].w * m2);
-        const size_t off = (size_t)row * d;
-        reinterpret_cast<float4*>(dx_resid + off)[c4] = o;
-        if (drop.seed) {  // gradient entering the dropped-out residual branch: mask * scale * dx
-          const uint32_t rk = drop_rowkey(dkey, (uint32_t)row);
-          float m0, m1, m2_, m3;
-          drop_pair(rk, 2u * c4, drop.thr16, drop.scale, m0, m1);
-          drop_pair(rk, 2u * c4 + 1u, drop.thr16, drop.scale, m2_, m3);
-          o.x *= m0; o.y *= m1; o.z *= m2_; o.w *= m3;
-        }
-        if (dx_bf16) reinterpret_cast<uint2*>(dx_bf16 + off)[c4] = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
-        ac.x += o.x; ac.y += o.y; ac.z += o.z; ac.w += o.w;
-      }
-    }
+#define LN_COLS_STAGED 0
+#include "ln_bwd_cols.cuh"
+#undef LN_COLS_STAGED
   }
-  if (act) {
-    float* pg = dgamma + 4 * c4;
-    float* pb = dbeta + 4 * c4;
-    atomicAdd(pg, ag.x); atomicAdd(pg + 1, ag.y); atomicAdd(pg + 2, ag.z); atomicAdd(pg + 3, ag.w);
-    atomicAdd(pb, ab.x); atomicAdd(pb + 1, ab.y); atomicAdd(pb + 2, ab.z); atomicAdd(pb + 3, ab.w);
-    if (dx_colsum) {
-      float* pc = dx_colsum + 4 * c4;
-      atomicAdd(pc, ac.x); atomicAdd(pc + 1, ac.y); atomicAdd(pc + 2, ac.z); atomicAdd(pc + 3, ac.w);
-    }
-  }
+  if (act) ln_cols_flush(c4, ag, ab, ac, dgamma, dbeta, dx_colsum);
 }
 
 
@@ -252,69 +211,11 @@ __global__ void __launch_bounds__(512) layernorm_bwd_staged_kernel(const bf16* _
       rv[r] = ok ? reinterpret_cast<const float4*>(sb + xb + (size_t)r * d * 4)[c4] : make_float4(0.f, 0.f, 0.f, 0.f);
       dv[r] = ok ? reinterpret_cast<const uint2*>(sb + 2 * xb + (size_t)r * d * 2)[c4] : make_uint2(0u, 0u);
     }
-    float sred[2 * LNB_ROWS];
-    float4 gy[LNB_ROWS], xh[LNB_ROWS];
-#pragma unroll
-    for (int r = 0; r < LNB_ROWS; ++r) {
-      const float2 d01 = unpack_bf16x2(dv[r].x), d23 = unpack_bf16x2(dv[r].y);
-      xh[r] = make_float4((xv[r].x - mu[r]) * rs[r], (xv[r].y - mu[r]) * rs[r], (xv[r].z - mu[r]) * rs[r], (xv[r].w - mu[r]) * rs[r]);
-      gy[r] = make_float4(d01.x * g.x, d01.y * g.y, d23.x * g.z, d23.y * g.w);
-      sred[r] = (gy[r].x + gy[r].y) + (gy[r].z + gy[r].w);
-      sred[LNB_ROWS + r] = (gy[r].x * xh[r].x + gy[r].y * xh[r].y) + (gy[r].z * xh[r].z + gy[r].w * xh[r].w);
-      ab.x += d01.x; ab.y += d01.y; ab.z += d23.x; ab.w += d23.y;
-      ag.x += d01.x * xh[r].x; ag.y += d01.y * xh[r].y; ag.z += d23.x * xh[r].z; ag.w += d23.y * xh[r].w;
-    }
-#pragma unroll
-    for (int i = 0; i < 2 * LNB_ROWS; ++i) sred[i] = warp_sum(sred[i]);
-    if (lane == 0) {
-#pragma unroll
-      for (int i = 0; i < 2 * LNB_ROWS; ++i) red[parity][wid][i] = sred[i];
-    }
-    __syncthreads();   // every thread has read its slice of ring slot s: the slot may be refilled
-    if (threadIdx.x == 0 && it + stages < n_iter) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      issue(it + stages);
-    }
-#pragma unroll
-    for (int i = 0; i < 2 * LNB_ROWS; ++i) {
-      float t = 0.f;
-      for (int w = 0; w < nwarps; ++w) t += red[parity][w][i];
-      sred[i] = t * inv_d;
-    }
-#pragma unroll
-    for (int r = 0; r < LNB_ROWS; ++r) {
-      const int row = rb + r;
-      if (act && row < row1) {
-        const float m1 = sred[r], m2 = sred[LNB_ROWS + r];
-        float4 o = rv[r];
-        o.x += rs[r] * (gy[r].x - m1 - xh[r].x * m2);
-        o.y += rs[r] * (gy[r].y - m1 - xh[r].y * m2);
-        o.z += rs[r] * (gy[r].z - m1 - xh[r].z * m2);
-        o.w += rs[r] * (gy[r].w - m1 - xh[r].w * m2);
-        const size_t off = (size_t)row * d;
-        reinterpret_cast<float4*>(dx_resid + off)[c4] = o;
-        if (drop.seed) {
-          const uint32_t rk = drop_rowkey(dkey, (uint32_t)row);
-          float m0, m1_, m2_, m3;
-          drop_pair(rk, 2u * c4, drop.thr16, drop.scale, m0, m1_);
-          drop_pair(rk, 2u * c4 + 1u, drop.thr16, drop.scale, m2_, m3);
-          o.x *= m0; o.y *= m1_; o.z *= m2_; o.w *= m3;
-        }
-        if (dx_bf16) reinterpret_cast<uint2*>(dx_bf16 + off)[c4] = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
-        ac.x += o.x; ac.y += o.y; ac.z += o.z; ac.w += o.w;
-      }
-    }
+#define LN_COLS_STAGED 1
+#include "ln_bwd_cols.cuh"
+#undef LN_COLS_STAGED
   }
-  if (act) {
-    float* pg = dgamma + 4 * c4;
-    float* pb = dbeta + 4 * c4;
-    atomicAdd(pg, ag.x); atomicAdd(pg + 1, ag.y); atomicAdd(pg + 2, ag.z); atomicAdd(pg + 3, ag.w);
-    atomicAdd(pb, ab.x); atomicAdd(pb + 1, ab.y); atomicAdd(pb + 2, ab.z); atomicAdd(pb + 3, ab.w);
-    if (dx_colsum) {
-      float* pc = dx_colsum + 4 * c4;
-      atomicAdd(pc, ac.x); atomicAdd(pc + 1, ac.y); atomicAdd(pc + 2, ac.z); atomicAdd(pc + 3, ac.w);
-    }
-  }
+  if (act) ln_cols_flush(c4, ag, ab, ac, dgamma, dbeta, dx_colsum);
 }
 
 
@@ -346,65 +247,12 @@ __global__ void __launch_bounds__(256, 2) layernorm_bwd_rows_kernel(const bf16* 
   const float inv_d = 1.0f / (float)d;
   const uint32_t dkey = drop.seed ? drop_key(drop) : 0u;
   const int gw = blockIdx.x * nwarps + wid, tw = gridDim.x * nwarps;
-  for (int row = gw; row < N; row += tw) {
-    const size_t off = (size_t)row * d;
-    const float4* x4 = reinterpret_cast<const float4*>(x + off);
-    const uint2* d2 = reinterpret_cast<const uint2*>(dy + off);
-    float4* r4 = reinterpret_cast<float4*>(dx_resid + off);
-    float4 xv[NV], rv[NV];
-    uint2 dv[NV];
-#pragma unroll
-    for (int k = 0; k < NV; ++k) { xv[k] = x4[lane + 32 * k]; dv[k] = d2[lane + 32 * k]; rv[k] = r4[lane + 32 * k]; }
-    const float mu = __ldg(mean + row), rs = __ldg(rstd + row);
-    float s1 = 0.f, s2 = 0.f;
-#pragma unroll
-    for (int k = 0; k < NV; ++k) {
-      const int c4 = lane + 32 * k;
-      const float4 g = *reinterpret_cast<const float4*>(sg + 4 * c4);
-      const float2 d01 = unpack_bf16x2(dv[k].x), d23 = unpack_bf16x2(dv[k].y);
-      xv[k] = make_float4((xv[k].x - mu) * rs, (xv[k].y - mu) * rs, (xv[k].z - mu) * rs, (xv[k].w - mu) * rs);   // xhat
-      const float g0 = d01.x * g.x, g1 = d01.y * g.y, g2 = d23.x * g.z, g3 = d23.y * g.w;
-      s1 += (g0 + g1) + (g2 + g3);
-      s2 += (g0 * xv[k].x + g1 * xv[k].y) + (g2 * xv[k].z + g3 * xv[k].w);
-      float4* ag = reinterpret_cast<float4*>(wacc + 4 * c4);
-      float4* ab = reinterpret_cast<float4*>(wacc + d + 4 * c4);
-      float4 t = *ag;
-      t.x += d01.x * xv[k].x; t.y += d01.y * xv[k].y; t.z += d23.x * xv[k].z; t.w += d23.y * xv[k].w;
-      *ag = t;
-      t = *ab;
-      t.x += d01.x; t.y += d01.y; t.z += d23.x; t.w += d23.y;
-      *ab = t;
-    }
-    const float m1 = warp_sum(s1) * inv_d, m2 = warp_sum(s2) * inv_d;
-    uint32_t rk = 0u;
-    if (drop.seed) rk = drop_rowkey(dkey, (uint32_t)row);
-    uint2* b2 = dx_bf16 ? reinterpret_cast<uint2*>(dx_bf16 + off) : nullptr;
-#pragma unroll
-    for (int k = 0; k < NV; ++k) {
-      const int c4 = lane + 32 * k;
-      const float4 g = *reinterpret_cast<const float4*>(sg + 4 * c4);
-      const float2 d01 = unpack_bf16x2(dv[k].x), d23 = unpack_bf16x2(dv[k].y);
-      float4 o = rv[k];
-      o.x += rs * (d01.x * g.x - m1 - xv[k].x * m2);
-      o.y += rs * (d01.y * g.y - m1 - xv[k].y * m2);
-      o.z += rs * (d23.x * g.z - m1 - xv[k].z * m2);
-      o.w += rs * (d23.y * g.w - m1 - xv[k].w * m2);
-      r4[c4] = o;
-      if (drop.seed) {  // gradient entering the dropped-out residual branch: mask * scale * dx
-        float m0, m1_, m2_, m3;
-        drop_pair(rk, 2u * c4, drop.thr16, drop.scale, m0, m1_);
-        drop_pair(rk, 2u * c4 + 1u, drop.thr16, drop.scale, m2_, m3);
-        o.x *= m0; o.y *= m1_; o.z *= m2_; o.w *= m3;
-      }
-      if (b2) b2[c4] = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
-      if (dx_colsum) {
-        float4* ac = reinterpret_cast<float4*>(wacc + 2 * d + 4 * c4);
-        float4 t = *ac;
-        t.x += o.x; t.y += o.y; t.z += o.z; t.w += o.w;
-        *ac = t;
-      }
-    }
-  }
+  for (int row = gw; row < N; row += tw)
+#define LN_ROW_GUARD 0
+#define LN_ROW_COLSUM dx_colsum
+#include "ln_bwd_row.cuh"
+#undef LN_ROW_GUARD
+#undef LN_ROW_COLSUM
   __syncthreads();
   // fold the warps' slices: one thread per column, one global atomic per column and CTA
   for (int i = threadIdx.x; i < d; i += blockDim.x) {
@@ -416,6 +264,53 @@ __global__ void __launch_bounds__(256, 2) layernorm_bwd_rows_kernel(const bf16* 
     atomicAdd(dgamma + i, a);
     atomicAdd(dbeta + i, b);
     if (dx_colsum) atomicAdd(dx_colsum + i, c);
+  }
+}
+
+
+// ---------------------------------------------------------------------------------------------
+// Backward, ordered (deterministic mode): the warp-per-row math for any d % 4 == 0, d <= 2048.  Block `blk` = rows
+// [64 blk, 64 blk + 64): warp w takes rows 64 blk + w, + 8, ... in ascending order into its own shared accumulators, the warps
+// are folded in order 0..7 and the block's dgamma | dbeta | colsum partials go to workspace row blk.
+// ---------------------------------------------------------------------------------------------
+template <int NV>
+__global__ void __launch_bounds__(256) layernorm_bwd_ordered_kernel(const bf16* __restrict__ dy, const float* __restrict__ x,
+                                                                    const float* __restrict__ gamma, const float* __restrict__ mean,
+                                                                    const float* __restrict__ rstd, float* __restrict__ dx_resid,
+                                                                    bf16* __restrict__ dx_bf16, float* __restrict__ ws, int N, int d,
+                                                                    int n_blocks, int with_colsum, DropCfg drop) {
+  extern __shared__ __align__(16) float lno_s[];   // gamma [d] | per-warp accumulators [8][3][d]
+  float* sg = lno_s;
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  float* wacc = lno_s + d + (size_t)wid * 3 * d;
+  for (int i = threadIdx.x; i < d; i += blockDim.x) sg[i] = gamma[i];
+  const int nv4 = d >> 2;
+  const float inv_d = 1.0f / (float)d;
+  const uint32_t dkey = drop.seed ? drop_key(drop) : 0u;
+  for (int blk = blockIdx.x; blk < n_blocks; blk += gridDim.x) {
+    for (int i = lane; i < 3 * d; i += 32) wacc[i] = 0.f;
+    __syncthreads();
+    const int r_end = min(N, (blk + 1) * ORD_ROWS);
+    for (int row = blk * ORD_ROWS + wid; row < r_end; row += 8)
+#define LN_ROW_GUARD 1
+#define LN_ROW_COLSUM with_colsum
+#include "ln_bwd_row.cuh"
+#undef LN_ROW_GUARD
+#undef LN_ROW_COLSUM
+    __syncthreads();
+    float* out = ws + (size_t)blk * 3 * d;
+    for (int i = threadIdx.x; i < d; i += blockDim.x) {
+      float a = 0.f, b = 0.f, c = 0.f;
+#pragma unroll
+      for (int w = 0; w < 8; ++w) {
+        const float* s = lno_s + d + (size_t)w * 3 * d;
+        a += s[i]; b += s[d + i]; c += s[2 * d + i];
+      }
+      out[i] = a;
+      out[d + i] = b;
+      if (with_colsum) out[2 * d + i] = c;
+    }
+    __syncthreads();   // the next block re-zeroes the accumulators just read
   }
 }
 
@@ -560,6 +455,52 @@ int neko_layernorm_bwd(const uint16_t* dy_bf16, const float* x, const float* gam
              dx_resid, reinterpret_cast<bf16*>(dx_bf16), dgamma, dbeta, dx_colsum, N, d, p.rows_per_cta, dc);
   NEKO_LAUNCH_CHECK("layernorm_bwd_kernel");
   return NEKO_OK;
+}
+
+int64_t neko_layernorm_bwd_ordered_workspace_bytes(int N, int d) {
+  using namespace neko;
+  NEKO_REQUIRE(N > 0 && d > 0 && d % 4 == 0 && d <= LN_MAX_D, "layernorm_bwd_ordered: need N > 0, d %% 4 == 0 and d <= %d", LN_MAX_D);
+  return (int64_t)((N + ORD_ROWS - 1) / ORD_ROWS) * 3 * d * (int64_t)sizeof(float);
+}
+
+int neko_layernorm_bwd_ordered(const uint16_t* dy_bf16, const float* x, const float* gamma, const float* mean, const float* rstd,
+                               float* dx_resid, uint16_t* dx_bf16, float* dgamma, float* dbeta, float* dx_colsum, int N, int d,
+                               const neko_dropout* branch_drop, void* workspace, int64_t workspace_bytes, void* stream) {
+  using namespace neko;
+  NEKO_REQUIRE(dy_bf16 && x && gamma && mean && rstd && dx_resid && dgamma && dbeta && workspace, "layernorm_bwd_ordered: null pointer");
+  const int64_t need = neko_layernorm_bwd_ordered_workspace_bytes(N, d);
+  if (need < 0) return (int)need;
+  NEKO_REQUIRE(workspace_bytes >= need, "layernorm_bwd_ordered: workspace of %lld bytes, need %lld", (long long)workspace_bytes, (long long)need);
+  NEKO_REQUIRE(ln_al(x, 16) && ln_al(dx_resid, 16) && ln_al(gamma, 16) && ln_al(dy_bf16, 8) && ln_al(dx_bf16, 8) && ln_al(workspace, 16),
+               "layernorm_bwd_ordered: x, dx_resid, gamma and the workspace must be 16-byte aligned, dy and dx_bf16 8-byte aligned");
+  const int n_blocks = (N + ORD_ROWS - 1) / ORD_ROWS;
+  const int need_v = (d / 4 + 31) / 32;
+  const size_t smem = (size_t)(1 + 8 * 3) * d * sizeof(float);
+  float* ws = static_cast<float*>(workspace);
+  const DropCfg dc = drop_cfg(branch_drop);
+  const int grid = ordered_grid(n_blocks);
+#define NEKO_LN_ORD(NV_) {                                                                                                          \
+    static bool attr_ = false;                                                                                                      \
+    if (!attr_) {                                                                                                                   \
+      cudaError_t e_ = cudaFuncSetAttribute(layernorm_bwd_ordered_kernel<NV_>, cudaFuncAttributeMaxDynamicSharedMemorySize,           \
+                                            (int)((1 + 8 * 3) * LN_MAX_D * sizeof(float)));                                        \
+      if (e_ != cudaSuccess) return check_cuda(e_, "cudaFuncSetAttribute(layernorm_bwd_ordered)");                                  \
+      attr_ = true;                                                                                                                 \
+    }                                                                                                                               \
+    layernorm_bwd_ordered_kernel<NV_><<<grid, 256, smem, as_stream(stream)>>>(                                                      \
+        reinterpret_cast<const bf16*>(dy_bf16), x, gamma, mean, rstd, dx_resid, reinterpret_cast<bf16*>(dx_bf16), ws, N, d,        \
+        n_blocks, dx_colsum != nullptr, dc); }
+  if (need_v <= 1) NEKO_LN_ORD(1) else if (need_v <= 2) NEKO_LN_ORD(2) else if (need_v <= 3) NEKO_LN_ORD(3)
+  else if (need_v <= 4) NEKO_LN_ORD(4) else if (need_v <= 6) NEKO_LN_ORD(6) else if (need_v <= 8) NEKO_LN_ORD(8)
+  else if (need_v <= 12) NEKO_LN_ORD(12) else NEKO_LN_ORD(16)
+#undef NEKO_LN_ORD
+  NEKO_LAUNCH_CHECK("layernorm_bwd_ordered_kernel");
+  OrdDst dst{};
+  dst.p[0] = dgamma; dst.p[1] = dbeta; dst.p[2] = dx_colsum;
+  dst.off[0] = 0; dst.off[1] = d; dst.off[2] = 2 * d;
+  dst.n = dx_colsum ? 3 : 2;
+  for (int i = dst.n; i < 7; ++i) dst.off[i] = i == dst.n ? dst.n * d : 0x7fffffff;
+  return ordered_colreduce(ws, 3LL * d, n_blocks, dst.n * d, dst, 1, as_stream(stream));
 }
 
 }  // extern "C"

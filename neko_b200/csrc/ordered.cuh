@@ -4,6 +4,8 @@
 
 namespace neko {
 
+constexpr int ORD_ROWS = 64;          // rows per fixed block of the column sums
+
 // Destination of an ordered column reduction: columns [off[i], off[i+1]) of the workspace rows go to p[i][0 ..].
 struct OrdDst {
   float* p[6];
